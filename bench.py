@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload sparse_ls|rosenbrock|logreg|batched] [--n N] [--coh C] [--quadratic-ls]
+                    [--dump-outputs DIR]
 
 A "step" is one iteration of the `for n = 1:max_iters` body of minimizeobjective
 (src/engine/optim.jl:50-160): one strong-Wolfe line search (>= 1 fdf! trial) + getβ + the
@@ -55,8 +56,9 @@ def parse():
     p.add_argument("--gather-block-mib", type=float, default=0.0,
                    help="logreg: size of the column blocks of the gathered vectors (0: library default, 40 MiB)")
     p.add_argument("--max-reps", type=int, default=100, help="cap on the repetitions of the K-step measurement")
-    p.add_argument("--min-timed-s", type=float, default=2.0,
-                   help="repeat the K-step measurement (fresh run from x0 each time) until the timed region is this long")
+    p.add_argument("--min-timed-s", type=float, default=0.0,
+                   help="repeat the K-step measurement (fresh run from x0 each time) until the timed region is this long "
+                        "(default 0: one measurement, exactly --steps timed steps)")
     p.add_argument("--no-parity-assert", action="store_true",
                    help="report parity_vs_n1 of the headline variant without failing when it exceeds 1e-10")
     p.add_argument("--write-fixture", action="store_true",
@@ -66,6 +68,10 @@ def parse():
                    help="sparse_ls only: the quadratic-aware line search (SURVEY.md §8f N1), one SpMV + one SpMVT per iteration")
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-e2e", action="store_true")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the timed path returns after its last step (iterate, gradient, "
+                        "objective, trace; a fixed sample of long vectors) as DIR/<name>.npy, so that two builds can be "
+                        "compared on the same inputs")
     return p.parse_args()
 
 
@@ -342,10 +348,46 @@ def parity_gate(args, par, what):
                              f"(--no-parity-assert reports it without failing)")
 
 
-def measure_device(cg, torch, args, ctx, obj, x0, n, coh, world, rank, local_rank, stream, barrier):
+DUMP_ENTRIES = 1 << 19        # --dump-outputs: entries kept of a longer output vector (4 MiB in float64)
+DUMP_LIMIT = 64 << 20         # --dump-outputs: bytes written at most, all files and ranks together
+
+
+def sample_index(n, cap):
+    """Sorted indices of the entries --dump-outputs keeps of an output of length n: all of them when n <= cap,
+    else cap of them drawn with a fixed seed, so that every run with the same arguments keeps the same ones."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+
+def run_outputs(run, cap):
+    """What a caller of the timed path holds after its last step: the iterate and the gradient (`Results.minimizer`,
+    `.gradient`: this rank's shard, sampled), f there, and the trace of the run up to that step."""
+    ret = run.results()
+    idx = sample_index(len(ret.minimizer), cap)
+    k, t = run.n, ret.trace
+    return {"minimizer": ret.minimizer[idx], "gradient": ret.gradient[idx], "sample_index": idx,
+            "objective": np.array([run.f_x]), "trace_objective": t.objective[:k], "trace_grad_norm": t.grad_norm[:k],
+            "trace_step_size": t.step_size[:k], "trace_objective_evals": t.objective_evals[:k]}
+
+
+def write_outputs(path, arrays, rank, world):
+    """path/<name>.npy (path/<name>_rank<r>.npy under torchrun), in float64 unless the output is float32"""
+    out = {k: np.asarray(v, dtype=np.float32 if np.asarray(v).dtype == np.float32 else np.float64)
+           for k, v in arrays.items()}
+    size = world * sum(a.nbytes for a in out.values())
+    assert size <= DUMP_LIMIT, f"--dump-outputs: {size} bytes > {DUMP_LIMIT}"
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
+def measure_device(cg, torch, args, ctx, obj, x0, n, coh, world, rank, local_rank, stream, barrier, dump=False):
     """Device-resident throughput of one configuration: W untimed iterations, then EXACTLY K timed ones (CUDA
-    events on the ctx stream), repeated from x0 until the timed region is at least --min-timed-s long; `ms` is
-    the mean over the repetitions.  The metric is iterations/s with ϵ out of reach, so a run only ends when the
+    events on the ctx stream), repeated from x0 until the timed region is at least --min-timed-s long (by default
+    once); `ms` is the mean over the repetitions.  `dump`: also return what the run holds after the last timed
+    step (run_outputs), read after the clock stopped.
+    The metric is iterations/s with ϵ out of reach, so a run only ends when the
     line search hits the FP64 floor of the objective (≈53 iterations on cfg 3, ≈28 on cfg 4: both problems are
     well conditioned).  If that happens inside a repetition, the clock stops at the end of the last completed
     iteration (the 100-trial zoom that fails is not an iteration and is not timed) and a fresh run continues the
@@ -408,7 +450,6 @@ def measure_device(cg, torch, args, ctx, obj, x0, n, coh, world, rank, local_ran
         for k, v in ctx.timing_read(reset=True).items():
             a = timers_tot.setdefault(k, [0.0, 0])
             a[0] += v[0]; a[1] += v[1]
-        run.info.close()
         reps += 1
         # every rank repeats the same number of times: decide on the slowest rank's clock
         tms = torch.tensor([ms], dtype=torch.float64, device="cuda")
@@ -425,15 +466,18 @@ def measure_device(cg, torch, args, ctx, obj, x0, n, coh, world, rank, local_ran
             dist.all_reduce(tstop, op=dist.ReduceOp.MAX)
         if float(tstop.item()) > 0:
             break
+        run.info.close()
     sampler.mark_end()
     barrier()
     ctx.timing(False)
     clocks = sampler.stop() if rank == 0 else None
+    outputs = run_outputs(run, DUMP_ENTRIES // world) if dump else None
+    run.info.close()
     return {"K": K, "W": W, "reps": reps, "ms": ms_tot / reps, "ms_median": float(np.median(rep_ms)),
             "timed_region_s": ms_tot * 1e-3, "wall_ms": wall_tot / reps,
             "evals": evals / reps, "evals_total": evals, "launches": launches / reps, "restarts": restarts, "life": life,
             "trace": trace_f, "timers": {k: (v[0] / reps, v[1] / reps) for k, v in timers_tot.items()}, "clocks": clocks,
-            "qkw": qkw}
+            "qkw": qkw, "outputs": outputs}
 
 
 def roofline_of(args, obj, m, n, coh, world, n_local, nnz_local):
@@ -518,7 +562,9 @@ def run_ours(args):
     coh = args.coh
 
     # ---------------- device-resident throughput (`value`) ----------------
-    m = measure_device(cg, torch, args, ctx, obj, x0, n, coh, world, rank, local_rank, stream, barrier)
+    dump = args.dump_outputs is not None
+    m = measure_device(cg, torch, args, ctx, obj, x0, n, coh, world, rank, local_rank, stream, barrier, dump)
+    outputs = m["outputs"]
     K, W, ms, qkw, life = m["K"], m["W"], m["ms"], m["qkw"], m["life"]
     roofline = roofline_of(args, obj, m, n, coh, world, n_local, nnz_local)
     par, par_note = parity_vs_n1(args, n, coh, m["trace"])
@@ -582,7 +628,9 @@ def run_ours(args):
         args2 = argparse.Namespace(**vars(args))
         args2.coh = coh2
         obj2, x02 = make_objective(cg, args2, ctx, n)
-        m2 = measure_device(cg, torch, args2, ctx, obj2, x02, n, coh2, world, rank, local_rank, stream, barrier)
+        m2 = measure_device(cg, torch, args2, ctx, obj2, x02, n, coh2, world, rank, local_rank, stream, barrier, dump)
+        if dump:
+            outputs.update({"secondary_" + k: v for k, v in m2["outputs"].items()})
         r2 = roofline_of(args2, obj2, m2, n, coh2, world, n_local, nnz_local)
         p2, p2_note = parity_vs_n1(args2, n, coh2, m2["trace"])
         secondary = {("coh%d" % coh2): {
@@ -597,6 +645,8 @@ def run_ours(args):
         obj2.close()
     if args.write_fixture and world == 1:
         write_fixture(args, n, coh, m["trace"])
+    if dump:
+        write_outputs(args.dump_outputs, outputs, rank, world)
 
     line = None
     if rank == 0:
@@ -660,7 +710,7 @@ def run_batched(args):
     X0p = torch.from_numpy(X0).pin_memory().numpy()
     cfg = cg.setupCGConfig(1e-5, cg.HagerZhang(), cg.DisableTrace(), max_iters=1000)
     ls = cg.setupStrongWolfeBisection(1e-5, 0.8, a_max_growth_factor=2.0, max_iters=1000, zoom_max_iters=100)
-    K, W = max(args.steps // 10, 2), max(min(args.warmup, 3), 1)
+    K, W = max(args.steps, 1), max(min(args.warmup, 3), 1)
     for _ in range(W):
         res = cg.minimizeobjective_batched(X0p, cfg, ls, ctx)
     ctx.timing(True)
@@ -680,6 +730,12 @@ def run_batched(args):
     clocks = sampler.stop() if rank == 0 else None
     kms = ctx.timing_read(reset=True)["batched"][0]
     ctx.timing(False)
+    if args.dump_outputs is not None:          # the last solve's per-problem results, the minimizers of sampled problems
+        rows = sample_index(nprob, max(DUMP_ENTRIES // (world * n), 1))
+        write_outputs(args.dump_outputs, {
+            "minimizer": res.minimizer[rows], "sample_index": rows, "objective": res.objective,
+            "grad_norm": res.grad_norm, "iters_ran": res.iters_ran, "status_code": res.status_code,
+            "fdf_evals": res.fdf_evals}, rank, world)
     t = torch.tensor([kms, wall], dtype=torch.float64, device="cuda")
     if world > 1:
         import torch.distributed as dist
@@ -776,6 +832,8 @@ def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs is not None:
+            raise SystemExit("bench.py: --dump-outputs writes the outputs of the device path (--impl ours)")
         if rank != 0:
             return
         threads = os.cpu_count() or 1

@@ -1,5 +1,6 @@
 """CPU checks of bench.py: the byte-accounting helpers behind `roofline.achieved`, the shard helper, the
-ncu-traffic lookup, and the reference arm's JSON line (the one leg of bench.py that runs without a GPU)."""
+ncu-traffic lookup, the reference arm's JSON line (the one leg of bench.py that runs without a GPU) and the
+files of --dump-outputs; on the GPU, that --steps K times K steps and two runs dump the same outputs."""
 import importlib.util
 import json
 import os
@@ -92,3 +93,41 @@ def test_parity_fixture_lookup(bench, tmp_path, monkeypatch):
         bench.parity_gate(a, rel, "x")
     a.no_parity_assert = True
     bench.parity_gate(a, rel, "x")
+
+
+def test_dump_outputs_sample_and_files(bench, tmp_path):
+    import numpy as np
+    assert np.array_equal(bench.sample_index(10, 16), np.arange(10))
+    i = bench.sample_index(200_000_000, 1000)
+    assert np.array_equal(i, bench.sample_index(200_000_000, 1000))                # seeded: the same entries every run
+    assert len(i) == 1000 and np.all(np.diff(i) > 0) and i[-1] < 200_000_000
+    bench.write_outputs(str(tmp_path / "o"), {"x": np.arange(3), "y": np.ones(2, np.float32)}, 0, 1)
+    assert np.load(tmp_path / "o" / "x.npy").dtype == np.float64 and np.load(tmp_path / "o" / "y.npy").dtype == np.float32
+    bench.write_outputs(str(tmp_path / "r"), {"x": np.zeros(2)}, 1, 2)
+    assert os.listdir(tmp_path / "r") == ["x_rank1.npy"]
+    with pytest.raises(AssertionError):
+        bench.write_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT // 8 + 1)}, 0, 1)
+    assert not os.path.exists(tmp_path / "big")
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_two_runs_are_identical(tmp_path):
+    import numpy as np
+
+    def run(d):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "4", "--warmup", "3", "--n", "200000",
+                            "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-2000:]
+        return json.loads(p.stdout.strip().splitlines()[-1])
+
+    a, _ = run(tmp_path / "a"), run(tmp_path / "b")
+    assert a["steps"] == 4 and a["config"]["repetitions"] == 1 and a["config"]["fdf_evals_in_timed_region"] >= 4
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b"))
+    assert {"minimizer.npy", "gradient.npy", "objective.npy", "secondary_minimizer.npy"} <= set(names)
+    for f in names:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f
+    if a["config"]["restarts_in_timed_region"] == 0:
+        assert len(np.load(tmp_path / "a" / "trace_objective.npy")) == 3 + 4
+    assert len(np.load(tmp_path / "a" / "minimizer.npy")) == 200_000
