@@ -1030,15 +1030,16 @@ static int state_create(cgo_ctx *ctx, cgo_obj *obj, const double *x0, bool x0_on
         st->xp_alloc = 1;
         st->m = lbfgs_m;
         if (lbfgs_m > 0) {
+            // m + 1 slots: a pair is staged into the one slot no live pair occupies, so rejecting it touches nothing live
             const size_t hist_bytes = sizeof(double) * (size_t)(st->n + 4);
-            for (int k = 0; k < lbfgs_m; ++k) {
+            for (int k = 0; k <= lbfgs_m; ++k) {
                 void *s = nullptr, *y = nullptr;
                 CGO_TRY(cgo_dev_alloc(ctx, hist_bytes, &s));
                 st->S.push_back((double *)s);
                 CGO_TRY(cgo_dev_alloc(ctx, hist_bytes, &y));
                 st->Y.push_back((double *)y);
             }
-            st->rho.assign(lbfgs_m, 0.0);
+            st->rho.assign(lbfgs_m + 1, 0.0);
             void *q = nullptr;
             CGO_TRY(cgo_dev_alloc(ctx, hist_bytes, &q));
             st->q = (double *)q;
@@ -1236,7 +1237,8 @@ extern "C" int cgo_solvesys_accept(cgo_state *st, int32_t fix_stale_iterate) {
 extern "C" int cgo_lbfgs_stage_pair(cgo_state *st, double out[CGO_PACK_LEN]) {
     CGO_CHECK(st && out, "NULL argument");
     CGO_CHECK(st->m > 0, "state was created without an L-BFGS history (lbfgs_m = 0)");
-    int slot = (st->count == 0) ? 0 : (st->head + 1) % st->m;
+    // the slot after the newest pair: the spare one (the ring has m + 1 slots and at most m pairs live)
+    const int slot = (st->head + 1) % (st->m + 1);
     LbfgsStage op;
     op.xp = (const double2 *)st->xp; op.x = (const double2 *)st->x;
     op.gp = (const double2 *)st->gp; op.g = (const double2 *)st->g;
@@ -1248,14 +1250,12 @@ extern "C" int cgo_lbfgs_stage_pair(cgo_state *st, double out[CGO_PACK_LEN]) {
 extern "C" int cgo_lbfgs_commit_pair(cgo_state *st, int32_t commit, double rho, double gamma) {
     CGO_CHECK(st != nullptr, "NULL state");
     CGO_CHECK(st->staged >= 0, "cgo_lbfgs_commit_pair without a staged pair");
-    if (commit) {
+    if (commit) {        // the staged slot becomes the newest pair; at count == m the oldest one becomes the spare
         st->head = st->staged;
         if (st->count < st->m) st->count++;
         st->rho[st->staged] = rho;
         st->gamma = gamma;
-    } else if (st->count == st->m) {
-        st->count--;     // the staged slot overwrote the oldest pair
-    }
+    }                    // a rejected pair leaves the history as it was (N&W Alg. 7.5)
     st->staged = -1;
     return 0;
 }
@@ -1276,8 +1276,8 @@ extern "C" int cgo_lbfgs_update_dir(cgo_state *st, double out[CGO_PACK_LEN]) {
     CGO_CHECK(st->m > 0, "state was created without an L-BFGS history (lbfgs_m = 0)");
     cgo_ctx *c = st->ctx;
     if (st->count == 0) return cgo_reset_direction(st, out);
-    const int cnt = st->count, m = st->m;
-    auto slot_of = [&](int k) { return ((st->head - k) % m + m) % m; };   // k = 0 newest
+    const int cnt = st->count, R = st->m + 1;
+    auto slot_of = [&](int k) { return ((st->head - k) % R + R) % R; };   // k = 0 newest
     double2 *q = (double2 *)st->q;
     // loop 1 (newest → oldest): dots land in d_scal[k]
     for (int k = 0; k < cnt; ++k) {

@@ -5,7 +5,7 @@ iteration and, because it sets `s = B\\y` (:81), is a mathematical no-op (SURVEY
 not built; `BroydenFamily` below is kept as what that update computes.  `LBFGS(m)` is the new flavour behind the same four-method plugin interface
 (initializeβ, initializeLineSearchContainer!, getβ, updatedir!): textbook two-loop recursion
 (Nocedal & Wright Alg. 7.4/7.5) over the m stored (s, y) pairs, s = xp − x, y = g⁺ − g,
-H₀ = (s·y / y·y) I, pair kept only when s·y > 0.
+H₀ = (s·y / y·y) I, pair kept only when s·y > 0; a rejected pair leaves the history unchanged.
 """
 from __future__ import annotations
 

@@ -627,7 +627,7 @@ typedef struct { /* LineSearchContainer, src/types.jl:84-100 */
     int64_t n;
 } ls_container;
 
-typedef struct { /* L-BFGS history (new flavour; N&W Alg 7.4/7.5) */
+typedef struct { /* L-BFGS history (new flavour; N&W Alg 7.4/7.5): a ring of m + 1 slots, at most m pairs live */
     int m, count, head;     /* head = slot of the newest pair */
     double **S, **Y;
     double *rho, *alpha;
@@ -980,9 +980,10 @@ static double beta_ls(solver *s, const double *g_next, const double *g, const do
 static void lbfgs_push(solver *s, const double *g_next, const double *g) {
     lbfgs_hist *H = &s->hist;
     ls_container *I = &s->info;
-    int slot = (H->count == 0) ? 0 : (H->head + 1) % H->m;
+    int slot = (H->head + 1) % (H->m + 1);
     double *S = H->S[slot], *Y = H->Y[slot];
-    /* write into the slot after the newest; only commit (advance head) when curvature holds */
+    /* write into the slot after the newest, which no live pair occupies; only commit (advance head)
+     * when curvature holds.  A rejected pair leaves the history unchanged. */
     for (int64_t i = 0; i < I->n; ++i) S[i] = I->xp[i] - I->x[i];
     for (int64_t i = 0; i < I->n; ++i) Y[i] = g_next[i] - g[i];
     double sy = vdot(s, S, Y);
@@ -992,9 +993,6 @@ static void lbfgs_push(solver *s, const double *g_next, const double *g) {
         if (H->count < H->m) H->count++;
         H->rho[slot] = 1.0 / sy;
         H->gamma = sy / yy;
-    } else if (H->count == H->m) {
-        /* the slot we scribbled on was the oldest pair: it is gone; shrink history by one */
-        H->count--;
     }
 }
 /* L-BFGS updatedir!: two-loop recursion, N&W Alg 7.4; u = −H g */
@@ -1008,7 +1006,7 @@ static void lbfgs_updatedir(solver *s, double *u, const double *g) {
     double *q = vtmp(n);
     for (int64_t i = 0; i < n; ++i) q[i] = g[i];
     for (int k = 0; k < H->count; ++k) {                /* newest → oldest */
-        int slot = ((H->head - k) % H->m + H->m) % H->m;
+        int slot = ((H->head - k) % (H->m + 1) + H->m + 1) % (H->m + 1);
         double al = H->rho[slot] * vdot(s, H->S[slot], q);
         H->alpha[slot] = al;
         const double *Y = H->Y[slot];
@@ -1016,7 +1014,7 @@ static void lbfgs_updatedir(solver *s, double *u, const double *g) {
     }
     for (int64_t i = 0; i < n; ++i) q[i] = H->gamma * q[i];
     for (int k = H->count - 1; k >= 0; --k) {           /* oldest → newest */
-        int slot = ((H->head - k) % H->m + H->m) % H->m;
+        int slot = ((H->head - k) % (H->m + 1) + H->m + 1) % (H->m + 1);
         double be = H->rho[slot] * vdot(s, H->Y[slot], q);
         double cf = H->alpha[slot] - be;
         const double *S = H->S[slot];
@@ -1049,11 +1047,11 @@ int orc_minimize(orc_objective *obj, const double *x0, const orc_config *cfg, do
     if (cfg->flavour == ORC_LBFGS) {
         int m = cfg->lbfgs_m > 0 ? cfg->lbfgs_m : 1;
         S.hist.m = m;
-        S.hist.S = (double **)calloc((size_t)m, sizeof(double *));
-        S.hist.Y = (double **)calloc((size_t)m, sizeof(double *));
-        for (int k = 0; k < m; ++k) { S.hist.S[k] = vtmp(D); S.hist.Y[k] = vtmp(D); }
-        S.hist.rho = (double *)calloc((size_t)m, sizeof(double));
-        S.hist.alpha = (double *)calloc((size_t)m, sizeof(double));
+        S.hist.S = (double **)calloc((size_t)m + 1, sizeof(double *));
+        S.hist.Y = (double **)calloc((size_t)m + 1, sizeof(double *));
+        for (int k = 0; k <= m; ++k) { S.hist.S[k] = vtmp(D); S.hist.Y[k] = vtmp(D); }
+        S.hist.rho = (double *)calloc((size_t)m + 1, sizeof(double));
+        S.hist.alpha = (double *)calloc((size_t)m + 1, sizeof(double));
     }
 
     double f_x = obj->fdf(obj, df_x, x);                                    /* :25 */
@@ -1121,7 +1119,7 @@ done:
     free(df_x); free(x);
     free(I->xp); free(I->df_xp); free(I->x); free(I->u);
     if (cfg->flavour == ORC_LBFGS) {
-        for (int k = 0; k < S.hist.m; ++k) { free(S.hist.S[k]); free(S.hist.Y[k]); }
+        for (int k = 0; k <= S.hist.m; ++k) { free(S.hist.S[k]); free(S.hist.Y[k]); }
         free(S.hist.S); free(S.hist.Y); free(S.hist.rho); free(S.hist.alpha);
     }
     return 0;

@@ -50,6 +50,14 @@ def make_pair(flavour="HagerZhang", linesearch="StrongWolfeBisection", eps=1e-5,
     return ocfg, cfg, ls
 
 
+def natural_lbfgs_rejection_case():
+    """(oracle config, host config, line search, x0) of a run of the chained Rosenbrock (n = 2) with LBFGS(1) and
+    Backtracking{Armijo}: Armijo alone does not keep s·y > 0, and from this start getβ rejects a pair while the
+    one-pair history is full, after which the run goes on to max_iters"""
+    ocfg, cfg, ls = make_pair("LBFGS", "Backtracking", eps=1e-10, max_iters=100, lbfgs_m=1)
+    return ocfg, cfg, ls, np.array([2.1769160886969896, 2.6836698800822507])
+
+
 def assert_same_run(ret, ora, exact=True, rtol=0.0, what=""):
     """Host-mirror Results vs OracleResult: statuses, counts, line-search decisions equal;
     f / ‖g‖ traces bit-identical (exact) or within rtol."""

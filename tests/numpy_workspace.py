@@ -71,7 +71,8 @@ class NumpyWorkspace:
         self._pending = None
         self.xp, self.df_xp, self.x, self.u, self.df_x = (_Vec(self, n) for n in ("xp", "df_xp", "x", "u", "df_x"))
         self.m = lbfgs_m
-        self.S, self.Y, self.rho = [None] * max(lbfgs_m, 1), [None] * max(lbfgs_m, 1), [0.0] * max(lbfgs_m, 1)
+        # a ring of m + 1 slots: a pair is staged into the one no live pair occupies
+        self.S, self.Y, self.rho = [None] * (lbfgs_m + 1), [None] * (lbfgs_m + 1), [0.0] * (lbfgs_m + 1)
         self.count, self.head, self.gamma, self.staged = 0, 0, 1.0, -1
 
     def _bdot(self, a, b):
@@ -179,7 +180,7 @@ class NumpyWorkspace:
 
     # L-BFGS (staging happens before accept: xp_ is the new point, x_ the old)
     def lbfgs_stage_pair(self):
-        slot = 0 if self.count == 0 else (self.head + 1) % self.m
+        slot = (self.head + 1) % (self.m + 1)
         self.S[slot] = self.xp_ - self.x_
         self.Y[slot] = self.gp_ - self.g_
         self.staged = slot
@@ -191,9 +192,7 @@ class NumpyWorkspace:
             self.count = min(self.count + 1, self.m)
             self.rho[self.staged] = float(rho)
             self.gamma = float(gamma)
-        elif self.count == self.m:
-            self.count -= 1
-        self.staged = -1
+        self.staged = -1             # a rejected pair leaves the history unchanged
 
     def lbfgs_update_dir(self):
         self._pending = None
@@ -201,7 +200,7 @@ class NumpyWorkspace:
             return self.reset_direction()
         q = self.g_.copy()
         alpha = {}
-        slots = [((self.head - k) % self.m + self.m) % self.m for k in range(self.count)]
+        slots = [(self.head - k) % (self.m + 1) for k in range(self.count)]
         for s in slots:
             alpha[s] = self.rho[s] * self._bdot(self.S[s], q)
             q = q - alpha[s] * self.Y[s]
@@ -214,6 +213,10 @@ class NumpyWorkspace:
 
     def download(self):
         return self.x_.copy(), self.g_.copy()
+
+    def download_vector(self, name):
+        self._mat()
+        return {"x": self.x_, "df_x": self.g_, "u": self.u_, "xp": self.xp_, "df_xp": self.gp_}[name].copy()
 
     def close(self):
         pass
