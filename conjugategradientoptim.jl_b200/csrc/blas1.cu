@@ -259,28 +259,20 @@ struct AxpyDir {
     }
 };
 
-// Sample-sharded logistic regression (multi-rank): every rank's Aᵀ_r c_r partial gradient slice
-// of this rank's feature shard sits in q[r·stride ..]; add them in rank order, scale, add the
-// regulariser, and reduce the same eight dots as the single-rank SpMVᵀ epilogue (csr.cu EpiGrad).
+// Logistic regression on k_spmv_direct (csr.cu): the passes of Aᵀ left s = Aᵀc in gp; scale it, add the
+// regulariser in place, and reduce the same eight dots as the fused SpMVᵀ epilogue (csr.cu EpiGrad).
 struct GradCombine {
     static constexpr int TCLASS = CGO_T_OTHER;
     static constexpr int K = 8;
     static constexpr int OCC = 2;
     struct In { double2 s, u, g, w; };
-    const double2 *q, *u, *g, *w;
+    const double2 *u, *g, *w;
     double2 *gp;
-    int nparts;
-    int64_t stride2;            // part stride in double2 units
     double invN, lambda;
     __device__ __forceinline__ void prologue() {}
     __device__ __forceinline__ In load(int64_t i) const {
         In r;
-        r.s = ld2rw(q + i);          // coherent loads: peers deliver q while this kernel waits for their flags
-        for (int p = 1; p < nparts; ++p) {
-            const double2 t = ld2rw(q + (int64_t)p * stride2 + i);
-            r.s.x = r.s.x + t.x;
-            r.s.y = r.s.y + t.y;
-        }
+        r.s = ld2rw(gp + i);
         r.u = cgo_ld2(u + i); r.g = cgo_ld2(g + i); r.w = cgo_ld2(w + i);
         return r;
     }
@@ -368,7 +360,7 @@ struct GradDots {
 
 // logistic loss and its derivative from the margins (csr.cu EpiLogit, oracle logreg_fdf), in place: z → c = −y σ;
 // Σ ℓ.  PUSH: this rank's shard of c also goes into every rank's all-gathered copy (peer memory), then flag
-// CGO_F_GPART + me of every rank
+// CGO_F_CALL + me of every rank
 template <bool PUSH>
 struct LogitLoss {
     static constexpr int TCLASS = CGO_T_OTHER;
@@ -1170,7 +1162,7 @@ int cgo_blas1_logit(cgo_ctx *c, double *zc, const double *y, int64_t n, int slot
     if (dst_all) {
         LogitLoss<true> op;
         op.zc = (double2 *)zc; op.y = (const double2 *)y; op.dst_all = dst_all; op.nranks = c->nranks;
-        red.flags_all = c->d_flags_peer; red.sig_all_slot = CGO_F_GPART; red.nranks = c->nranks; red.me = c->rank;
+        red.flags_all = c->d_flags_peer; red.sig_all_slot = CGO_F_CALL; red.nranks = c->nranks; red.me = c->rank;
         red.sig_val = epoch;
         return launch_blas1(c, op, n, red);
     }
@@ -1184,17 +1176,12 @@ int cgo_blas1_grad_dots(cgo_state *st) {
     return launch_blas1(st->ctx, op, st->n, cgo_red_args(st->ctx, CGO_P_DPHI));
 }
 
-int cgo_blas1_grad_combine(cgo_state *st, const double *q, int nparts, int64_t stride, double invN, double lambda,
-                           unsigned long long wait_epoch) {
+int cgo_blas1_grad_combine(cgo_state *st, double invN, double lambda) {
     GradCombine op;
-    op.q = (const double2 *)q; op.u = (const double2 *)st->u; op.g = (const double2 *)st->g;
+    op.u = (const double2 *)st->u; op.g = (const double2 *)st->g;
     op.w = (const double2 *)st->xp; op.gp = (double2 *)st->gp;
-    op.nparts = nparts; op.stride2 = stride / 2; op.invN = invN; op.lambda = lambda;
-    RedArgs red = cgo_red_args(st->ctx, CGO_P_DPHI);
-    if (wait_epoch) {
-        red.wait_all = st->ctx->flags_local + CGO_F_GPART; red.wait_val = wait_epoch; red.nranks = st->ctx->nranks;
-    }
-    return launch_blas1(st->ctx, op, st->n, red);
+    op.invN = invN; op.lambda = lambda;
+    return launch_blas1(st->ctx, op, st->n, cgo_red_args(st->ctx, CGO_P_DPHI));
 }
 
 // ------------------------------------------------------------------ solvesystem (solve_system.jl)

@@ -85,9 +85,7 @@ extern "C" int cgo_ctx_create(int device, void *cuda_stream, cgo_ctx **out) {
     cudaDeviceProp prop;
     CGO_CUDA(cudaGetDeviceProperties(&prop, device));
     c->sms = prop.multiProcessorCount;
-    if (const char *e = getenv("CGO_CSR_PASS_OCC")) c->csr_pass_occ = (e[0] == '3') ? 3 : 2;
     if (const char *e = getenv("CGO_CSR_MODE")) c->csr_mode = atoi(e);
-    if (const char *e = getenv("CGO_DIRECT_CFG")) c->direct_cfg = atoi(e);
     if (cuda_stream) {
         c->stream = (cudaStream_t)cuda_stream;
     } else {
@@ -368,15 +366,6 @@ extern "C" int cgo_shard_range(int64_t n, int nranks, int rank, int64_t align, i
     return 0;
 }
 
-int cgo_allgather_bytes(cgo_ctx *c, const void *send, void *recv, size_t bytes) {
-    if (c->nranks == 1) {
-        CGO_CUDA(cudaMemcpyAsync(recv, send, bytes, cudaMemcpyDeviceToDevice, c->stream));
-        return 0;
-    }
-    CGO_NCCL(g_nccl.AllGather(send, recv, bytes, ncclInt8, (ncclComm_t)c->comm, c->stream));
-    return 0;
-}
-
 // ring halo exchange: my head goes to the previous rank (its right halo), my tail to the next
 // rank (its left halo)
 int cgo_sendrecv_ring(cgo_ctx *c, const double *send_to_prev, double *recv_from_next,
@@ -413,25 +402,6 @@ int cgo_allgatherv_f64(cgo_ctx *c, const double *mine, double *full, const int64
         if (cnt > 0) CGO_NCCL(g_nccl.Send(mine, (size_t)cnt, ncclFloat64, to, comm, c->stream));
         if (lo[from + 1] > lo[from])
             CGO_NCCL(g_nccl.Recv(full + lo[from], (size_t)(lo[from + 1] - lo[from]), ncclFloat64, from, comm, c->stream));
-    }
-    CGO_NCCL(g_nccl.GroupEnd());
-    return 0;
-}
-// all-to-all of shard slices: slice [lo[s], lo[s+1]) of `full` goes to rank s; the slice of MY
-// shard computed by rank s lands in recv + s * stride.
-int cgo_alltoallv_f64(cgo_ctx *c, const double *full, const int64_t *lo, double *recv, int64_t stride) {
-    const int R = c->nranks, me = c->rank;
-    const int64_t cnt = lo[me + 1] - lo[me];
-    if (cnt > 0)
-        CGO_CUDA(cudaMemcpyAsync(recv + (size_t)me * stride, full + lo[me], sizeof(double) * (size_t)cnt, cudaMemcpyDeviceToDevice, c->stream));
-    if (R == 1) return 0;
-    ncclComm_t comm = (ncclComm_t)c->comm;
-    CGO_NCCL(g_nccl.GroupStart());
-    for (int k = 1; k < R; ++k) {
-        const int to = (me + k) % R, from = (me + R - k) % R;
-        if (lo[to + 1] > lo[to])
-            CGO_NCCL(g_nccl.Send(full + lo[to], (size_t)(lo[to + 1] - lo[to]), ncclFloat64, to, comm, c->stream));
-        if (cnt > 0) CGO_NCCL(g_nccl.Recv(recv + (size_t)from * stride, (size_t)cnt, ncclFloat64, from, comm, c->stream));
     }
     CGO_NCCL(g_nccl.GroupEnd());
     return 0;

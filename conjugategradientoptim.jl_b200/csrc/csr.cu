@@ -5,10 +5,13 @@
 // large objective, SURVEY.md §0-3; the definitions are restated in oracle/cgo_oracle.c
 // sparse_ls_fdf / logreg_fdf).  One trial  evalϕdϕ! (src/cg_utils.jl:3-22)  is three kernels:
 //   K_a  xp = x + a u  [after u = −g + βu, cg_flavours.jl:10-12]           BLAS-1, blas1.cu
-//   K_b  r  = A xp − b,  Σ r²                (logreg: margins, loss, c)     k_csr_rows
-//   K_c  g⁺ = Aᵀ r  + every dot of getβ / norm(df_xp) / dϕ                  k_csr_rows on Aᵀ
+//   K_b  r  = A xp − b,  Σ r²                (logreg: margins, loss, c)     SpMV with A
+//   K_c  g⁺ = Aᵀ r  + every dot of getβ / norm(df_xp) / dϕ                  SpMV with Aᵀ
 // Aᵀ is an explicit CSR whose rows are sorted by source entry, so the gradient is a gather
 // (no atomics on data) and reproduces the sequential scatter order of the oracle bit for bit.
+// An objective runs every SpMV on one of two kernel families, chosen at creation (CsrObj::direct):
+// the fused k_csr_rows, whose row epilogues reduce the dots, or — for matrices whose gathers do not
+// coalesce — k_spmv_direct, which keeps no reduction, followed by BLAS-1 dot passes.
 //
 // k_csr_rows is a "CSR-stream" kernel: a CTA owns 256 consecutive rows at a time; their
 // nonzeros are one contiguous range of val/col, which a producer warp streams into a circular
@@ -92,11 +95,9 @@ constexpr int TS_THREADS = CGO_B + 32;
 constexpr int TS_OCC = 2;
 constexpr int TS_UN = 10;                   // gathers in flight per lane
 constexpr int TS_SMEM_BUDGET = 115200;      // two CTAs per SM (228 KB - 2 x 1 KB reserved)
-// OCC CTAs per SM: 2 for the streaming-bound kernels (a ring of ~3 tiles of 10 entries per row);
-// 3 for the short rows of a column-block pass, which are gather-latency bound and want more warps
-template <int NOPS, int OCC = TS_OCC>
+template <int NOPS>
 struct TsLayout {
-    static constexpr int BUDGET = OCC == 2 ? TS_SMEM_BUDGET : (228 * 1024) / OCC - 1024 - 256;
+    static constexpr int BUDGET = TS_SMEM_BUDGET;
     static constexpr int RP_BYTES = (CGO_B + 2) * 8;
     static constexpr int OP_BYTES = CGO_B * 8;
     static constexpr int DESC_BYTES = RP_BYTES + NOPS * OP_BYTES;
@@ -134,8 +135,7 @@ __device__ __forceinline__ double ld_gather_f64(const double *p, uint64_t pol) {
 }
 // predicated gather: a lane whose row has ended issues no request at all.  (A gather instruction
 // costs one L1TEX wavefront per distinct 128-byte line; re-reading a dummy address on the idle
-// lanes — the first version — spent half of the gather bandwidth of the 5-entry rows of a
-// column-block pass on nothing.)
+// lanes — the first version — spent half of the gather bandwidth of 5-entry rows on nothing.)
 __device__ __forceinline__ double ld_gather_f64_if(const double *p, uint64_t pol, bool on) {
     double r = 0.0;
     asm volatile(
@@ -212,12 +212,12 @@ __device__ __forceinline__ void ts_produce(const CsrMat &A, const Epi &epi, cons
     }
 }
 
-template <class Epi, int OCC>
-__global__ void __launch_bounds__(TS_THREADS, OCC)
+template <class Epi>
+__global__ void __launch_bounds__(TS_THREADS, TS_OCC)
 k_csr_rows(CsrMat A, const double *__restrict__ xg, Epi epi, RedArgs red) {
     constexpr int K = Epi::K;
     constexpr int NOPS = Epi::NOPS;
-    using L = TsLayout<NOPS, OCC>;
+    using L = TsLayout<NOPS>;
     constexpr int RING = L::RING, CHMAX = L::CHMAX;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double *s_val = reinterpret_cast<double *>(smem_raw + L::OFF_VAL);
@@ -269,7 +269,6 @@ k_csr_rows(CsrMat A, const double *__restrict__ xg, Epi epi, RedArgs red) {
                     if (valid) {
                         rs = rp[tid]; re = rp[tid + 1];
                         pre = epi.load(reinterpret_cast<const double *>(desc + L::RP_BYTES), tid);
-                        if (Epi::HAS_INIT) sum = epi.init(pre);     // column-blocked pass: continue the row sum
                     }
                     p0 = rp[0];
                     p1 = rp[nvalid];
@@ -313,32 +312,22 @@ k_csr_rows(CsrMat A, const double *__restrict__ xg, Epi epi, RedArgs red) {
     cgo_grid_finish<K, BarLanes>(red, nact, s_red, bar);
 }
 
-template <class Epi, int OCC>
-static int launch_csr_occ(cgo_ctx *c, const CsrMat &A, const double *xg, const Epi &epi, const RedArgs &red, int tclass) {
+template <class Epi>
+static int launch_csr(cgo_ctx *c, const CsrMat &A, const double *xg, const Epi &epi, const RedArgs &red, int tclass) {
     const int64_t ntiles = (A.nrows + CGO_B - 1) / CGO_B;
     int64_t nact = ntiles < red.G ? ntiles : red.G;
-    int64_t phys = (int64_t)c->sms * OCC;
+    int64_t phys = (int64_t)c->sms * TS_OCC;
     int grid = (int)(nact < phys ? nact : phys);
     if (grid < 1) grid = 1;
     CGO_CHECK(!A.sliced, "internal: k_csr_rows on a matrix in the sliced layout");
-    const size_t smem = TsLayout<Epi::NOPS, OCC>::BYTES;
-    CGO_CUDA(cudaFuncSetAttribute(k_csr_rows<Epi, OCC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = TsLayout<Epi::NOPS>::BYTES;
+    CGO_CUDA(cudaFuncSetAttribute(k_csr_rows<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cgo_timer_begin(c, tclass);
-    k_csr_rows<Epi, OCC><<<grid, TS_THREADS, smem, c->stream>>>(A, xg, epi, red);
+    k_csr_rows<Epi><<<grid, TS_THREADS, smem, c->stream>>>(A, xg, epi, red);
     cgo_timer_end(c);
     c->launches++;
     CGO_CUDA(cudaGetLastError());
     return 0;
-}
-template <class Epi>
-static int launch_csr(cgo_ctx *c, const CsrMat &A, const double *xg, const Epi &epi, const RedArgs &red, int tclass) {
-    return launch_csr_occ<Epi, TS_OCC>(c, A, xg, epi, red, tclass);
-}
-// a column-block pass: short rows, gather-latency bound
-template <class Epi>
-static int launch_csr_pass(cgo_ctx *c, const CsrMat &A, const double *xg, const Epi &epi, const RedArgs &red, int tclass) {
-    if (c->csr_pass_occ == 3) return launch_csr_occ<Epi, 3>(c, A, xg, epi, red, tclass);
-    return launch_csr_occ<Epi, TS_OCC>(c, A, xg, epi, red, tclass);
 }
 
 // ------------------------------------------------------------------ row epilogues
@@ -348,9 +337,7 @@ static int launch_csr_pass(cgo_ctx *c, const CsrMat &A, const double *xg, const 
 // row sum is known.
 struct EpiStore {                       // y = A x
     static constexpr int K = 1, NOPS = 0;
-    static constexpr bool HAS_INIT = false;
     struct Pre {};
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     double *y;
     __device__ __forceinline__ const double *operand(int) const { return nullptr; }
     __device__ __forceinline__ Pre load(const double *, int) const { return Pre(); }
@@ -361,9 +348,7 @@ struct EpiStore {                       // y = A x
 template <bool PUSH>
 struct EpiResidualT {
     static constexpr int K = 1, NOPS = 1;
-    static constexpr bool HAS_INIT = false;
     struct Pre { double b; };
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     const double *b;
     double *r;
     double *prev_right, *next_left;      // PUSH
@@ -385,9 +370,7 @@ struct EpiResidualT {
 template <bool LOGREG>
 struct EpiGrad {
     static constexpr int K = 8, NOPS = LOGREG ? 3 : 2;
-    static constexpr bool HAS_INIT = false;
     struct Pre { double u, g, w; };
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     double *gp;
     const double *g, *u, *w;
     double invN, lambda;
@@ -418,9 +401,7 @@ struct EpiGrad {
 //   t = −y z; e = exp(−|t|); ℓ = max(t,0) + log1p(e); σ = t ≥ 0 ? 1/(1+e) : e/(1+e); c = −y σ
 struct EpiLogit {
     static constexpr int K = 1, NOPS = 1;
-    static constexpr bool HAS_INIT = false;
     struct Pre { double y; };
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     const double *label;
     double *c;
     __device__ __forceinline__ const double *operand(int) const { return label; }
@@ -440,9 +421,7 @@ struct EpiLogit {
 // hv = Aᵀ v with u·hv and hv·hv
 struct EpiStoreSq {
     static constexpr int K = 1, NOPS = 0;
-    static constexpr bool HAS_INIT = false;
     struct Pre {};
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     double *y;
     __device__ __forceinline__ const double *operand(int) const { return nullptr; }
     __device__ __forceinline__ Pre load(const double *, int) const { return Pre(); }
@@ -453,9 +432,7 @@ struct EpiStoreSq {
 };
 struct EpiHv {
     static constexpr int K = 2, NOPS = 1;
-    static constexpr bool HAS_INIT = false;
     struct Pre { double u; };
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     double *hv;
     const double *u;
     __device__ __forceinline__ const double *operand(int) const { return u; }
@@ -470,9 +447,7 @@ struct EpiHv {
 // quadratic-aware line search: v = A u with r·v, v·v and r·r (r = residual at x)
 struct EpiQuadV {
     static constexpr int K = 3, NOPS = 1;
-    static constexpr bool HAS_INIT = false;
     struct Pre { double r; };
-    __device__ __forceinline__ double init(const Pre &) const { return 0.0; }
     double *v;
     const double *r;
     __device__ __forceinline__ const double *operand(int) const { return r; }
@@ -484,35 +459,6 @@ struct EpiQuadV {
         acc[2] = acc[2] + p.r * p.r;
     }
 };
-
-// Column-blocked matrices (CsrBlocked below): pass j > 0 of a row continues the sum pass j − 1
-// left in `partial` (one more staged operand), so the products of a row are still added one by one
-// in storage order — bit-identical to the single-pass kernel.
-template <class Base>
-struct WithInit : Base {
-    static constexpr int K = Base::K, NOPS = Base::NOPS + 1;
-    static constexpr bool HAS_INIT = true;
-    struct Pre { typename Base::Pre base; double init; };
-    const double *partial;
-    __device__ __forceinline__ const double *operand(int o) const { return o < Base::NOPS ? Base::operand(o) : partial; }
-    __device__ __forceinline__ Pre load(const double *ops, int t) const {
-        Pre p;
-        p.base = Base::load(ops, t);
-        p.init = ops[Base::NOPS * CGO_B + t];
-        return p;
-    }
-    __device__ __forceinline__ double init(const Pre &p) const { return p.init; }
-    __device__ __forceinline__ void row(int64_t i, double sum, const Pre &p, double (&acc)[K]) const {
-        Base::row(i, sum, p.base, acc);
-    }
-};
-template <class Base>
-static WithInit<Base> with_init(const Base &b, const double *partial) {
-    WithInit<Base> w;
-    static_cast<Base &>(w) = b;
-    w.partial = partial;
-    return w;
-}
 
 // ------------------------------------------------------------------ the gather-bound SpMV kernel
 // Matrices whose gathers do not coalesce — every lane of a warp-level gather touches its own 128-byte line: the
@@ -713,9 +659,7 @@ static int launch_direct(cgo_ctx *c, const CsrMat &A, const double *xg, const F 
     // ragged rows of Aᵀ, ms; profiles/r2_exp_coh0_n2e8_k_spmv_direct_configs.txt): 10 × 4: 7.5–7.9 / 9.3–10.5;
     // 8 × 4: 8.0 / 9.1; 6 × 5: 7.7–8.1 / 9.1; 5 × 4: 7.7 / 9.3; 8 × 5 (spills): 8.4 / 9.5; 10 × 3: 7.9 / 10.5.
     // Ragged slices waste the tail of a wide batch, equal-length rows like the widest batch that does not spill.
-    const int cfg = c->direct_cfg ? c->direct_cfg : (A.ragged ? 3 : 2);
-    if (cfg == 1) return launch_direct_k<F, 8, 4>(c, A, xg, f, da, tclass);
-    if (cfg == 3) return launch_direct_k<F, 6, 5>(c, A, xg, f, da, tclass);
+    if (A.ragged) return launch_direct_k<F, 6, 5>(c, A, xg, f, da, tclass);
     return launch_direct_k<F, 10, 4>(c, A, xg, f, da, tclass);
 }
 
@@ -1106,8 +1050,8 @@ static int build_transpose(cgo_ctx *c, const Src &src, const Fin &fin, int64_t n
 // such matrices the columns are cut into nb blocks of at most ctx->gather_block_bytes and the
 // matrix is stored block-major: blk[j] holds the entries of every row whose column lies in block
 // j (rows' columns must ascend, which both logistic-regression matrices do by construction).  One
-// pass per block keeps its window of the gathered vector L2-resident; passes chain the row sums
-// (WithInit), so the arithmetic order is unchanged.
+// k_spmv_direct pass per block keeps its window of the gathered vector L2-resident; passes chain the
+// row sums (DirStoreInit), so the arithmetic order is unchanged.
 struct CsrBlocked {
     std::vector<CsrMat> blk;
     void free_all() { for (auto &m : blk) csr_free(m); blk.clear(); }
@@ -1187,29 +1131,9 @@ static int build_blocked(cgo_ctx *c, const CsrMat &A, int64_t ncols, CsrBlocked 
     if (rc) out.free_all();
     return rc;
 }
-// one pass per column block; the last pass runs the real epilogue
-// (`wait_first`: red's flag wait guards the gathered vector, so the FIRST pass has to honour it)
-template <class Epi>
-static int launch_csr_blocked(cgo_ctx *c, const CsrMat &A, const CsrBlocked &B, const double *xg, const Epi &epi,
-                              double *partial, const RedArgs &red, int tclass, bool wait_first = false) {
-    if (B.blk.empty()) return launch_csr(c, A, xg, epi, red, tclass);
-    const size_t nb = B.blk.size();
-    RedArgs scratch = cgo_red_args(c, CGO_PACK_LEN - 1);
-    if (c->csr_pass_occ == 3) scratch.G = c->sms * 3;     // nothing is reduced in these passes: any sweep order will do
-    if (wait_first) {
-        scratch.wait0 = red.wait0; scratch.wait1 = red.wait1; scratch.wait_all = red.wait_all;
-        scratch.wait_val = red.wait_val; scratch.nranks = red.nranks;
-    }
-    for (size_t j = 0; j + 1 < nb; ++j) {
-        EpiStore es{partial};
-        if (j == 0) CGO_TRY(launch_csr_pass(c, B.blk[j], xg, es, scratch, tclass));
-        else CGO_TRY(launch_csr_pass(c, B.blk[j], xg, with_init(es, partial), scratch, tclass));
-    }
-    return launch_csr_pass(c, B.blk[nb - 1], xg, with_init(epi, partial), red, tclass);
-}
-
-// the same with k_spmv_direct (sliced blocks): every pass just stores the running row sums, the epilogue and its
-// reductions are a BLAS-1 kernel of the caller's.  `wait`: flag hand-off that guards the gathered vector (first pass)
+// one k_spmv_direct pass per column block (sliced blocks): every pass just stores the running row sums, the
+// epilogue and its reductions are a BLAS-1 kernel of the caller's.  `wait`: flag hand-off that guards the gathered
+// vector (first pass)
 static int spmv_direct_passes(cgo_ctx *c, const CsrMat &M, const CsrBlocked &B, const double *xg, double *out,
                               const RedArgs *wait, int tclass) {
     if (B.blk.empty()) return launch_direct(c, M, xg, DirStore{out}, dir_args(c, wait), tclass);
@@ -1223,8 +1147,13 @@ static int spmv_direct_passes(cgo_ctx *c, const CsrMat &M, const CsrBlocked &B, 
 // ------------------------------------------------------------------ the objective
 struct CsrObj : cgo_obj {
     bool logreg = false;
+    // the SpMV kernel family of every evaluation, fixed at creation.  false: the fused k_csr_rows, whose epilogues
+    // reduce the dots (reduction site V = 1, U = 1).  true: k_spmv_direct on the sliced layout, the dots are
+    // BLAS-1 passes (V = 2, U = CGO_U_VEC).  Least squares: A.sliced after set-up; logistic regression: also when
+    // column-blocked or sharded.
+    bool direct = false;
     CsrMat A, AT;
-    CsrBlocked Ab, ATb;                // column-blocked copies (logreg, large gather ranges)
+    CsrBlocked Ab, ATb;                // column-blocked copies (logreg on k_spmv_direct, large gather ranges)
     bool have_unblocked = true;        // A / AT arrays still allocated (test hooks need them)
     int64_t nrows = 0;                 // local rows of A (residuals / samples)
     double *b = nullptr;               // rhs (LS) or labels (logreg), nrows
@@ -1244,7 +1173,6 @@ struct CsrObj : cgo_obj {
     // straight from the generator) and gathers the all-gathered c, so every row of Aᵀc is added over all samples in
     // the single-GPU order.  The state vectors are feature shards [flo[rank], flo[rank+1]).
     bool lr_sharded = false;
-    bool lr_direct = false;            // k_spmv_direct passes + BLAS-1 epilogues (sliced matrices)
     std::vector<int64_t> flo, slo;     // feature / sample shard boundaries, nranks + 1
     double *xp_full = nullptr;         // all-gathered trial point, n_global
     double *c_full = nullptr;          // all-gathered c = −y σ, nsamples
@@ -1287,124 +1215,98 @@ struct CsrObj : cgo_obj {
         cgo_shard_range(n_global, ctx->nranks, q, 2, &lo, &hi);
         return hi - lo;
     }
-    // sharded least squares over peer memory: K_a and K_b push their boundary elements into the
-    // neighbours' halos and hand off with flags; no separate exchange step
-    int eval_trial_ls_peer(cgo_state *st, double a, bool fused, double beta, double *out) {
-        const int R = ctx->nranks, me = ctx->rank, prev = (me + R - 1) % R, next = (me + 1) % R;
-        const unsigned long long e = ++ctx->epoch;
-        unsigned long long *fprev = (unsigned long long *)ctx->flags_peer[(size_t)prev];
-        unsigned long long *fnext = (unsigned long long *)ctx->flags_peer[(size_t)next];
-        const int64_t nprev = shard_len_of(prev);
-        HaloPush hp;
-        double *xp_prev = (double *)st->xpeers[st->xp_alloc][(size_t)prev] + halo;   // origin of prev's xp
-        double *xp_next = (double *)st->xpeers[st->xp_alloc][(size_t)next] + halo;
-        hp.prev_right = xp_prev + nprev;
-        hp.next_left = xp_next - halo;
-        hp.sig_prev = fprev + CGO_F_XP_FROM_NEXT;       // I am prev's next
-        hp.sig_next = fnext + CGO_F_XP_FROM_PREV;
-        hp.epoch = e;
-        CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta, &hp));                          // K_a + halo push
-        EpiResidualT<true> e1;
-        e1.b = b; e1.r = r; e1.halo = halo; e1.nrows = nrows;
-        e1.prev_right = (double *)rpeers[(size_t)prev] + halo + nprev;
-        e1.next_left = (double *)rpeers[(size_t)next];
-        RedArgs rb = cgo_red_args(ctx, CGO_P_PHI);
-        rb.wait0 = ctx->flags_local + CGO_F_XP_FROM_PREV; rb.wait1 = ctx->flags_local + CGO_F_XP_FROM_NEXT; rb.wait_val = e;
-        rb.sig0 = fprev + CGO_F_R_FROM_NEXT; rb.sig1 = fnext + CGO_F_R_FROM_PREV; rb.sig_val = e;
-        CGO_TRY(launch_csr(ctx, A, st->xp, e1, rb, CGO_T_SPMV));                       // K_b + halo push
-        EpiGrad<false> e2{st->gp, st->g, st->u, nullptr, 0.0, 0.0};
-        RedArgs rc = cgo_red_args(ctx, CGO_P_DPHI);
-        rc.wait0 = ctx->flags_local + CGO_F_R_FROM_PREV; rc.wait1 = ctx->flags_local + CGO_F_R_FROM_NEXT; rc.wait_val = e;
-        CGO_TRY(launch_csr(ctx, AT, r, e2, rc, CGO_T_SPMVT));                          // K_c
-        CGO_TRY(cgo_finish_pack(ctx, 12, out));
-        out[CGO_P_PHI] = 0.5 * out[CGO_P_PHI];
-        return 0;
-    }
     // fill v[−halo, 0) and v[nloc, nloc + halo) from the ring neighbours
     int exchange(double *v, int64_t nloc) {
         if (halo == 0) return 0;
         return cgo_sendrecv_ring(ctx, v, v + nloc, v + nloc - halo, v - halo, halo);
     }
-    // ∇²f u = Aᵀ(A u) along the current direction (north_star's Hessian-vector product; the reference
-    // engine never calls one, src/engine/optim.jl:83-145).  `r` is scratch between trials.
-    // ---- gather-bound matrices (sliced layout): k_spmv_direct + the dots as BLAS-1 passes
-    bool direct() const { return A.sliced != 0; }
     void reduction_site(int32_t *V, int32_t *U) const override {
-        if (direct() || lr_direct) { *V = 2; *U = CGO_U_VEC; } else { *V = 1; *U = 1; }
+        if (direct) { *V = 2; *U = CGO_U_VEC; } else { *V = 1; *U = 1; }
     }
-    // logistic regression through k_spmv_direct.  One rank: K_a | passes of A → margins | logit + loss (BLAS-1) |
-    // passes of Aᵀ | /N + λw + dots (BLAS-1).  R ranks: K_a also stores its shard of xp into every rank's
-    // all-gathered copy; the logit kernel stores its shard of c into every rank's all-gathered c; flags hand the
-    // data to the consuming passes (without peer memory: two NCCL all-gathers).
-    int eval_trial_lr_direct(cgo_state *st, double a, bool fused, double beta, double *out) {
-        const int R = ctx->nranks;
-        const double invN = 1.0 / (double)nsamples;
-        RedArgs wx, wc;                           // flag waits of the first K_b / K_c pass
-        const RedArgs *pwx = nullptr, *pwc = nullptr;
-        unsigned long long e = 0;
-        if (R > 1 && lr_peer) {
-            e = ++ctx->epoch;
-            HaloPush hp;
-            hp.dst_all = d_xpf_dst; hp.epoch = e;
-            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta, &hp));                     // K_a + all-gather of xp
-            wx.wait_all = ctx->flags_local + CGO_F_XPALL; wx.wait_val = e; wx.nranks = R; pwx = &wx;
-            wc.wait_all = ctx->flags_local + CGO_F_GPART; wc.wait_val = e; wc.nranks = R; pwc = &wc;
-        } else {
-            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                          // K_a
-            if (R > 1) CGO_TRY(cgo_allgatherv_f64(ctx, st->xp, xp_full, flo.data()));
-        }
-        const double *w_all = R > 1 ? xp_full : st->xp;
-        CGO_TRY(spmv_direct_passes(ctx, A, Ab, w_all, r, pwx, CGO_T_SPMV));            // K_b: margins of my samples
-        CGO_TRY(cgo_blas1_logit(ctx, r, b, nrows, CGO_P_PHI, (R > 1 && lr_peer) ? d_cf_dst : nullptr, e));   // c, Σ loss [+ all-gather of c]
-        if (R > 1 && !lr_peer) CGO_TRY(cgo_allgatherv_f64(ctx, r, c_full, slo.data()));
-        const double *c_all = R > 1 ? c_full : r;
-        CGO_TRY(spmv_direct_passes(ctx, AT, ATb, c_all, st->gp, pwc, CGO_T_SPMVT));    // K_c: Aᵀc over my features
-        CGO_TRY(cgo_blas1_grad_combine(st, st->gp, 1, 0, invN, lambda));               // /N + λw, dots
-        CGO_TRY(cgo_finish_pack(ctx, 12, out));
-        out[CGO_P_PHI] = out[CGO_P_PHI] / (double)nsamples + (0.5 * lambda) * out[CGO_P_XPXP];
-        return 0;
+
+    // ---- least squares: one trial = K_a, K_b (residual), K_c (gradient), on either kernel family
+    // sharded least squares over peer memory: K_a and K_b push their boundary elements into the ring neighbours'
+    // halos and hand off with flags; there is no separate exchange step
+    struct PeerLinks {
+        HaloPush xp;                            // K_a: xp's boundary elements, flags CGO_F_XP_FROM_*
+        double *r_prev_right, *r_next_left;     // K_b: where r's boundary elements go
+        RedArgs kb, kc;                         // K_b: waits for xp's halos, signals r's; K_c: waits for r's
+    };
+    PeerLinks peer_links(cgo_state *st) {
+        const int R = ctx->nranks, me = ctx->rank, prev = (me + R - 1) % R, next = (me + 1) % R;
+        const unsigned long long e = ++ctx->epoch;
+        unsigned long long *fprev = (unsigned long long *)ctx->flags_peer[(size_t)prev];
+        unsigned long long *fnext = (unsigned long long *)ctx->flags_peer[(size_t)next];
+        const int64_t nprev = shard_len_of(prev);
+        PeerLinks pl;
+        pl.xp.prev_right = (double *)st->xpeers[st->xp_alloc][(size_t)prev] + halo + nprev;   // prev's xp + its n
+        pl.xp.next_left = (double *)st->xpeers[st->xp_alloc][(size_t)next];                    // next's xp − halo
+        pl.xp.sig_prev = fprev + CGO_F_XP_FROM_NEXT;                                           // I am prev's next
+        pl.xp.sig_next = fnext + CGO_F_XP_FROM_PREV;
+        pl.xp.epoch = e;
+        pl.r_prev_right = (double *)rpeers[(size_t)prev] + halo + nprev;
+        pl.r_next_left = (double *)rpeers[(size_t)next];
+        pl.kb = cgo_red_args(ctx, CGO_P_PHI);
+        pl.kb.wait0 = ctx->flags_local + CGO_F_XP_FROM_PREV; pl.kb.wait1 = ctx->flags_local + CGO_F_XP_FROM_NEXT;
+        pl.kb.wait_val = e;
+        pl.kb.sig0 = fprev + CGO_F_R_FROM_NEXT; pl.kb.sig1 = fnext + CGO_F_R_FROM_PREV; pl.kb.sig_val = e;
+        pl.kc = cgo_red_args(ctx, CGO_P_DPHI);
+        pl.kc.wait0 = ctx->flags_local + CGO_F_R_FROM_PREV; pl.kc.wait1 = ctx->flags_local + CGO_F_R_FROM_NEXT;
+        pl.kc.wait_val = e;
+        return pl;
     }
-    int eval_trial_ls_direct(cgo_state *st, double a, bool fused, double beta, double *out) {
-        const bool peer = r_is_peer && st->peer_x;
-        RedArgs fb, fc;                                                                   // flag hand-offs only
-        if (peer) {
-            const int R = ctx->nranks, me = ctx->rank, prev = (me + R - 1) % R, next = (me + 1) % R;
-            const unsigned long long e = ++ctx->epoch;
-            unsigned long long *fprev = (unsigned long long *)ctx->flags_peer[(size_t)prev];
-            unsigned long long *fnext = (unsigned long long *)ctx->flags_peer[(size_t)next];
-            const int64_t nprev = shard_len_of(prev);
-            HaloPush hp;
-            hp.prev_right = (double *)st->xpeers[st->xp_alloc][(size_t)prev] + halo + nprev;
-            hp.next_left = (double *)st->xpeers[st->xp_alloc][(size_t)next];
-            hp.sig_prev = fprev + CGO_F_XP_FROM_NEXT;
-            hp.sig_next = fnext + CGO_F_XP_FROM_PREV;
-            hp.epoch = e;
-            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta, &hp));                         // K_a + halo push
-            DirResidual<true> f1{b, r, (double *)rpeers[(size_t)prev] + halo + nprev, (double *)rpeers[(size_t)next], halo, nrows};
-            fb.wait0 = ctx->flags_local + CGO_F_XP_FROM_PREV; fb.wait1 = ctx->flags_local + CGO_F_XP_FROM_NEXT; fb.wait_val = e;
-            fb.sig0 = fprev + CGO_F_R_FROM_NEXT; fb.sig1 = fnext + CGO_F_R_FROM_PREV; fb.sig_val = e;
-            CGO_TRY(launch_direct(ctx, A, st->xp, f1, dir_args(ctx, &fb), CGO_T_SPMV));    // K_b + halo push
-            fc.wait0 = ctx->flags_local + CGO_F_R_FROM_PREV; fc.wait1 = ctx->flags_local + CGO_F_R_FROM_NEXT; fc.wait_val = e;
-        } else {
-            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                              // K_a
-            CGO_TRY(exchange(st->xp, st->n));
-            DirResidual<false> f1{b, r, nullptr, nullptr, 0, nrows};
-            CGO_TRY(launch_direct(ctx, A, st->xp, f1, dir_args(ctx), CGO_T_SPMV));         // K_b
+    // K_b: r = A x − b, and Σ r² into pack slot CGO_P_PHI when `sumsq` (without it, k_csr_rows still reduces, into
+    // the scratch slot; k_spmv_direct runs no BLAS-1 pass).  pl: also push r's boundary elements to the neighbours
+    int residual(const double *x, bool sumsq, const PeerLinks *pl) {
+        if (direct) {
+            if (pl) {
+                DirResidual<true> f{b, r, pl->r_prev_right, pl->r_next_left, halo, nrows};
+                CGO_TRY(launch_direct(ctx, A, x, f, dir_args(ctx, &pl->kb), CGO_T_SPMV));
+            } else {
+                CGO_TRY(launch_direct(ctx, A, x, DirResidual<false>{b, r, nullptr, nullptr, 0, nrows}, dir_args(ctx), CGO_T_SPMV));
+            }
+            return sumsq ? cgo_blas1_sumsq(ctx, r, nrows, CGO_P_PHI) : 0;
         }
-        CGO_TRY(cgo_blas1_sumsq(ctx, r, nrows, CGO_P_PHI));                               // Σ r²
-        if (!peer) CGO_TRY(exchange(r, nrows));
-        DirGradLS f2{st->gp};
-        CGO_TRY(launch_direct(ctx, AT, r, f2, peer ? dir_args(ctx, &fc) : dir_args(ctx), CGO_T_SPMVT));   // K_c
-        CGO_TRY(cgo_blas1_grad_dots(st));                                                 // dϕ, ‖g⁺‖², getβ dots
+        if (pl) {
+            EpiResidualT<true> e{b, r, pl->r_prev_right, pl->r_next_left, halo, nrows};
+            return launch_csr(ctx, A, x, e, pl->kb, CGO_T_SPMV);
+        }
+        EpiResidualT<false> e{b, r, nullptr, nullptr, 0, nrows};
+        return launch_csr(ctx, A, x, e, cgo_red_args(ctx, sumsq ? CGO_P_PHI : CGO_PACK_LEN - 1), CGO_T_SPMV);
+    }
+    // K_c: g⁺ = Aᵀ r with dϕ, ‖g⁺‖² and the getβ dots into pack slots CGO_P_DPHI…  pl: wait for r's halos
+    int gradient(cgo_state *st, const PeerLinks *pl) {
+        if (direct) {
+            CGO_TRY(launch_direct(ctx, AT, r, DirGradLS{st->gp}, pl ? dir_args(ctx, &pl->kc) : dir_args(ctx), CGO_T_SPMVT));
+            return cgo_blas1_grad_dots(st);
+        }
+        EpiGrad<false> e{st->gp, st->g, st->u, nullptr, 0.0, 0.0};
+        return launch_csr(ctx, AT, r, e, pl ? pl->kc : cgo_red_args(ctx, CGO_P_DPHI), CGO_T_SPMVT);
+    }
+    int finish_ls(double *out) {
         CGO_TRY(cgo_finish_pack(ctx, 12, out));
         out[CGO_P_PHI] = 0.5 * out[CGO_P_PHI];
         return 0;
     }
+    int eval_trial_ls(cgo_state *st, double a, bool fused, double beta, double *out) {
+        const bool peer = r_is_peer && st->peer_x;
+        PeerLinks links;
+        const PeerLinks *pl = nullptr;
+        if (peer) { links = peer_links(st); pl = &links; }
+        CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta, pl ? &pl->xp : nullptr));      // K_a (+ halo push)
+        if (!peer) CGO_TRY(exchange(st->xp, st->n));
+        CGO_TRY(residual(st->xp, true, pl));                                           // K_b (+ halo push)
+        if (!peer) CGO_TRY(exchange(r, nrows));
+        CGO_TRY(gradient(st, pl));                                                     // K_c
+        return finish_ls(out);
+    }
+    // ∇²f u = Aᵀ(A u) along the current direction (north_star's Hessian-vector product; the reference
+    // engine never calls one, src/engine/optim.jl:83-145).  `r` is scratch here.
     int hessvec_dir(cgo_state *st, double *out) override {
         CGO_CHECK(!logreg, "the Hessian-vector product is implemented for least squares");
         r_state = nullptr; r_at_x = r_at_xp = false;                                      // r is scratch here
         CGO_TRY(cgo_sendrecv_ring(ctx, st->u, st->u + st->n, st->u + st->n - halo, st->u - halo, halo));
-        if (direct()) {
+        if (direct) {
             CGO_TRY(launch_direct(ctx, A, st->u, DirStore{r}, dir_args(ctx), CGO_T_SPMV));
             CGO_TRY(cgo_blas1_sumsq(ctx, r, nrows, 0));                                   // u·Hu = ‖Au‖²
             CGO_TRY(exchange(r, nrows));
@@ -1432,18 +1334,11 @@ struct CsrObj : cgo_obj {
         // drifts by ≈ ε‖r₀‖ per step — after 64 accepted steps: then r = A x − b is formed again
         if (!(r_state == st && r_at_x) || quad_steps >= 64) {
             CGO_TRY(cgo_sendrecv_ring(ctx, st->x, st->x + st->n, st->x + st->n - halo, st->x - halo, halo));
-            if (direct()) {
-                DirResidual<false> f1{b, r, nullptr, nullptr, 0, nrows};
-                CGO_TRY(launch_direct(ctx, A, st->x, f1, dir_args(ctx), CGO_T_SPMV));
-            } else {
-                EpiResidualT<false> e0;
-                e0.b = b; e0.r = r; e0.prev_right = e0.next_left = nullptr; e0.halo = 0; e0.nrows = nrows;
-                CGO_TRY(launch_csr(ctx, A, st->x, e0, cgo_red_args(ctx, CGO_PACK_LEN - 1), CGO_T_SPMV));
-            }
+            CGO_TRY(residual(st->x, false, nullptr));
             r_state = st; r_at_x = true; r_at_xp = false; quad_steps = 0;
         }
         CGO_TRY(cgo_sendrecv_ring(ctx, st->u, st->u + st->n, st->u + st->n - halo, st->u - halo, halo));
-        if (direct()) {
+        if (direct) {
             CGO_TRY(launch_direct(ctx, A, st->u, DirStore{qv}, dir_args(ctx), CGO_T_SPMV));
             CGO_TRY(cgo_blas1_dots3(ctx, r, qv, nrows, 0));                               // r·v, v·v, r·r
             return cgo_finish_pack(ctx, 3, out);
@@ -1459,19 +1354,55 @@ struct CsrObj : cgo_obj {
         CGO_TRY(cgo_blas1_axpy_dir(st, a, false, 0.0));                                   // xp = x + a u
         CGO_TRY(cgo_blas1_residual_axpy(ctx, r, qv, a, nrows, CGO_P_PHI));                // r += a v, Σ r²
         CGO_TRY(exchange(r, nrows));
-        if (direct()) {
-            CGO_TRY(launch_direct(ctx, AT, r, DirGradLS{st->gp}, dir_args(ctx), CGO_T_SPMVT));
-            CGO_TRY(cgo_blas1_grad_dots(st));
-            CGO_TRY(cgo_finish_pack(ctx, 12, out));
-            out[CGO_P_PHI] = 0.5 * out[CGO_P_PHI];
-            return 0;
+        CGO_TRY(gradient(st, nullptr));                                                   // K_c
+        return finish_ls(out);
+    }
+
+    // ---- logistic regression
+    // k_spmv_direct.  One rank: K_a | passes of A → margins | logit + loss (BLAS-1) | passes of Aᵀ | /N + λw + dots
+    // (BLAS-1).  R ranks: K_a also stores its shard of xp into every rank's all-gathered copy; the logit kernel stores
+    // its shard of c into every rank's all-gathered c; flags hand the data to the consuming passes (without peer
+    // memory: two NCCL all-gathers).
+    int eval_trial_lr_direct(cgo_state *st, double a, bool fused, double beta, double *out) {
+        const int R = ctx->nranks;
+        RedArgs wx, wc;                           // flag waits of the first K_b / K_c pass
+        const RedArgs *pwx = nullptr, *pwc = nullptr;
+        unsigned long long e = 0;
+        if (R > 1 && lr_peer) {
+            e = ++ctx->epoch;
+            HaloPush hp;
+            hp.dst_all = d_xpf_dst; hp.epoch = e;
+            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta, &hp));                     // K_a + all-gather of xp
+            wx.wait_all = ctx->flags_local + CGO_F_XPALL; wx.wait_val = e; wx.nranks = R; pwx = &wx;
+            wc.wait_all = ctx->flags_local + CGO_F_CALL; wc.wait_val = e; wc.nranks = R; pwc = &wc;
+        } else {
+            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                          // K_a
+            if (R > 1) CGO_TRY(cgo_allgatherv_f64(ctx, st->xp, xp_full, flo.data()));
         }
-        EpiGrad<false> e2{st->gp, st->g, st->u, nullptr, 0.0, 0.0};
-        CGO_TRY(launch_csr(ctx, AT, r, e2, cgo_red_args(ctx, CGO_P_DPHI), CGO_T_SPMVT));  // K_c
+        const double *w_all = R > 1 ? xp_full : st->xp;
+        CGO_TRY(spmv_direct_passes(ctx, A, Ab, w_all, r, pwx, CGO_T_SPMV));            // K_b: margins of my samples
+        CGO_TRY(cgo_blas1_logit(ctx, r, b, nrows, CGO_P_PHI, (R > 1 && lr_peer) ? d_cf_dst : nullptr, e));   // c, Σ loss [+ all-gather of c]
+        if (R > 1 && !lr_peer) CGO_TRY(cgo_allgatherv_f64(ctx, r, c_full, slo.data()));
+        const double *c_all = R > 1 ? c_full : r;
+        CGO_TRY(spmv_direct_passes(ctx, AT, ATb, c_all, st->gp, pwc, CGO_T_SPMVT));    // K_c: Aᵀc over my features
+        CGO_TRY(cgo_blas1_grad_combine(st, 1.0 / (double)nsamples, lambda));           // /N + λw, dots
+        return finish_lr(out);
+    }
+    // the fused k_csr_rows, one pass of each matrix (single rank)
+    int eval_trial_lr_fused(cgo_state *st, double a, bool fused, double beta, double *out) {
+        CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                                             // K_a
+        EpiLogit e1{b, r};
+        CGO_TRY(launch_csr(ctx, A, st->xp, e1, cgo_red_args(ctx, CGO_P_PHI), CGO_T_SPMV));            // K_b
+        EpiGrad<true> e2{st->gp, st->g, st->u, st->xp, 1.0 / (double)nsamples, lambda};
+        CGO_TRY(launch_csr(ctx, AT, r, e2, cgo_red_args(ctx, CGO_P_DPHI), CGO_T_SPMVT));              // K_c
+        return finish_lr(out);
+    }
+    int finish_lr(double *out) {
         CGO_TRY(cgo_finish_pack(ctx, 12, out));
-        out[CGO_P_PHI] = 0.5 * out[CGO_P_PHI];
+        out[CGO_P_PHI] = out[CGO_P_PHI] / (double)nsamples + (0.5 * lambda) * out[CGO_P_XPXP];
         return 0;
     }
+
     void on_accept(cgo_state *st) override {
         r_at_x = (r_state == st) && r_at_xp;
         r_at_xp = false;
@@ -1479,39 +1410,18 @@ struct CsrObj : cgo_obj {
     }
     int eval_trial(cgo_state *st, double a, bool fused, double beta, double *out) override {
         r_state = st; r_at_xp = true; r_at_x = false; quad_steps = 0;        // r = A xp − b (least squares) / c (logreg)
-        if (!logreg && direct()) return eval_trial_ls_direct(st, a, fused, beta, out);
-        if (!logreg && r_is_peer && st->peer_x) return eval_trial_ls_peer(st, a, fused, beta, out);
-        if (logreg && lr_direct) return eval_trial_lr_direct(st, a, fused, beta, out);
-        CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                               // K_a
-        CGO_TRY(exchange(st->xp, st->n));
-        if (logreg) {
-            EpiLogit e1{b, r};
-            CGO_TRY(launch_csr_blocked(ctx, A, Ab, st->xp, e1, r, cgo_red_args(ctx, CGO_P_PHI), CGO_T_SPMV));   // K_b
-            EpiGrad<true> e2{st->gp, st->g, st->u, st->xp, 1.0 / (double)nsamples, lambda};
-            CGO_TRY(launch_csr_blocked(ctx, AT, ATb, r, e2, st->gp, cgo_red_args(ctx, CGO_P_DPHI), CGO_T_SPMVT)); // K_c
-            CGO_TRY(cgo_finish_pack(ctx, 12, out));
-            out[CGO_P_PHI] = out[CGO_P_PHI] / (double)nsamples + (0.5 * lambda) * out[CGO_P_XPXP];
-        } else {
-            EpiResidualT<false> e1;
-            e1.b = b; e1.r = r; e1.prev_right = e1.next_left = nullptr; e1.halo = 0; e1.nrows = nrows;
-            CGO_TRY(launch_csr(ctx, A, st->xp, e1, cgo_red_args(ctx, CGO_P_PHI), CGO_T_SPMV));   // K_b
-            CGO_TRY(exchange(r, nrows));
-            EpiGrad<false> e2{st->gp, st->g, st->u, nullptr, 0.0, 0.0};
-            CGO_TRY(launch_csr(ctx, AT, r, e2, cgo_red_args(ctx, CGO_P_DPHI), CGO_T_SPMVT));      // K_c
-            CGO_TRY(cgo_finish_pack(ctx, 12, out));
-            out[CGO_P_PHI] = 0.5 * out[CGO_P_PHI];
-        }
-        return 0;
+        if (!logreg) return eval_trial_ls(st, a, fused, beta, out);
+        return direct ? eval_trial_lr_direct(st, a, fused, beta, out) : eval_trial_lr_fused(st, a, fused, beta, out);
     }
     // SURVEY.md §8(d): A and Aᵀ streamed once (8 B value + 4 B index per entry + row pointers)
     // plus the vector passes R x,u W xp | gather xp, R b, W r | gather r, W g⁺, R u (,g)
     double bytes_per_eval() const override {
-        if (lr_direct)      // K_a 24d_loc | A_r + gather + W z | logit R z, y W c | Aᵀ_f + gather + W q | R q, u, g, w W g⁺
+        if (logreg && direct)   // K_a 24d_loc | A_r + gather + W z | logit R z, y W c | Aᵀ_f + gather + W q | R q, u, g, w W g⁺
             return 12.0 * (double)(A.nnz + AT.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
                    8.0 * (5.0 * (double)nrows + (ctx->nranks > 1 ? (double)n_global + (double)nsamples : 0.0) + 11.0 * (double)n_local);
-        // (gather-bound matrices: the dots are separate BLAS-1 passes, R r | R g⁺, g, u instead of the staged u, g)
+        // (k_spmv_direct: the dots are separate BLAS-1 passes, R r | R g⁺, g, u instead of the staged u, g)
         return 12.0 * (double)(A.nnz + AT.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
-               8.0 * (3.0 * (double)nrows + 6.0 * (double)n_local) + (direct() ? 8.0 * ((double)nrows + (double)n_local) : 0.0);
+               8.0 * (3.0 * (double)nrows + 6.0 * (double)n_local) + (direct ? 8.0 * ((double)nrows + (double)n_local) : 0.0);
     }
     int default_x0(uint64_t, double, double *x0) override {
         for (int64_t i = 0; i < n_local; ++i) x0[i] = 0.0;
@@ -1583,6 +1493,7 @@ extern "C" int cgo_obj_sparse_ls_create_synthetic(cgo_ctx *ctx, int64_t n, int32
             CGO_TRY(csr_make_sliced(ctx, o->A));
             CGO_TRY(csr_make_sliced(ctx, o->AT));
         }
+        o->direct = o->A.sliced != 0;          // (not sliced without entries)
         return 0;
     };
     int rc = body();
@@ -1623,11 +1534,11 @@ extern "C" int cgo_obj_sparse_ls_create_csr(cgo_ctx *ctx, int64_t nrows, int64_t
         float la = 1.f, lt = 1.f;
         CGO_TRY(csr_gather_lines(ctx, o->A, &la));
         CGO_TRY(csr_gather_lines(ctx, o->AT, &lt));
-        o->A.lines_per_gather = la; o->AT.lines_per_gather = lt;
         if (ctx->csr_mode == 2 || (ctx->csr_mode == 0 && la > 4.0f && lt > 4.0f && nrows >= 4096)) {
             CGO_TRY(csr_make_sliced(ctx, o->A));
             CGO_TRY(csr_make_sliced(ctx, o->AT));
         }
+        o->direct = o->A.sliced != 0;          // (not sliced without entries)
         return 0;
     };
     int rc = body();
@@ -1709,9 +1620,12 @@ extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t 
             LrFeatFin fin{sp};
             CGO_TRY(build_transpose(ctx, src, fin, fhi - flo, o->AT));
         }
-        // K_b gathers over all d features, K_c over all N samples
-        CGO_TRY(build_blocked(ctx, o->A, d, o->Ab));
-        CGO_TRY(build_blocked(ctx, o->AT, N, o->ATb));
+        // K_b gathers over all d features, K_c over all N samples.  Column blocks are k_spmv_direct passes: the
+        // forced k_csr_rows (CGO_CSR_MODE=1) runs single-pass whatever the gather range
+        if (ctx->csr_mode != 1) {
+            CGO_TRY(build_blocked(ctx, o->A, d, o->Ab));
+            CGO_TRY(build_blocked(ctx, o->AT, N, o->ATb));
+        }
         const bool blocked = !o->Ab.blk.empty() || !o->ATb.blk.empty();
         if (blocked && o->A.nnz > (int64_t)200000000 / R) {
             // production sizes: drop the single-pass copies (only the CSR test hooks read them)
@@ -1721,8 +1635,8 @@ extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t 
         }
         // uniformly random columns: gather-bound (k_spmv_direct + BLAS-1 epilogues) whenever the gathers are what
         // costs — column-blocked sizes, and always when sharded
-        o->lr_direct = ctx->csr_mode != 1 && (R > 1 || blocked || ctx->csr_mode == 2);
-        if (o->lr_direct) {
+        o->direct = ctx->csr_mode != 1 && (R > 1 || blocked || ctx->csr_mode == 2);
+        if (o->direct) {
             if (o->Ab.blk.empty()) CGO_TRY(csr_make_sliced(ctx, o->A));
             if (o->ATb.blk.empty()) CGO_TRY(csr_make_sliced(ctx, o->AT));
             for (auto &m : o->Ab.blk) CGO_TRY(csr_make_sliced(ctx, m));

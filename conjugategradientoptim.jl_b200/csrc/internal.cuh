@@ -72,10 +72,8 @@ struct cgo_ctx {
     bool own_stream = false;
     int G = 296;
     size_t gather_block_bytes = (size_t)40 << 20;   // column-block size of large random gathers (csr.cu)
-    int csr_pass_occ = 2;                           // CTAs per SM of the column-block passes (CGO_CSR_PASS_OCC=3 to try 3)
     int64_t launches = 0;
     int csr_mode = 0;        // 0: per matrix (sliced layout + k_spmv_direct when its gathers do not coalesce); 1: never; 2: always (CGO_CSR_MODE)
-    int direct_cfg = 0;      // k_spmv_direct variant (CGO_DIRECT_CFG: 0 = by matrix, 2 = 10 gathers per batch × 4 CTAs/SM, 1 = 8 × 4, 3 = 6 × 5)
     unsigned long long *d_progress = nullptr;   // [1..3] set-up scratch; [4] k_spmv_direct's slice queue
     // reduction scratch
     double *d_partial = nullptr;     // CGO_MAXK * Gmax
@@ -120,10 +118,10 @@ void cgo_dev_free(cgo_ctx *ctx, void *ptr, size_t bytes);
 // flag slots of a rank's block
 // (CGO_F_PACK + r: rank r's scalar pack of the current exchange has landed in my gather block)
 constexpr int CGO_MAX_RANKS = 64;
-// (CGO_F_XPALL + r: rank r's shard of xp has landed in my all-gathered copy; CGO_F_GPART + r: rank r's
-// partial-gradient slice of my feature shard has landed)
+// (CGO_F_XPALL + r: rank r's shard of xp has landed in my all-gathered copy; CGO_F_CALL + r: rank r's shard of
+// c = −y σ has landed in my all-gathered c)
 enum { CGO_F_XP_FROM_PREV = 0, CGO_F_XP_FROM_NEXT = 1, CGO_F_R_FROM_PREV = 2, CGO_F_R_FROM_NEXT = 3, CGO_F_PACK = 8,
-       CGO_F_XPALL = 8 + CGO_MAX_RANKS, CGO_F_GPART = 8 + 2 * CGO_MAX_RANKS, CGO_F_N = 8 + 3 * CGO_MAX_RANKS };
+       CGO_F_XPALL = 8 + CGO_MAX_RANKS, CGO_F_CALL = 8 + 2 * CGO_MAX_RANKS, CGO_F_N = 8 + 3 * CGO_MAX_RANKS };
 // allocate `bytes` of device memory on every rank (collective) and map every peer's block:
 // peers[r] is rank r's block in this process's address space (peers[rank] == *local).
 int cgo_peer_alloc(cgo_ctx *ctx, size_t bytes, void **local, std::vector<void *> &peers);
@@ -143,11 +141,9 @@ void cgo_timer_end(cgo_ctx *ctx);
 void cgo_timer_collect(cgo_ctx *ctx);          // after a stream sync: fold pending timers
 int cgo_finish_pack(cgo_ctx *ctx, int K, double *out_host);
 int cgo_combine_ranks(cgo_ctx *ctx, int K, double *out_dev);   // multi-rank: Σ_r d_pack[0..K) in rank order → out_dev
-int cgo_allgather_bytes(cgo_ctx *ctx, const void *send_dev, void *recv_dev, size_t bytes_per_rank);
 int cgo_sendrecv_ring(cgo_ctx *ctx, const double *send_to_prev, double *recv_from_next,
                       const double *send_to_next, double *recv_from_prev, int64_t count);
 int cgo_allgatherv_f64(cgo_ctx *ctx, const double *mine, double *full, const int64_t *lo);
-int cgo_alltoallv_f64(cgo_ctx *ctx, const double *full, const int64_t *lo, double *recv, int64_t stride);
 
 // ------------------------------------------------------------------ objective interface
 struct cgo_state;
@@ -218,14 +214,12 @@ int cgo_blas1_axpy_dir(cgo_state *st, double a, bool fused_dir, double beta, con
 int cgo_blas1_residual_axpy(cgo_ctx *ctx, double *r, const double *v, double a, int64_t nrows, int slot);
 int cgo_blas1_sumsq(cgo_ctx *ctx, const double *a, int64_t n, int slot);                        // Σ a²
 int cgo_blas1_dots3(cgo_ctx *ctx, const double *a, const double *b, int64_t n, int slot);       // {a·b, b·b, a·a}
-// margins → c = −y σ in place, Σ loss → pack slot; dst_all != NULL: also all-gather c over peer memory (flag CGO_F_GPART)
+// margins → c = −y σ in place, Σ loss → pack slot; dst_all != NULL: also all-gather c over peer memory (flag CGO_F_CALL)
 int cgo_blas1_logit(cgo_ctx *ctx, double *zc, const double *y, int64_t n, int slot, void *const *dst_all, unsigned long long epoch);
 int cgo_blas1_grad_dots(cgo_state *st);     // the eight dots of EpiGrad over (g⁺, g, u) → pack slots CGO_P_DPHI…
-// sample-sharded logistic regression: g⁺ = (Σ_r q[r·stride + i]) / N + λ xp, partial gradients
-// added in rank order, fused with the dot pack of EpiGrad (slots CGO_P_DPHI .. CGO_P_UU)
-// wait_epoch != 0: spin until every rank's CGO_F_GPART flag reached it before reading q
-int cgo_blas1_grad_combine(cgo_state *st, const double *q, int nparts, int64_t stride, double invN, double lambda,
-                           unsigned long long wait_epoch = 0);
+// logistic regression on k_spmv_direct: g⁺ = g⁺ · invN + λ xp in place (g⁺ holds Aᵀc), fused with the dot pack of
+// EpiGrad (slots CGO_P_DPHI .. CGO_P_UU)
+int cgo_blas1_grad_combine(cgo_state *st, double invN, double lambda);
 
 // ------------------------------------------------------------------ CSR (csr.cu)
 struct CsrMat {
@@ -237,6 +231,4 @@ struct CsrMat {
     // (all first entries of the slice's rows in row order, then all second entries, …) instead of row-major
     int32_t sliced = 0;
     int32_t ragged = 0;          // sliced: more than one slice in 16 has rows of different lengths (picks the batch width)
-    int64_t max_tile_nnz = 0;    // most entries in any 256-row tile
-    float lines_per_gather = 1.f;   // distinct 128-byte lines one warp-level gather touches (sampled at set-up)
 };

@@ -90,7 +90,9 @@ int cgo_ctx_stream(cgo_ctx *ctx, void **cuda_stream_out);
 int cgo_ctx_set_reduction_ctas(cgo_ctx *ctx, int G);        /* canonical-order G (default 296) */
 /* objectives whose gathers range over a vector larger than this are stored column-blocked and
  * evaluated one block per pass, so that the gathered window stays L2-resident (default 40 MiB;
- * 0 = never block).  Applies to objectives created afterwards; results are bit-identical. */
+ * 0 = never block).  Column blocks apply to the k_spmv_direct family (cgo_ctx_set_csr_mode): an
+ * objective forced onto k_csr_rows runs single-pass.  Applies to objectives created afterwards;
+ * results are bit-identical. */
 int cgo_ctx_set_gather_block_bytes(cgo_ctx *ctx, int64_t bytes);
 /* which SpMV kernel family CSR objectives created afterwards use: 0 = per matrix (default: k_spmv_direct + BLAS-1
  * dots when its gathers do not coalesce, the fused k_csr_rows otherwise), 1 = always k_csr_rows, 2 = always

@@ -258,7 +258,7 @@ def test_lbfgs_natural_rejection_at_full_history_matches_oracle(ctx):
 
 # --------------------------------------------------------------------------------------------- CSR ring
 def _ts_layout(nops=0, budget=115200, nd=3, lanes=256, maxk=12, nw=8):
-    """RING and CHMAX of TsLayout<NOPS, 2> (csr.cu): the ring of k_csr_rows holds RING entries, a tile longer than
+    """RING and CHMAX of TsLayout<NOPS> (csr.cu): the ring of k_csr_rows holds RING entries, a tile longer than
     CHMAX entries streams in CHMAX chunks, TS_ND = nd descriptors"""
     desc = (lanes + 2) * 8 + nops * lanes * 8
     tail = 2 * nd * 8 + nd * 4 + maxk * nw * 8

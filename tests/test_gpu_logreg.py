@@ -106,24 +106,29 @@ def test_column_blocked_passes_are_bit_identical(block_elems):
     """Large random gathers are evaluated one L2-sized column block per pass (csr.cu CsrBlocked);
     passes chain the row sums, so f, g and whole runs must not change by a single bit."""
     N, d, lam = 20_000, 3000, 1e-4
-    c0, c1, c2 = cg.Context(0), cg.Context(0), cg.Context(0)
+    c0, c1, c2, c3 = cg.Context(0), cg.Context(0), cg.Context(0), cg.Context(0)
     c0.set_gather_block_bytes(0)
     c0.set_csr_mode(2)                       # single pass through k_spmv_direct: same kernels, same order of the dots
     c1.set_gather_block_bytes(8 * block_elems)
     c2.set_gather_block_bytes(0)             # single pass through the fused k_csr_rows (dots in the row-per-lane order)
+    c3.set_gather_block_bytes(8 * block_elems)
+    c3.set_csr_mode(1)                       # forced k_csr_rows: column blocks apply to k_spmv_direct only
     a, b = cg.LogRegGPU(N, d, 20, 24, lam, c0), cg.LogRegGPU(N, d, 20, 24, lam, c1)
-    f = cg.LogRegGPU(N, d, 20, 24, lam, c2)
+    f, h = cg.LogRegGPU(N, d, 20, 24, lam, c2), cg.LogRegGPU(N, d, 20, 24, lam, c3)
     assert a.csr_blocks(False) == 1 and a.csr_blocks(True) == 1
     assert b.csr_blocks(False) == -(-d // block_elems) and b.csr_blocks(True) == -(-N // block_elems)
-    assert a.trial_site == b.trial_site == (2, 4) and f.trial_site == (1, 1)
+    assert h.csr_blocks(False) == 1 and h.csr_blocks(True) == 1
+    assert a.trial_site == b.trial_site == (2, 4) and f.trial_site == h.trial_site == (1, 1)
     w = 0.5 * np.random.default_rng(3).standard_normal(d)
     wa, wb = a.make_workspace(w, fuse_direction=False), b.make_workspace(w, fuse_direction=False)
-    wf = f.make_workspace(w, fuse_direction=False)
+    wf, wh = f.make_workspace(w, fuse_direction=False), h.make_workspace(w, fuse_direction=False)
     assert wa.f_x0 == wb.f_x0 and np.array_equal(wa.pack, wb.pack)
     assert np.array_equal(wa.download()[1], wb.download()[1])
+    assert wh.f_x0 == wf.f_x0 and np.array_equal(wh.pack, wf.pack)
+    assert np.array_equal(wh.download()[1], wf.download()[1])
     assert np.array_equal(wa.download()[1], wf.download()[1])          # the gradient does not depend on the kernel family
     assert abs(wf.f_x0 - wa.f_x0) <= 1e-14 * abs(wa.f_x0)              # the loss only through the order of its sum
-    wa.close(); wb.close(); wf.close(); f.close(); c2.close()
+    wa.close(); wb.close(); wf.close(); wh.close(); f.close(); h.close(); c2.close(); c3.close()
     _, cfg, ls = make_pair("LBFGS", max_iters=25, c1=1e-4, c2=0.9)
     ra = cg.minimizeobjective(a, np.zeros(d), cfg, ls)
     rb = cg.minimizeobjective(b, np.zeros(d), cfg, ls)
