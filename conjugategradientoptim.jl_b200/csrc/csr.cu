@@ -19,6 +19,7 @@
 // the 256 row lanes gather the vector entries and add up their row's products in storage
 // order.  Rows and tiles of any length work.
 #include <cub/device/device_scan.cuh>
+#include <cmath>
 
 #include "internal.cuh"
 #include "reduce.cuh"
@@ -1144,6 +1145,186 @@ static int spmv_direct_passes(cgo_ctx *c, const CsrMat &M, const CsrBlocked &B, 
     return 0;
 }
 
+// ------------------------------------------------------------------ long rows (logistic regression from a host CSR)
+// A row with more than CGO_LONG_ROW entries would chain its products on one lane of k_spmv_direct: the ones column
+// of an intercept is a row of Aᵀ with N entries.  Such rows are taken out of the matrix the row kernels see (they
+// are empty in its sliced copy and in every column block), stored once, unblocked, and summed in the canonical order
+// of include/cgoptim.h with V = 1, U = 4.  A work unit is one (long row, virtual CTA) pair with data; k_long_rows
+// spreads the units over the whole grid, and each adds its lanes' products and combines its 256 lanes into one
+// partial.  k_long_finish, one CTA per long row, combines the row's partials and stores the row sum where the row
+// kernel stores the others.
+constexpr int LONG_U = 4;                    // items per lane and tile
+constexpr int LONG_TILE = CGO_B * LONG_U;
+constexpr int LONG_TB = 2;                   // tiles of one unit whose loads are in flight together
+struct LongRows {
+    int64_t n = 0;                           // long rows
+    CsrMat M;                                // the long rows, row-major, entries in storage order
+    int64_t *row = nullptr;                  // their indices in the whole matrix (device)
+    std::vector<int64_t> h_row, h_rowptr;    // host copies of `row` and M.rowptr
+    int G = 0;                               // the G the work units are laid out for
+    int64_t nunits = 0;
+    int2 *unit = nullptr;                    // (long row, virtual CTA) of every unit
+    int64_t *ubase = nullptr;                // first unit of every long row, n + 1
+    double *partial = nullptr;               // one per unit
+    void free_all() {
+        csr_free(M);
+        cudaFree(row); cudaFree(unit); cudaFree(ubase); cudaFree(partial);
+        *this = LongRows();
+    }
+};
+
+__global__ void __launch_bounds__(CGO_B) k_long_rows(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G,
+                                                     const double *__restrict__ xg, double *__restrict__ partial) {
+    __shared__ double s_red[CGO_NW];
+    const int t = threadIdx.x;
+    const uint64_t gpol = l2_policy_evict_last();
+    for (int64_t u = blockIdx.x; u < nunits; u += gridDim.x) {
+        const int2 w = unit[u];
+        const int64_t p0 = L.rowptr[w.x], len = L.rowptr[w.x + 1] - p0;
+        const int64_t ntiles = (len + LONG_TILE - 1) / LONG_TILE;
+        double acc[1] = {0.0};
+#pragma unroll 1
+        for (int64_t tile = w.y; tile < ntiles; tile += (int64_t)LONG_TB * G) {
+            // the lane's items of tiles tile, tile + G, …: index order, values and indices coalesced across the lanes
+            constexpr int NI = LONG_TB * LONG_U;
+            int32_t cj[NI];
+            double vj[NI], xj[NI];
+            bool on[NI];
+#pragma unroll
+            for (int j = 0; j < NI; ++j) {
+                const int64_t k = (tile + (int64_t)(j / LONG_U) * G) * LONG_TILE + (j % LONG_U) * CGO_B + t;
+                on[j] = k < len;
+                cj[j] = ld_stream_s32_if(L.col + p0 + k, on[j]);
+                vj[j] = ld_stream_f64_if(L.val + p0 + k, on[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < NI; ++j) xj[j] = ld_gather_f64_if(xg + cj[j], gpol, on[j]);
+#pragma unroll
+            for (int j = 0; j < NI; ++j) {
+                const double p = vj[j] * xj[j];
+                if (on[j]) acc[0] = acc[0] + p;
+            }
+        }
+        cgo_cta_combine<1>(acc, s_red);
+        if (t == 0) partial[u] = acc[0];
+    }
+}
+// one CTA per long row: lane t adds the row's partials t, t + 256, …, then the CTA combine
+__global__ void __launch_bounds__(CGO_B) k_long_finish(const int64_t *__restrict__ ubase, const int64_t *__restrict__ row,
+                                                       const double *__restrict__ partial, double *out) {
+    __shared__ double s_red[CGO_NW];
+    const int64_t b = ubase[blockIdx.x], nact = ubase[blockIdx.x + 1] - b;
+    double acc[1] = {0.0};
+    for (int64_t c = threadIdx.x; c < nact; c += CGO_B) acc[0] = acc[0] + partial[b + c];
+    cgo_cta_combine<1>(acc, s_red);
+    if (threadIdx.x == 0) out[row[blockIdx.x]] = acc[0];
+}
+
+// lay the work units out for the ctx's G (at the first evaluation, and again when G changes)
+static int long_units(cgo_ctx *c, LongRows &L) {
+    if (L.G == c->G) return 0;
+    std::vector<int2> unit;
+    std::vector<int64_t> ubase((size_t)L.n + 1, 0);
+    for (int64_t r = 0; r < L.n; ++r) {
+        const int64_t ntiles = (L.h_rowptr[(size_t)r + 1] - L.h_rowptr[(size_t)r] + LONG_TILE - 1) / LONG_TILE;
+        const int64_t nact = ntiles < c->G ? ntiles : c->G;
+        for (int64_t v = 0; v < nact; ++v) unit.push_back(make_int2((int)r, (int)v));
+        ubase[(size_t)r + 1] = (int64_t)unit.size();
+    }
+    cudaFree(L.unit); cudaFree(L.partial);
+    L.unit = nullptr; L.partial = nullptr; L.G = 0;
+    L.nunits = (int64_t)unit.size();
+    CGO_CUDA(cudaMalloc(&L.unit, sizeof(int2) * unit.size()));
+    CGO_CUDA(cudaMalloc(&L.partial, sizeof(double) * unit.size()));
+    CGO_CUDA(cudaMemcpyAsync(L.unit, unit.data(), sizeof(int2) * unit.size(), cudaMemcpyHostToDevice, c->stream));
+    CGO_CUDA(cudaMemcpyAsync(L.ubase, ubase.data(), sizeof(int64_t) * ubase.size(), cudaMemcpyHostToDevice, c->stream));
+    CGO_CUDA(cudaStreamSynchronize(c->stream));
+    L.G = c->G;
+    return 0;
+}
+// out[row] = the sum of every long row, after the row kernels' last pass over the same output
+static int long_rows_sum(cgo_ctx *c, LongRows &L, const double *xg, double *out, int tclass) {
+    if (L.n == 0) return 0;
+    CGO_TRY(long_units(c, L));
+    const int64_t phys = (int64_t)c->sms * 8;
+    const int grid = (int)(L.nunits < phys ? L.nunits : phys);
+    cgo_timer_begin(c, tclass);
+    k_long_rows<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, xg, L.partial);
+    cgo_timer_end(c);
+    c->launches++;
+    CGO_CUDA(cudaGetLastError());
+    cgo_timer_begin(c, tclass);
+    k_long_finish<<<(unsigned)L.n, CGO_B, 0, c->stream>>>(L.ubase, L.row, L.partial, out);
+    cgo_timer_end(c);
+    c->launches++;
+    CGO_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// set-up: the rows of A longer than CGO_LONG_ROW move to L; A keeps them as empty rows (count + scan + copy)
+__global__ void k_strip_count(CsrMat A, int64_t *cnt) {
+    GRID_STRIDE(i, A.nrows + 1) {
+        const int64_t len = i < A.nrows ? A.rowptr[i + 1] - A.rowptr[i] : 0;
+        cnt[i] = len > CGO_LONG_ROW ? 0 : len;
+    }
+}
+__global__ void k_long_copy(CsrMat A, const int64_t *row, CsrMat L) {
+    for (int64_t r = blockIdx.x; r < L.nrows; r += gridDim.x) {
+        const int64_t s0 = A.rowptr[row[r]], d0 = L.rowptr[r], n = L.rowptr[r + 1] - d0;
+        for (int64_t e = threadIdx.x; e < n; e += blockDim.x) { L.col[d0 + e] = A.col[s0 + e]; L.val[d0 + e] = A.val[s0 + e]; }
+    }
+}
+static int split_long_rows(cgo_ctx *c, CsrMat &A, LongRows &L) {
+    cudaStream_t s = c->stream;
+    std::vector<int64_t> rp((size_t)A.nrows + 1);
+    CGO_CUDA(cudaMemcpyAsync(rp.data(), A.rowptr, sizeof(int64_t) * rp.size(), cudaMemcpyDeviceToHost, s));
+    CGO_CUDA(cudaStreamSynchronize(s));
+    L.h_rowptr.assign(1, 0);
+    for (int64_t i = 0; i < A.nrows; ++i) {
+        const int64_t len = rp[(size_t)i + 1] - rp[(size_t)i];
+        if (len <= CGO_LONG_ROW) continue;
+        L.h_row.push_back(i);
+        L.h_rowptr.push_back(L.h_rowptr.back() + len);
+    }
+    L.n = (int64_t)L.h_row.size();
+    if (L.n == 0) return 0;
+    CsrMat S;
+    int64_t *cnt = nullptr;
+    void *tmp = nullptr;
+    auto body = [&]() -> int {
+        CGO_TRY(csr_alloc(L.M, L.n, L.h_rowptr.back()));
+        CGO_CUDA(cudaMalloc(&L.row, sizeof(int64_t) * (size_t)L.n));
+        CGO_CUDA(cudaMalloc(&L.ubase, sizeof(int64_t) * (size_t)(L.n + 1)));
+        CGO_CUDA(cudaMemcpyAsync(L.M.rowptr, L.h_rowptr.data(), sizeof(int64_t) * (size_t)(L.n + 1), cudaMemcpyHostToDevice, s));
+        CGO_CUDA(cudaMemcpyAsync(L.row, L.h_row.data(), sizeof(int64_t) * (size_t)L.n, cudaMemcpyHostToDevice, s));
+        k_long_copy<<<(unsigned)(L.n < (int64_t)c->sms * 4 ? L.n : (int64_t)c->sms * 4), 256, 0, s>>>(A, L.row, L.M);
+        CGO_CUDA(cudaGetLastError());
+        CGO_CUDA(cudaMalloc(&cnt, sizeof(int64_t) * (size_t)(A.nrows + 1)));
+        k_strip_count<<<grid_for(A.nrows + 1, c->sms), 256, 0, s>>>(A, cnt);
+        CGO_CUDA(cudaGetLastError());
+        S.nrows = A.nrows;
+        CGO_CUDA(cudaMalloc(&S.rowptr, sizeof(int64_t) * (size_t)(A.nrows + 1 + CSR_PAD)));
+        size_t tmp_bytes = 0;
+        CGO_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, cnt, S.rowptr, A.nrows + 1, s));
+        CGO_CUDA(cudaMalloc(&tmp, tmp_bytes > 0 ? tmp_bytes : 1));
+        CGO_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, cnt, S.rowptr, A.nrows + 1, s));
+        CGO_CUDA(cudaMemcpyAsync(&S.nnz, S.rowptr + A.nrows, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+        CGO_CUDA(cudaStreamSynchronize(s));
+        CGO_CUDA(cudaMalloc(&S.col, sizeof(int32_t) * (size_t)(S.nnz + CSR_PAD)));
+        CGO_CUDA(cudaMalloc(&S.val, sizeof(double) * (size_t)(S.nnz + CSR_PAD)));
+        k_blk_copy<<<grid_for(A.nrows, c->sms), 256, 0, s>>>(A, A.rowptr, S);
+        CGO_CUDA(cudaGetLastError());
+        CGO_CUDA(cudaStreamSynchronize(s));
+        return 0;
+    };
+    const int rc = body();
+    cudaFree(cnt); cudaFree(tmp);
+    if (rc) { csr_free(S); return rc; }
+    csr_free(A);
+    A = S;
+    return 0;
+}
+
 // ------------------------------------------------------------------ the objective
 struct CsrObj : cgo_obj {
     bool logreg = false;
@@ -1154,6 +1335,7 @@ struct CsrObj : cgo_obj {
     bool direct = false;
     CsrMat A, AT;
     CsrBlocked Ab, ATb;                // column-blocked copies (logreg on k_spmv_direct, large gather ranges)
+    LongRows LA, LAT;                  // rows taken out of A / AT (logreg from a host CSR on k_spmv_direct)
     bool have_unblocked = true;        // A / AT arrays still allocated (test hooks need them)
     int64_t nrows = 0;                 // local rows of A (residuals / samples)
     double *b = nullptr;               // rhs (LS) or labels (logreg), nrows
@@ -1185,6 +1367,7 @@ struct CsrObj : cgo_obj {
         if (ctx && cgo_ctx_alive(ctx)) cudaSetDevice(ctx->device);
         csr_free(A); csr_free(AT);
         Ab.free_all(); ATb.free_all();
+        LA.free_all(); LAT.free_all();
         if (r_is_peer) { cgo_peer_free(ctx, r_base, rpeers, true); r_base = nullptr; }
         if (lr_peer) {
             cgo_peer_free(ctx, xp_full, xpf_peers, true); xp_full = nullptr;
@@ -1381,10 +1564,12 @@ struct CsrObj : cgo_obj {
         }
         const double *w_all = R > 1 ? xp_full : st->xp;
         CGO_TRY(spmv_direct_passes(ctx, A, Ab, w_all, r, pwx, CGO_T_SPMV));            // K_b: margins of my samples
+        CGO_TRY(long_rows_sum(ctx, LA, w_all, r, CGO_T_SPMV));                           // … of the long rows
         CGO_TRY(cgo_blas1_logit(ctx, r, b, nrows, CGO_P_PHI, (R > 1 && lr_peer) ? d_cf_dst : nullptr, e));   // c, Σ loss [+ all-gather of c]
         if (R > 1 && !lr_peer) CGO_TRY(cgo_allgatherv_f64(ctx, r, c_full, slo.data()));
         const double *c_all = R > 1 ? c_full : r;
         CGO_TRY(spmv_direct_passes(ctx, AT, ATb, c_all, st->gp, pwc, CGO_T_SPMVT));    // K_c: Aᵀc over my features
+        CGO_TRY(long_rows_sum(ctx, LAT, c_all, st->gp, CGO_T_SPMVT));                    // … and over the long rows
         CGO_TRY(cgo_blas1_grad_combine(st, 1.0 / (double)nsamples, lambda));           // /N + λw, dots
         return finish_lr(out);
     }
@@ -1417,7 +1602,7 @@ struct CsrObj : cgo_obj {
     // plus the vector passes R x,u W xp | gather xp, R b, W r | gather r, W g⁺, R u (,g)
     double bytes_per_eval() const override {
         if (logreg && direct)   // K_a 24d_loc | A_r + gather + W z | logit R z, y W c | Aᵀ_f + gather + W q | R q, u, g, w W g⁺
-            return 12.0 * (double)(A.nnz + AT.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
+            return 12.0 * (double)(A.nnz + AT.nnz + LA.M.nnz + LAT.M.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
                    8.0 * (5.0 * (double)nrows + (ctx->nranks > 1 ? (double)n_global + (double)nsamples : 0.0) + 11.0 * (double)n_local);
         // (k_spmv_direct: the dots are separate BLAS-1 passes, R r | R g⁺, g, u instead of the staged u, g)
         return 12.0 * (double)(A.nnz + AT.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
@@ -1431,6 +1616,15 @@ struct CsrObj : cgo_obj {
 
 static int check_i32(int64_t v, const char *what) {
     CGO_CHECK(v < 2147483647LL, "%s = %lld does not fit the int32 column index", what, (long long)v);
+    return 0;
+}
+
+// a host CSR's arrays (both host-CSR constructors): argument errors name the offending row or entry
+static int check_host_csr(int64_t nrows, int64_t ncols, const int64_t *rowptr, const int32_t *col, const double *val) {
+    const int64_t nnz = rowptr[nrows];
+    CGO_CHECK(nnz == 0 || (col && val), "NULL col/val");
+    for (int64_t i = 0; i < nrows; ++i) CGO_CHECK(rowptr[i] <= rowptr[i + 1], "rowptr not monotone at row %lld", (long long)i);
+    for (int64_t p = 0; p < nnz; ++p) CGO_CHECK(col[p] >= 0 && col[p] < ncols, "column index out of range at entry %lld", (long long)p);
     return 0;
 }
 
@@ -1509,10 +1703,8 @@ extern "C" int cgo_obj_sparse_ls_create_csr(cgo_ctx *ctx, int64_t nrows, int64_t
     CGO_CHECK(ctx && rowptr && b && out, "NULL argument");
     CGO_CHECK(ctx->nranks == 1, "cgo_obj_sparse_ls_create_csr is single-GPU");
     CGO_CHECK(nrows >= 1 && ncols >= 1, "empty matrix");
+    CGO_TRY(check_host_csr(nrows, ncols, rowptr, col, val));
     const int64_t nnz = rowptr[nrows];
-    CGO_CHECK(nnz == 0 || (col && val), "NULL col/val");
-    for (int64_t i = 0; i < nrows; ++i) CGO_CHECK(rowptr[i] <= rowptr[i + 1], "rowptr not monotone at row %lld", (long long)i);
-    for (int64_t p = 0; p < nnz; ++p) CGO_CHECK(col[p] >= 0 && col[p] < ncols, "column index out of range at entry %lld", (long long)p);
     CGO_CUDA(cudaSetDevice(ctx->device));
     CsrObj *o = new CsrObj();
     o->ctx = ctx; o->n_global = ncols; o->n_local = ncols; o->offset = 0; o->nrows = nrows; o->halo = 0;
@@ -1573,6 +1765,38 @@ struct LrFeatFin {                  // key = global entry index of the generator
     }
 };
 
+// column blocks, kernel family and layout of a logistic regression's A (samples × all features) and Aᵀ (both
+// constructors).  `long_rows`: rows were taken out of A or Aᵀ (split_long_rows), which only k_spmv_direct adds back.
+static int lr_layout(cgo_ctx *ctx, CsrObj *o, bool long_rows) {
+    const int R = ctx->nranks;
+    // K_b gathers over all d features, K_c over all N samples.  Column blocks are k_spmv_direct passes: the
+    // forced k_csr_rows (CGO_CSR_MODE=1) runs single-pass whatever the gather range
+    if (ctx->csr_mode != 1) {
+        CGO_TRY(build_blocked(ctx, o->A, o->n_global, o->Ab));
+        CGO_TRY(build_blocked(ctx, o->AT, o->nsamples, o->ATb));
+    }
+    const bool blocked = !o->Ab.blk.empty() || !o->ATb.blk.empty();
+    if (blocked && o->A.nnz > (int64_t)200000000 / R) {
+        // production sizes: drop the single-pass copies (only the CSR test hooks read them)
+        if (!o->Ab.blk.empty()) { cudaFree(o->A.col); cudaFree(o->A.val); o->A.col = nullptr; o->A.val = nullptr; }
+        if (!o->ATb.blk.empty()) { cudaFree(o->AT.col); cudaFree(o->AT.val); o->AT.col = nullptr; o->AT.val = nullptr; }
+        o->have_unblocked = false;
+    }
+    // uniformly random columns: gather-bound (k_spmv_direct + BLAS-1 epilogues) whenever the gathers are what
+    // costs — column-blocked sizes, and always when sharded
+    o->direct = ctx->csr_mode != 1 && (R > 1 || blocked || ctx->csr_mode == 2 || long_rows);
+    if (o->direct) {
+        if (o->Ab.blk.empty()) CGO_TRY(csr_make_sliced(ctx, o->A));
+        if (o->ATb.blk.empty()) CGO_TRY(csr_make_sliced(ctx, o->AT));
+        for (auto &m : o->Ab.blk) CGO_TRY(csr_make_sliced(ctx, m));
+        for (auto &m : o->ATb.blk) CGO_TRY(csr_make_sliced(ctx, m));
+        // a matrix left without entries (every row long) has nothing to reorder: its empty rows are stored as zeros
+        if (o->A.nnz == 0) o->A.sliced = 1;
+        if (o->AT.nnz == 0) o->AT.sliced = 1;
+    }
+    return 0;
+}
+
 extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t d, int32_t K, uint64_t seed,
                                                double lambda, cgo_obj **out) {
     CGO_CHECK(ctx && out, "NULL argument");
@@ -1620,28 +1844,7 @@ extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t 
             LrFeatFin fin{sp};
             CGO_TRY(build_transpose(ctx, src, fin, fhi - flo, o->AT));
         }
-        // K_b gathers over all d features, K_c over all N samples.  Column blocks are k_spmv_direct passes: the
-        // forced k_csr_rows (CGO_CSR_MODE=1) runs single-pass whatever the gather range
-        if (ctx->csr_mode != 1) {
-            CGO_TRY(build_blocked(ctx, o->A, d, o->Ab));
-            CGO_TRY(build_blocked(ctx, o->AT, N, o->ATb));
-        }
-        const bool blocked = !o->Ab.blk.empty() || !o->ATb.blk.empty();
-        if (blocked && o->A.nnz > (int64_t)200000000 / R) {
-            // production sizes: drop the single-pass copies (only the CSR test hooks read them)
-            if (!o->Ab.blk.empty()) { cudaFree(o->A.col); cudaFree(o->A.val); o->A.col = nullptr; o->A.val = nullptr; }
-            if (!o->ATb.blk.empty()) { cudaFree(o->AT.col); cudaFree(o->AT.val); o->AT.col = nullptr; o->AT.val = nullptr; }
-            o->have_unblocked = false;
-        }
-        // uniformly random columns: gather-bound (k_spmv_direct + BLAS-1 epilogues) whenever the gathers are what
-        // costs — column-blocked sizes, and always when sharded
-        o->direct = ctx->csr_mode != 1 && (R > 1 || blocked || ctx->csr_mode == 2);
-        if (o->direct) {
-            if (o->Ab.blk.empty()) CGO_TRY(csr_make_sliced(ctx, o->A));
-            if (o->ATb.blk.empty()) CGO_TRY(csr_make_sliced(ctx, o->AT));
-            for (auto &m : o->Ab.blk) CGO_TRY(csr_make_sliced(ctx, m));
-            for (auto &m : o->ATb.blk) CGO_TRY(csr_make_sliced(ctx, m));
-        }
+        CGO_TRY(lr_layout(ctx, o, false));
         if (o->lr_sharded) {
             const size_t xb = sizeof(double) * (size_t)(d + CSR_PAD), cb = sizeof(double) * (size_t)(N + CSR_PAD);
             if (ctx->peer_ok) {
@@ -1676,6 +1879,49 @@ extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t 
     return 0;
 }
 
+extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, const int64_t *rowptr, const int32_t *col,
+                                         const double *val, const double *y, double lambda, cgo_obj **out) {
+    CGO_CHECK(ctx && rowptr && y && out, "NULL argument");
+    CGO_CHECK(ctx->nranks == 1, "cgo_obj_logreg_create_csr is single-GPU");
+    CGO_CHECK(N >= 1 && d >= 1, "logreg: need nsamples >= 1 and nfeat >= 1 (nsamples=%lld, nfeat=%lld)", (long long)N, (long long)d);
+    CGO_TRY(check_i32(N, "nsamples"));
+    CGO_TRY(check_i32(d, "nfeat"));
+    CGO_CHECK(rowptr[0] == 0, "rowptr[0] = %lld: row pointers are 0-based", (long long)rowptr[0]);
+    CGO_TRY(check_host_csr(N, d, rowptr, col, val));
+    for (int64_t i = 0; i < N; ++i) CGO_CHECK(y[i] == 1.0 || y[i] == -1.0, "label %g of sample %lld is not +1 or -1", y[i], (long long)i);
+    CGO_CHECK(std::isfinite(lambda) && lambda >= 0.0, "logreg: lambda = %g must be finite and >= 0", lambda);
+    CGO_CUDA(cudaSetDevice(ctx->device));
+    const int64_t nnz = rowptr[N];
+    CsrObj *o = new CsrObj();
+    o->ctx = ctx; o->logreg = true; o->lambda = lambda; o->nsamples = N;
+    o->n_global = d; o->n_local = d; o->offset = 0; o->nrows = N; o->halo = 0;
+    auto body = [&]() -> int {
+        cudaStream_t s = ctx->stream;
+        CGO_TRY(csr_alloc(o->A, N, nnz));
+        CGO_CUDA(cudaMemcpyAsync(o->A.rowptr, rowptr, sizeof(int64_t) * (size_t)(N + 1), cudaMemcpyHostToDevice, s));
+        if (nnz) {
+            CGO_CUDA(cudaMemcpyAsync(o->A.col, col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, s));
+            CGO_CUDA(cudaMemcpyAsync(o->A.val, val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, s));
+        }
+        CGO_CUDA(cudaMalloc(&o->b, sizeof(double) * (size_t)(N + CSR_PAD)));
+        CGO_CUDA(cudaMemsetAsync(o->b, 0, sizeof(double) * (size_t)(N + CSR_PAD), s));
+        CGO_CUDA(cudaMemcpyAsync(o->b, y, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, s));
+        CGO_TRY(o->alloc_r());
+        CsrSrc src{o->A.col, nnz};
+        CsrFin fin{o->A.rowptr, N, o->A.val};
+        CGO_TRY(build_transpose(ctx, src, fin, d, o->AT));
+        if (ctx->csr_mode != 1) {            // k_csr_rows keeps every row (sequential sums)
+            CGO_TRY(split_long_rows(ctx, o->A, o->LA));
+            CGO_TRY(split_long_rows(ctx, o->AT, o->LAT));
+        }
+        return lr_layout(ctx, o, o->LA.n > 0 || o->LAT.n > 0);
+    };
+    int rc = body();
+    if (rc) { delete o; return rc; }
+    *out = o;
+    return 0;
+}
+
 // ------------------------------------------------------------------ test hooks
 static CsrObj *as_csr(cgo_obj *o) { return dynamic_cast<CsrObj *>(o); }
 
@@ -1691,16 +1937,12 @@ extern "C" int cgo_obj_csr_nnz(cgo_obj *obj, int transposed, int64_t *nrows, int
     CGO_CHECK(o != nullptr, "not a CSR objective");
     const CsrMat &M = transposed ? o->AT : o->A;
     if (nrows) *nrows = M.nrows;
-    if (nnz) *nnz = M.nnz;
+    if (nnz) *nnz = M.nnz + (transposed ? o->LAT : o->LA).M.nnz;
     return 0;
 }
-extern "C" int cgo_obj_csr_download(cgo_obj *obj, int transposed, int64_t *rowptr, int32_t *col, double *val, double *b) {
-    CsrObj *o = as_csr(obj);
-    CGO_CHECK(o != nullptr, "not a CSR objective");
-    CGO_CHECK(o->have_unblocked, "the single-pass CSR copy was dropped at this size (column-blocked storage only)");
-    const CsrMat &M = transposed ? o->AT : o->A;
-    cudaStream_t s = o->ctx->stream;
-    CGO_CUDA(cudaSetDevice(o->ctx->device));
+// M row-major on the host (any of the three may be NULL)
+static int csr_download_mat(cgo_ctx *c, const CsrMat &M, int64_t *rowptr, int32_t *col, double *val) {
+    cudaStream_t s = c->stream;
     if (rowptr) CGO_CUDA(cudaMemcpyAsync(rowptr, M.rowptr, sizeof(int64_t) * (size_t)(M.nrows + 1), cudaMemcpyDeviceToHost, s));
     int32_t *ctmp = nullptr; double *vtmp = nullptr;          // row-major copies of a sliced matrix
     auto body = [&]() -> int {
@@ -1708,19 +1950,56 @@ extern "C" int cgo_obj_csr_download(cgo_obj *obj, int transposed, int64_t *rowpt
         if (M.sliced && M.nnz && (col || val)) {
             CGO_CUDA(cudaMalloc(&ctmp, sizeof(int32_t) * (size_t)M.nnz));
             CGO_CUDA(cudaMalloc(&vtmp, sizeof(double) * (size_t)M.nnz));
-            k_slice_permute<<<grid_for((M.nrows + 31) / 32 * 32, o->ctx->sms), 256, 0, s>>>(M, M.col, M.val, ctmp, vtmp, true);
+            k_slice_permute<<<grid_for((M.nrows + 31) / 32 * 32, c->sms), 256, 0, s>>>(M, M.col, M.val, ctmp, vtmp, true);
             CGO_CUDA(cudaGetLastError());
             csrc = ctmp; vsrc = vtmp;
         }
         if (col && M.nnz) CGO_CUDA(cudaMemcpyAsync(col, csrc, sizeof(int32_t) * (size_t)M.nnz, cudaMemcpyDeviceToHost, s));
         if (val && M.nnz) CGO_CUDA(cudaMemcpyAsync(val, vsrc, sizeof(double) * (size_t)M.nnz, cudaMemcpyDeviceToHost, s));
-        if (b) CGO_CUDA(cudaMemcpyAsync(b, o->b, sizeof(double) * (size_t)o->nrows, cudaMemcpyDeviceToHost, s));
         CGO_CUDA(cudaStreamSynchronize(s));
         return 0;
     };
     int rc = body();
     cudaFree(ctmp); cudaFree(vtmp);
     return rc;
+}
+// the whole matrix: M with the long rows of L put back in their places
+static int csr_download_whole(cgo_ctx *c, const CsrMat &M, const LongRows &L, int64_t *rowptr, int32_t *col, double *val) {
+    if (L.n == 0) return csr_download_mat(c, M, rowptr, col, val);
+    std::vector<int64_t> rp((size_t)M.nrows + 1);
+    std::vector<int32_t> ci((size_t)M.nnz), lc((size_t)L.M.nnz);
+    std::vector<double> va((size_t)M.nnz), lv((size_t)L.M.nnz);
+    CGO_TRY(csr_download_mat(c, M, rp.data(), ci.data(), va.data()));
+    CGO_TRY(csr_download_mat(c, L.M, nullptr, lc.data(), lv.data()));
+    int64_t q = 0, r = 0;
+    for (int64_t i = 0; i < M.nrows; ++i) {
+        if (rowptr) rowptr[i] = q;
+        int64_t p0 = rp[(size_t)i], p1 = rp[(size_t)i + 1];
+        const int32_t *cs = ci.data(); const double *vs = va.data();
+        if (r < L.n && L.h_row[(size_t)r] == i) {
+            p0 = L.h_rowptr[(size_t)r]; p1 = L.h_rowptr[(size_t)r + 1];
+            cs = lc.data(); vs = lv.data();
+            ++r;
+        }
+        for (int64_t p = p0; p < p1; ++p, ++q) {
+            if (col) col[q] = cs[p];
+            if (val) val[q] = vs[p];
+        }
+    }
+    if (rowptr) rowptr[M.nrows] = q;
+    return 0;
+}
+extern "C" int cgo_obj_csr_download(cgo_obj *obj, int transposed, int64_t *rowptr, int32_t *col, double *val, double *b) {
+    CsrObj *o = as_csr(obj);
+    CGO_CHECK(o != nullptr, "not a CSR objective");
+    CGO_CHECK(o->have_unblocked, "the single-pass CSR copy was dropped at this size (column-blocked storage only)");
+    CGO_CUDA(cudaSetDevice(o->ctx->device));
+    CGO_TRY(csr_download_whole(o->ctx, transposed ? o->AT : o->A, transposed ? o->LAT : o->LA, rowptr, col, val));
+    if (b) {
+        CGO_CUDA(cudaMemcpyAsync(b, o->b, sizeof(double) * (size_t)o->nrows, cudaMemcpyDeviceToHost, o->ctx->stream));
+        CGO_CUDA(cudaStreamSynchronize(o->ctx->stream));
+    }
+    return 0;
 }
 // y = A x (transposed: Aᵀ x) through the production kernel; single GPU (no halo)
 extern "C" int cgo_obj_spmv(cgo_obj *obj, int transposed, const double *x_host, double *y_host) {
@@ -1743,6 +2022,7 @@ extern "C" int cgo_obj_spmv(cgo_obj *obj, int transposed, const double *x_host, 
             EpiStore es{dy};
             CGO_TRY(launch_csr(c, M, dx, es, cgo_red_args(c, CGO_PACK_LEN - 1), transposed ? CGO_T_SPMVT : CGO_T_SPMV));
         }
+        CGO_TRY(long_rows_sum(c, transposed ? o->LAT : o->LA, dx, dy, transposed ? CGO_T_SPMVT : CGO_T_SPMV));
         CGO_CUDA(cudaMemcpyAsync(y_host, dy, sizeof(double) * (size_t)nout, cudaMemcpyDeviceToHost, c->stream));
         CGO_CUDA(cudaStreamSynchronize(c->stream));
         return 0;

@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _capi as capi
 from ._capi import (D_GU, D_UU, P_DIR_GU, P_DIR_UU, P_DPHI, P_GPG, P_GPGP, P_PHI, P_UG, P_UU, P_UY, P_YGP, P_YY,
-                    PACK_LEN, check, dptr, lib)
+                    PACK_LEN, CgoError, check, dptr, lib)
 
 f64 = np.float64
 
@@ -299,6 +299,26 @@ def LogRegGPU(nsamples: int, nfeat: int, nnz_per_row: int = 20, seed: int = 24, 
     ctx = ctx or default_context()
     h = C.c_void_p()
     check(lib().cgo_obj_logreg_create_synthetic(ctx.h, nsamples, nfeat, nnz_per_row, seed, lam, C.byref(h)))
+    return DeviceObjective(ctx, h)
+
+
+def LogRegGPU_from_csr(nsamples, nfeat, rowptr, col, val, y, lam: float = 1e-6,
+                       ctx: Optional[Context] = None) -> DeviceObjective:
+    """(1/N) Σ log(1 + exp(−y_i a_i·w)) + (λ/2)‖w‖² on the caller's CSR (0-based int64 row pointers, int32 columns)
+    and labels y_i ∈ {−1, +1}; single GPU.  An intercept is a column of ones in every row, and λ penalises its
+    weight like the others."""
+    ctx = ctx or default_context()
+    rowptr = np.ascontiguousarray(rowptr, dtype=np.int64)
+    col = np.ascontiguousarray(col, dtype=np.int32)
+    val = np.ascontiguousarray(val, dtype=np.float64)
+    y = np.ascontiguousarray(y, dtype=np.float64)
+    if rowptr.size != nsamples + 1 or y.size != nsamples:
+        raise CgoError(f"rowptr needs nsamples + 1 = {nsamples + 1} entries and y nsamples (got {rowptr.size}, {y.size})")
+    if col.size < rowptr[-1] or val.size < rowptr[-1]:
+        raise CgoError(f"col and val need rowptr[-1] = {rowptr[-1]} entries (got {col.size}, {val.size})")
+    h = C.c_void_p()
+    check(lib().cgo_obj_logreg_create_csr(ctx.h, nsamples, nfeat, rowptr.ctypes.data, col.ctypes.data,
+                                          val.ctypes.data, y.ctypes.data, lam, C.byref(h)))
     return DeviceObjective(ctx, h)
 
 

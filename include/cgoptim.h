@@ -25,6 +25,10 @@
  *   +0.0; the 256 lanes of a virtual CTA are combined by a xor-butterfly (16,8,4,2,1) inside
  *   each warp, then sequentially over the 8 warps; the min(G, ntiles) CTA partials are combined
  *   by the last-arriving block in exactly the same way (lane t takes partials t, t+256, ...).
+ *   Long rows (logistic regression from a host CSR, cgo_obj_logreg_create_csr, on the k_spmv_direct family): a row
+ *   of A or Aᵀ with more than CGO_LONG_ROW entries is summed in this order too — its products val_k · x[col_k], k in
+ *   storage order, are the items, with V=1, U=4 and the ctx's G.  Every other row of every CSR matrix is summed
+ *   sequentially in storage order.
  *   CSR matrices whose gathers do not coalesce (the synthetic least-squares matrix with coh_log2 < 4; a host
  *   CSR whose warp-level gathers touch more than four lines on average: cgo_obj_reduction_site tells) are
  *   multiplied by a kernel without reductions, and their dots come from BLAS-1 passes (V=2, U=4).
@@ -158,6 +162,15 @@ int cgo_obj_sparse_ls_create_csr(cgo_ctx *ctx, int64_t nrows, int64_t ncols, con
 int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat,
                                     int32_t nnz_per_row, uint64_t seed, double lambda,
                                     cgo_obj **out);
+/* rows of more than CGO_LONG_ROW entries (an intercept's column of ones is a row of Aᵀ with nsamples entries) are
+ * summed by the whole grid in the canonical order instead of on one lane (see the canonical reduction order above) */
+#define CGO_LONG_ROW 1024
+/* (1/N) Σ log(1 + exp(−y_i a_i·w)) + (λ/2)‖w‖² from a host CSR (int64 row pointers, int32 columns, 0-based), labels
+ * y_i ∈ {−1, +1}; single GPU.  An intercept is a column of ones, and λ penalises it like every other weight.  Every
+ * matrix with a row longer than CGO_LONG_ROW runs on k_spmv_direct; forced onto k_csr_rows (cgo_ctx_set_csr_mode 1)
+ * it keeps sequential row sums, exact but slow on long rows. */
+int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, const int64_t *rowptr,
+                              const int32_t *col, const double *val, const double *y, double lambda, cgo_obj **out);
 /* t·f0(x) − Σ log(ubs − x) − Σ log(x − lbs) around `inner` (which must outlive it): evalbarrier!
  * (src/engine/primal_barrier.jl:112-133) with the box constraints of examples/constrained.jl:17-47;
  * lbs / ubs are this rank's shard.  cgo_obj_barrier_set_t changes t between centering steps (:246);

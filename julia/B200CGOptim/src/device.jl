@@ -115,6 +115,16 @@ function LogRegGPU(nsamples::Integer, nfeat::Integer, ctx::Context; nnz_per_row 
         (Ptr{Cvoid}, Int64, Int64, Int32, UInt64, Float64, Ref{Ptr{Cvoid}}), ctx.h, nsamples, nfeat, nnz_per_row, seed, λ, h))
     return _wrap(ctx, h[])
 end
+"CSR logistic regression on the caller's CSR (0-based int64 row pointers, int32 columns) and labels ±1; single GPU.
+An intercept is a column of ones, and λ penalises its weight like the others."
+function LogRegGPU(nsamples::Integer, nfeat::Integer, rowptr::Vector{Int64}, col::Vector{Int32},
+                   val::Vector{Float64}, y::Vector{Float64}, ctx::Context; λ = 1e-6)
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:cgo_obj_logreg_create_csr, LIBCGOPTIM[]), Cint,
+        (Ptr{Cvoid}, Int64, Int64, Ptr{Int64}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Float64, Ref{Ptr{Cvoid}}),
+        ctx.h, nsamples, nfeat, rowptr, col, val, y, λ, h))
+    return _wrap(ctx, h[])
+end
 
 "Token for one of the device vectors of a workspace (keeps the reference's call shapes)."
 struct DeviceVector{W}
