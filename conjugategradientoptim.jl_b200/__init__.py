@@ -21,6 +21,6 @@ from .engine import (BoxConstraint, CvxInequalityConstraint, LinesearchSolveSys,
                      setupLinesearchSolveSys, setupPrimalBarrierConfig, solvesystem, verifyt0)
 from .engine.optim import linesearch_  # noqa: F401
 from .device import (Context, DeviceLineSearchContainer, DeviceObjective, DeviceStart, DeviceVector,  # noqa: F401
-                     BoxBarrierGPU, LogRegGPU, LogRegGPU_from_csr, RosenbrockChainedGPU, RosenbrockGPU, SparseLSGPU, SparseLSGPU_from_csr, UserObjectiveGPU, default_context,
+                     BoxBarrierGPU, LogRegGPU, LogRegGPU_from_csr, RosenbrockChainedGPU, RosenbrockGPU, SoftmaxRegGPU_from_csr, SparseLSGPU, SparseLSGPU_from_csr, UserObjectiveGPU, default_context,
                      dot, shard_range, BatchedResults, minimizeobjective_batched, batched_lanes)
 from .device import DeviceLineSearchContainer as LineSearchContainer  # noqa: F401

@@ -390,6 +390,38 @@ struct LogitLoss {
     }
 };
 
+// softmax regression (csr.cu eval_trial_softmax): Z (N × K, row-major) → C = P − Y in place; Σ ℓ.  The items are the
+// samples, V = 2 as LogitLoss.  Sample i, sequentially over k: m = max z_ik; s = Σ exp(z_ik − m) from +0.0;
+// ℓ = (m + log s) − z_{i,y_i}; c_ik = exp(z_ik − m) / s − [k = y_i].  NaN and Inf pass through.
+struct SoftmaxLoss {
+    static constexpr int TCLASS = CGO_T_OTHER;
+    static constexpr int K = 1;
+    static constexpr int OCC = 2;
+    struct In { double2 y; };
+    double *zc;
+    const double2 *y;
+    int nc;
+    __device__ __forceinline__ void prologue() {}
+    __device__ __forceinline__ In load(int64_t q) const { return In{cgo_ld2(y + q)}; }
+    __device__ __forceinline__ void one(int64_t i, double yy, double (&acc)[K]) const {
+        double *z = zc + i * nc;
+        const int lab = (int)yy;
+        double m = z[0];
+        for (int k = 1; k < nc; ++k) { const double v = z[k]; m = v > m ? v : m; }
+        double s = 0.0;
+        for (int k = 0; k < nc; ++k) s = s + exp(z[k] - m);
+        acc[0] = acc[0] + ((m + log(s)) - z[lab]);
+        for (int k = 0; k < nc; ++k) {
+            const double p = exp(z[k] - m) / s;
+            z[k] = k == lab ? p - 1.0 : p;
+        }
+    }
+    __device__ __forceinline__ void apply(int64_t q, const In &in, double (&acc)[K], bool v2) const {
+        one(2 * q, in.y.x, acc);
+        if (v2) one(2 * q + 1, in.y.y, acc);
+    }
+};
+
 // updateiteratesolvesys! (src/engine/solve_system.jl:237-253): x_next[i] = base[i] + m*df_xp[i]
 // (base = x_next itself as the reference writes it, or x for Alg. 3.1 as published)
 struct SolveSysProject {
@@ -1169,6 +1201,11 @@ int cgo_blas1_logit(cgo_ctx *c, double *zc, const double *y, int64_t n, int slot
     LogitLoss<false> op;
     op.zc = (double2 *)zc; op.y = (const double2 *)y; op.dst_all = nullptr; op.nranks = 1;
     return launch_blas1(c, op, n, red);
+}
+int cgo_blas1_softmax(cgo_ctx *c, double *zc, const double *y, int64_t n, int nclass, int slot) {
+    SoftmaxLoss op;
+    op.zc = zc; op.y = (const double2 *)y; op.nc = nclass;
+    return launch_blas1(c, op, n, cgo_red_args(c, slot));
 }
 int cgo_blas1_grad_dots(cgo_state *st) {
     GradDots op;

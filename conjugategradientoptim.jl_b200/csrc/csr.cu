@@ -664,6 +664,95 @@ static int launch_direct(cgo_ctx *c, const CsrMat &A, const double *xg, const F 
     return launch_direct_k<F, 10, 4>(c, A, xg, f, da, tclass);
 }
 
+// ------------------------------------------------------------------ the K-column SpMM (softmax regression)
+// Y = A X with X (ncols × K) and Y (nrows × K) row-major: the SpMV of A ⊗ I_K on the flat vectors, whose row
+// (i, k) holds row i's entries in storage order at columns col·K + k.  A group of GW = 2^gw_log2 lanes owns one
+// row, lane k of the group one class (class tiles of 32 when K > 32).  The group's lanes read each entry's column
+// index and value from the same address (one request per group, once per class tile) and gather x[col·K + k]:
+// one gather instruction reads whole contiguous segments.  Each (row, class) sum is added entry by entry in
+// storage order from f.init(i·K + k), so it is bit for bit the row sum k_spmv_direct makes of the expanded matrix,
+// and column-block passes chain through DirStoreInit as they do there.  Plain row-major CSR (no sliced layout).
+// Work units (32 / GW rows, one class tile) come from the slice queue of k_spmv_direct.
+constexpr int MM_UN = 8;                    // entries per batch whose loads are in flight together
+constexpr int MM_OCC = 4;
+template <class F>
+__global__ void __launch_bounds__(CGO_B, MM_OCC)
+k_spmm_direct(CsrMat A, int K, int gw_log2, const double *__restrict__ xg, F f, DirArgs da) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int gw = 1 << gw_log2, rpw = 32 >> gw_log2;
+    const int sub = lane >> gw_log2, kl = lane & (gw - 1);
+    const int nct = (K + gw - 1) >> gw_log2;
+    const int64_t nrows = A.nrows, nunits = (nrows + rpw - 1) / rpw * nct;
+    const uint64_t gpol = l2_policy_evict_last();
+    for (;;) {
+        unsigned long long s0 = 0;
+        if (lane == 0) s0 = atomicAdd(da.next, (unsigned long long)DIR_GRAB);
+        s0 = __shfl_sync(0xffffffffu, s0, 0);
+        if ((int64_t)s0 >= nunits) break;
+#pragma unroll 1
+        for (int g = 0; g < DIR_GRAB; ++g) {
+            const int64_t s = (int64_t)s0 + g;
+            if (s >= nunits) break;
+            const int64_t rg = s / nct;
+            const int k = (int)(s - rg * nct) * gw + kl;
+            const int64_t row = rg * rpw + sub;
+            const bool inrow = row < nrows, valid = inrow && k < K;
+            int64_t rp0 = 0;
+            int len = 0;
+            if (inrow) { rp0 = __ldg(A.rowptr + row); len = (int)(__ldg(A.rowptr + row + 1) - rp0); }
+            const int maxlen = __reduce_max_sync(0xffffffffu, len);
+            const int64_t y = row * K + k;
+            double sum = valid ? f.init(y) : 0.0;
+            for (int k0 = 0; k0 < maxlen; k0 += MM_UN) {
+                int32_t cj[MM_UN];
+                double vj[MM_UN], xj[MM_UN];
+#pragma unroll
+                for (int j = 0; j < MM_UN; ++j) {
+                    const bool on = len > k0 + j;
+                    cj[j] = ld_stream_s32_if(A.col + rp0 + k0 + j, on);
+                    vj[j] = ld_stream_f64_if(A.val + rp0 + k0 + j, on);
+                }
+#pragma unroll
+                for (int j = 0; j < MM_UN; ++j) xj[j] = ld_gather_f64_if(xg + (int64_t)cj[j] * K + k, gpol, valid && len > k0 + j);
+#pragma unroll
+                for (int j = 0; j < MM_UN; ++j) {
+                    const double p = vj[j] * xj[j];
+                    if (len > k0 + j) sum = sum + p;
+                }
+            }
+            if (valid) f.row(y, sum);
+        }
+    }
+    // the last CTA re-arms the queue
+    __shared__ bool is_last;
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) is_last = atomicAdd(da.ticket, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (is_last && tid == 0) {
+        *da.ticket = 0u;
+        *da.next = 0ULL;
+        __threadfence();
+    }
+}
+template <class F>
+static int launch_spmm(cgo_ctx *c, const CsrMat &A, int K, const double *xg, const F &f, int tclass) {
+    CGO_CHECK(!A.sliced && K >= 1, "internal: k_spmm_direct needs a row-major matrix");
+    int gw_log2 = 0;
+    while ((1 << gw_log2) < K && gw_log2 < 5) ++gw_log2;
+    const int64_t nct = (K + (1 << gw_log2) - 1) >> gw_log2;
+    const int64_t nunits = (A.nrows + (32 >> gw_log2) - 1) / (32 >> gw_log2) * nct;
+    int64_t want = (nunits + 8 * DIR_GRAB - 1) / (8 * DIR_GRAB), phys = (int64_t)c->sms * MM_OCC;
+    int grid = (int)(want < phys ? want : phys);
+    if (grid < 1) grid = 1;
+    cgo_timer_begin(c, tclass);
+    k_spmm_direct<F><<<grid, CGO_B, 0, c->stream>>>(A, K, gw_log2, xg, f, dir_args(c));
+    cgo_timer_end(c);
+    c->launches++;
+    CGO_CUDA(cudaGetLastError());
+    return 0;
+}
+
 // ------------------------------------------------------------------ counter-based hash
 // (generator spec: oracle/cgo_oracle.c hash3 / u01; restated, identical arithmetic)
 __host__ __device__ __forceinline__ uint64_t g_mix64(uint64_t z) {
@@ -1083,9 +1172,10 @@ __global__ void k_blk_copy(CsrMat A, const int64_t *first, CsrMat B) {
         for (int64_t e = 0; e < n; ++e) { B.col[d0 + e] = A.col[s0 + e]; B.val[d0 + e] = A.val[s0 + e]; }
     }
 }
-static int build_blocked(cgo_ctx *c, const CsrMat &A, int64_t ncols, CsrBlocked &out) {
+// `width`: doubles gathered per column (1 for an SpMV, K for the K-column SpMM)
+static int build_blocked(cgo_ctx *c, const CsrMat &A, int64_t ncols, int64_t width, CsrBlocked &out) {
     out.free_all();
-    const int64_t cap = (int64_t)(c->gather_block_bytes / sizeof(double));
+    const int64_t cap = (int64_t)(c->gather_block_bytes / (sizeof(double) * (size_t)width));
     if (cap <= 0 || ncols <= cap || A.nnz == 0) return 0;
     const int64_t nb = (ncols + cap - 1) / cap;
     const int64_t bc = (((ncols + nb - 1) / nb) + 1) & ~(int64_t)1;
@@ -1144,6 +1234,15 @@ static int spmv_direct_passes(cgo_ctx *c, const CsrMat &M, const CsrBlocked &B, 
     }
     return 0;
 }
+// the same for the K-column SpMM (row-major blocks)
+static int spmm_passes(cgo_ctx *c, const CsrMat &M, const CsrBlocked &B, int K, const double *xg, double *out, int tclass) {
+    if (B.blk.empty()) return launch_spmm(c, M, K, xg, DirStore{out}, tclass);
+    for (size_t j = 0; j < B.blk.size(); ++j) {
+        if (j == 0) CGO_TRY(launch_spmm(c, B.blk[j], K, xg, DirStore{out}, tclass));
+        else CGO_TRY(launch_spmm(c, B.blk[j], K, xg, DirStoreInit{out, out}, tclass));
+    }
+    return 0;
+}
 
 // ------------------------------------------------------------------ long rows (logistic regression from a host CSR)
 // A row with more than CGO_LONG_ROW entries would chain its products on one lane of k_spmv_direct: the ones column
@@ -1162,10 +1261,11 @@ struct LongRows {
     int64_t *row = nullptr;                  // their indices in the whole matrix (device)
     std::vector<int64_t> h_row, h_rowptr;    // host copies of `row` and M.rowptr
     int G = 0;                               // the G the work units are laid out for
+    int width = 1;                           // sums per long row (K for the K-column SpMM)
     int64_t nunits = 0;
     int2 *unit = nullptr;                    // (long row, virtual CTA) of every unit
     int64_t *ubase = nullptr;                // first unit of every long row, n + 1
-    double *partial = nullptr;               // one per unit
+    double *partial = nullptr;               // `width` per unit
     void free_all() {
         csr_free(M);
         cudaFree(row); cudaFree(unit); cudaFree(ubase); cudaFree(partial);
@@ -1235,7 +1335,7 @@ static int long_units(cgo_ctx *c, LongRows &L) {
     L.unit = nullptr; L.partial = nullptr; L.G = 0;
     L.nunits = (int64_t)unit.size();
     CGO_CUDA(cudaMalloc(&L.unit, sizeof(int2) * unit.size()));
-    CGO_CUDA(cudaMalloc(&L.partial, sizeof(double) * unit.size()));
+    CGO_CUDA(cudaMalloc(&L.partial, sizeof(double) * unit.size() * (size_t)L.width));
     CGO_CUDA(cudaMemcpyAsync(L.unit, unit.data(), sizeof(int2) * unit.size(), cudaMemcpyHostToDevice, c->stream));
     CGO_CUDA(cudaMemcpyAsync(L.ubase, ubase.data(), sizeof(int64_t) * ubase.size(), cudaMemcpyHostToDevice, c->stream));
     CGO_CUDA(cudaStreamSynchronize(c->stream));
@@ -1255,6 +1355,90 @@ static int long_rows_sum(cgo_ctx *c, LongRows &L, const double *xg, double *out,
     CGO_CUDA(cudaGetLastError());
     cgo_timer_begin(c, tclass);
     k_long_finish<<<(unsigned)L.n, CGO_B, 0, c->stream>>>(L.ubase, L.row, L.partial, out);
+    cgo_timer_end(c);
+    c->launches++;
+    CGO_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// The long rows of the K-column SpMM: for every class k the items of a long row are val_p · x[col_p·K + k], summed
+// exactly as k_long_rows + k_long_finish sum that row of A ⊗ I_K.  The (long row, virtual CTA) units are those of
+// the SpMV; k_long_rows_k spreads (unit, tile of LONG_KT classes) over the grid, so each lane reads its entries once
+// per class tile and keeps LONG_KT accumulators, and the CTA combine reduces each of them as it reduces one.
+// Partials are stored unit-major, K per unit; k_long_finish_k runs one CTA per (long row, class).
+constexpr int LONG_KT = 8;
+__global__ void __launch_bounds__(CGO_B) k_long_rows_k(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G, int K,
+                                                       const double *__restrict__ xg, double *__restrict__ partial) {
+    __shared__ double s_red[LONG_KT * CGO_NW];
+    const int t = threadIdx.x;
+    const uint64_t gpol = l2_policy_evict_last();
+    const int nct = (K + LONG_KT - 1) / LONG_KT;
+    for (int64_t wi = blockIdx.x; wi < nunits * nct; wi += gridDim.x) {
+        const int64_t u = wi / nct;
+        const int k0 = (int)(wi - u * nct) * LONG_KT;
+        const int2 w = unit[u];
+        const int64_t p0 = L.rowptr[w.x], len = L.rowptr[w.x + 1] - p0;
+        const int64_t ntiles = (len + LONG_TILE - 1) / LONG_TILE;
+        double acc[LONG_KT];
+#pragma unroll
+        for (int kk = 0; kk < LONG_KT; ++kk) acc[kk] = 0.0;
+#pragma unroll 1
+        for (int64_t tile = w.y; tile < ntiles; tile += G) {
+            int32_t cj[LONG_U];
+            double vj[LONG_U];
+            bool on[LONG_U];
+#pragma unroll
+            for (int j = 0; j < LONG_U; ++j) {
+                const int64_t k = tile * LONG_TILE + j * CGO_B + t;
+                on[j] = k < len;
+                cj[j] = ld_stream_s32_if(L.col + p0 + k, on[j]);
+                vj[j] = ld_stream_f64_if(L.val + p0 + k, on[j]);
+            }
+            double xj[LONG_U][LONG_KT];
+#pragma unroll
+            for (int j = 0; j < LONG_U; ++j)
+#pragma unroll
+                for (int kk = 0; kk < LONG_KT; ++kk)
+                    xj[j][kk] = ld_gather_f64_if(xg + (int64_t)cj[j] * K + k0 + kk, gpol, on[j] && k0 + kk < K);
+#pragma unroll
+            for (int j = 0; j < LONG_U; ++j)
+#pragma unroll
+                for (int kk = 0; kk < LONG_KT; ++kk) {
+                    const double p = vj[j] * xj[j][kk];
+                    if (on[j]) acc[kk] = acc[kk] + p;
+                }
+        }
+        cgo_cta_combine<LONG_KT>(acc, s_red);
+        if (t == 0) {
+#pragma unroll
+            for (int kk = 0; kk < LONG_KT; ++kk)
+                if (k0 + kk < K) partial[u * K + k0 + kk] = acc[kk];
+        }
+    }
+}
+__global__ void __launch_bounds__(CGO_B) k_long_finish_k(const int64_t *__restrict__ ubase, const int64_t *__restrict__ row, int K,
+                                                         const double *__restrict__ partial, double *out) {
+    __shared__ double s_red[CGO_NW];
+    const int k = (int)blockIdx.y;
+    const int64_t b = ubase[blockIdx.x], nact = ubase[blockIdx.x + 1] - b;
+    double acc[1] = {0.0};
+    for (int64_t c = threadIdx.x; c < nact; c += CGO_B) acc[0] = acc[0] + partial[(b + c) * K + k];
+    cgo_cta_combine<1>(acc, s_red);
+    if (threadIdx.x == 0) out[row[blockIdx.x] * K + k] = acc[0];
+}
+static int long_rows_sum_k(cgo_ctx *c, LongRows &L, const double *xg, double *out, int tclass) {
+    if (L.n == 0) return 0;
+    CGO_TRY(long_units(c, L));
+    const int K = L.width;
+    const int64_t items = L.nunits * ((K + LONG_KT - 1) / LONG_KT), phys = (int64_t)c->sms * 8;
+    const int grid = (int)(items < phys ? items : phys);
+    cgo_timer_begin(c, tclass);
+    k_long_rows_k<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, K, xg, L.partial);
+    cgo_timer_end(c);
+    c->launches++;
+    CGO_CUDA(cudaGetLastError());
+    cgo_timer_begin(c, tclass);
+    k_long_finish_k<<<dim3((unsigned)L.n, (unsigned)K), CGO_B, 0, c->stream>>>(L.ubase, L.row, K, L.partial, out);
     cgo_timer_end(c);
     c->launches++;
     CGO_CUDA(cudaGetLastError());
@@ -1328,6 +1512,9 @@ static int split_long_rows(cgo_ctx *c, CsrMat &A, LongRows &L) {
 // ------------------------------------------------------------------ the objective
 struct CsrObj : cgo_obj {
     bool logreg = false;
+    // classes of the softmax objective (logreg also true): the state vector is W (d × K, feature-major), Z = A W and
+    // C = P − Y live in `r` (N × K, row-major), and every product with A or Aᵀ is the K-column SpMM.  1 otherwise
+    int32_t nclass = 1;
     // the SpMV kernel family of every evaluation, fixed at creation.  false: the fused k_csr_rows, whose epilogues
     // reduce the dots (reduction site V = 1, U = 1).  true: k_spmv_direct on the sliced layout, the dots are
     // BLAS-1 passes (V = 2, U = CGO_U_VEC).  Least squares: A.sliced after set-up; logistic regression: also when
@@ -1378,7 +1565,7 @@ struct CsrObj : cgo_obj {
         cudaFree(xp_full); cudaFree(c_full);
     }
     int alloc_r() {
-        size_t bytes = sizeof(double) * (size_t)(nrows + 2 * halo + 4);
+        size_t bytes = sizeof(double) * (size_t)(nrows * nclass + 2 * halo + 4);
         if (ctx->nranks > 1 && ctx->peer_ok && halo > 0) {
             bytes = sizeof(double) * (size_t)((n_alloc > nrows ? n_alloc : nrows) + 2 * halo + 4);   // rank-independent
             void *p = nullptr;
@@ -1582,6 +1769,18 @@ struct CsrObj : cgo_obj {
         CGO_TRY(launch_csr(ctx, AT, r, e2, cgo_red_args(ctx, CGO_P_DPHI), CGO_T_SPMVT));              // K_c
         return finish_lr(out);
     }
+    // softmax regression, single rank: K_a | SpMM passes of A → Z | softmax + loss (BLAS-1) | SpMM passes of Aᵀ |
+    // /N + λW + dots (BLAS-1)
+    int eval_trial_softmax(cgo_state *st, double a, bool fused, double beta, double *out) {
+        CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                                   // K_a
+        CGO_TRY(spmm_passes(ctx, A, Ab, nclass, st->xp, r, CGO_T_SPMV));                    // K_b: Z = A W
+        CGO_TRY(long_rows_sum_k(ctx, LA, st->xp, r, CGO_T_SPMV));                           // … of the long rows
+        CGO_TRY(cgo_blas1_softmax(ctx, r, b, nrows, nclass, CGO_P_PHI));                   // C = P − Y, Σ loss
+        CGO_TRY(spmm_passes(ctx, AT, ATb, nclass, r, st->gp, CGO_T_SPMVT));                 // K_c: Aᵀ C
+        CGO_TRY(long_rows_sum_k(ctx, LAT, r, st->gp, CGO_T_SPMVT));                         // … and over the long rows
+        CGO_TRY(cgo_blas1_grad_combine(st, 1.0 / (double)nsamples, lambda));               // /N + λW, dots
+        return finish_lr(out);
+    }
     int finish_lr(double *out) {
         CGO_TRY(cgo_finish_pack(ctx, 12, out));
         out[CGO_P_PHI] = out[CGO_P_PHI] / (double)nsamples + (0.5 * lambda) * out[CGO_P_XPXP];
@@ -1596,11 +1795,15 @@ struct CsrObj : cgo_obj {
     int eval_trial(cgo_state *st, double a, bool fused, double beta, double *out) override {
         r_state = st; r_at_xp = true; r_at_x = false; quad_steps = 0;        // r = A xp − b (least squares) / c (logreg)
         if (!logreg) return eval_trial_ls(st, a, fused, beta, out);
+        if (nclass > 1) return eval_trial_softmax(st, a, fused, beta, out);
         return direct ? eval_trial_lr_direct(st, a, fused, beta, out) : eval_trial_lr_fused(st, a, fused, beta, out);
     }
     // SURVEY.md §8(d): A and Aᵀ streamed once (8 B value + 4 B index per entry + row pointers)
     // plus the vector passes R x,u W xp | gather xp, R b, W r | gather r, W g⁺, R u (,g)
     double bytes_per_eval() const override {
+        if (nclass > 1)         // K_a 24n | A_r + W Z | softmax R Z, y W C | Aᵀ_r + W g⁺ | R g⁺, u, g, w W g⁺  (n = d K)
+            return 12.0 * (double)(A.nnz + AT.nnz + LA.M.nnz + LAT.M.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
+                   8.0 * (3.0 * (double)nrows * (double)nclass + (double)nrows + 11.0 * (double)n_local);
         if (logreg && direct)   // K_a 24d_loc | A_r + gather + W z | logit R z, y W c | Aᵀ_f + gather + W q | R q, u, g, w W g⁺
             return 12.0 * (double)(A.nnz + AT.nnz + LA.M.nnz + LAT.M.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
                    8.0 * (5.0 * (double)nrows + (ctx->nranks > 1 ? (double)n_global + (double)nsamples : 0.0) + 11.0 * (double)n_local);
@@ -1772,8 +1975,8 @@ static int lr_layout(cgo_ctx *ctx, CsrObj *o, bool long_rows) {
     // K_b gathers over all d features, K_c over all N samples.  Column blocks are k_spmv_direct passes: the
     // forced k_csr_rows (CGO_CSR_MODE=1) runs single-pass whatever the gather range
     if (ctx->csr_mode != 1) {
-        CGO_TRY(build_blocked(ctx, o->A, o->n_global, o->Ab));
-        CGO_TRY(build_blocked(ctx, o->AT, o->nsamples, o->ATb));
+        CGO_TRY(build_blocked(ctx, o->A, o->n_global, 1, o->Ab));
+        CGO_TRY(build_blocked(ctx, o->AT, o->nsamples, 1, o->ATb));
     }
     const bool blocked = !o->Ab.blk.empty() || !o->ATb.blk.empty();
     if (blocked && o->A.nnz > (int64_t)200000000 / R) {
@@ -1922,6 +2125,66 @@ extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, con
     return 0;
 }
 
+extern "C" int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, int32_t K, const int64_t *rowptr,
+                                          const int32_t *col, const double *val, const int32_t *labels, double lambda,
+                                          cgo_obj **out) {
+    CGO_CHECK(ctx && rowptr && labels && out, "NULL argument");
+    CGO_CHECK(ctx->nranks == 1, "cgo_obj_softmax_create_csr is single-GPU");
+    CGO_CHECK(ctx->csr_mode != 1, "softmax: the objective runs on the K-column SpMM (CGO_CSR_MODE=1 forbids it)");
+    CGO_CHECK(N >= 1 && d >= 1, "softmax: need nsamples >= 1 and nfeat >= 1 (nsamples=%lld, nfeat=%lld)", (long long)N, (long long)d);
+    CGO_CHECK(K >= 2 && K <= 256, "softmax: nclasses = %d must be in [2, 256]", (int)K);
+    CGO_TRY(check_i32(N, "nsamples"));
+    CGO_TRY(check_i32(d, "nfeat"));
+    CGO_CHECK(rowptr[0] == 0, "rowptr[0] = %lld: row pointers are 0-based", (long long)rowptr[0]);
+    CGO_TRY(check_host_csr(N, d, rowptr, col, val));
+    for (int64_t i = 0; i < N; ++i)
+        CGO_CHECK(labels[i] >= 0 && labels[i] < K, "label %d of sample %lld is not in [0, %d)", (int)labels[i], (long long)i, (int)K);
+    CGO_CHECK(std::isfinite(lambda) && lambda >= 0.0, "softmax: lambda = %g must be finite and >= 0", lambda);
+    CGO_CUDA(cudaSetDevice(ctx->device));
+    const int64_t nnz = rowptr[N];
+    CsrObj *o = new CsrObj();
+    o->ctx = ctx; o->logreg = true; o->nclass = K; o->lambda = lambda; o->nsamples = N;
+    o->n_global = d * K; o->n_local = d * K; o->offset = 0; o->nrows = N; o->halo = 0;
+    o->LA.width = o->LAT.width = K;
+    auto body = [&]() -> int {
+        cudaStream_t s = ctx->stream;
+        CGO_TRY(csr_alloc(o->A, N, nnz));
+        CGO_CUDA(cudaMemcpyAsync(o->A.rowptr, rowptr, sizeof(int64_t) * (size_t)(N + 1), cudaMemcpyHostToDevice, s));
+        if (nnz) {
+            CGO_CUDA(cudaMemcpyAsync(o->A.col, col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, s));
+            CGO_CUDA(cudaMemcpyAsync(o->A.val, val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, s));
+        }
+        // labels as doubles (exact below 2^53), read in pairs by the softmax kernel
+        std::vector<double> yd((size_t)N);
+        for (int64_t i = 0; i < N; ++i) yd[(size_t)i] = (double)labels[i];
+        CGO_CUDA(cudaMalloc(&o->b, sizeof(double) * (size_t)(N + CSR_PAD)));
+        CGO_CUDA(cudaMemsetAsync(o->b, 0, sizeof(double) * (size_t)(N + CSR_PAD), s));
+        CGO_CUDA(cudaMemcpyAsync(o->b, yd.data(), sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, s));
+        CGO_TRY(o->alloc_r());
+        CsrSrc src{o->A.col, nnz};
+        CsrFin fin{o->A.rowptr, N, o->A.val};
+        CGO_TRY(build_transpose(ctx, src, fin, d, o->AT));
+        CGO_TRY(split_long_rows(ctx, o->A, o->LA));
+        CGO_TRY(split_long_rows(ctx, o->AT, o->LAT));
+        // K_b gathers d·K doubles, K_c N·K: column blocks of gather_block_bytes / 8K features / samples
+        CGO_TRY(build_blocked(ctx, o->A, d, K, o->Ab));
+        CGO_TRY(build_blocked(ctx, o->AT, N, K, o->ATb));
+        if ((!o->Ab.blk.empty() || !o->ATb.blk.empty()) && o->A.nnz > (int64_t)200000000) {
+            // production sizes: drop the single-pass copies (only the CSR download reads them)
+            if (!o->Ab.blk.empty()) { cudaFree(o->A.col); cudaFree(o->A.val); o->A.col = nullptr; o->A.val = nullptr; }
+            if (!o->ATb.blk.empty()) { cudaFree(o->AT.col); cudaFree(o->AT.val); o->AT.col = nullptr; o->AT.val = nullptr; }
+            o->have_unblocked = false;
+        }
+        CGO_CUDA(cudaStreamSynchronize(s));
+        o->direct = true;                     // dots in BLAS-1 passes: reduction site (2, 4)
+        return 0;
+    };
+    int rc = body();
+    if (rc) { delete o; return rc; }
+    *out = o;
+    return 0;
+}
+
 // ------------------------------------------------------------------ test hooks
 static CsrObj *as_csr(cgo_obj *o) { return dynamic_cast<CsrObj *>(o); }
 
@@ -2001,11 +2264,33 @@ extern "C" int cgo_obj_csr_download(cgo_obj *obj, int transposed, int64_t *rowpt
     }
     return 0;
 }
+// softmax objective: Z = A W (d·K → N·K) or Aᵀ C (N·K → d·K), through the trial's passes (column blocks included)
+static int spmm_hook(CsrObj *o, int transposed, const double *x_host, double *y_host) {
+    cgo_ctx *c = o->ctx;
+    CGO_CUDA(cudaSetDevice(c->device));
+    const int64_t K = o->nclass, nin = (transposed ? o->A.nrows : o->AT.nrows) * K, nout = (transposed ? o->AT.nrows : o->A.nrows) * K;
+    const int tclass = transposed ? CGO_T_SPMVT : CGO_T_SPMV;
+    double *dx = nullptr, *dy = nullptr;
+    auto body = [&]() -> int {
+        CGO_CUDA(cudaMalloc(&dx, sizeof(double) * (size_t)nin));
+        CGO_CUDA(cudaMalloc(&dy, sizeof(double) * (size_t)nout));
+        CGO_CUDA(cudaMemcpyAsync(dx, x_host, sizeof(double) * (size_t)nin, cudaMemcpyHostToDevice, c->stream));
+        CGO_TRY(spmm_passes(c, transposed ? o->AT : o->A, transposed ? o->ATb : o->Ab, o->nclass, dx, dy, tclass));
+        CGO_TRY(long_rows_sum_k(c, transposed ? o->LAT : o->LA, dx, dy, tclass));
+        CGO_CUDA(cudaMemcpyAsync(y_host, dy, sizeof(double) * (size_t)nout, cudaMemcpyDeviceToHost, c->stream));
+        CGO_CUDA(cudaStreamSynchronize(c->stream));
+        return 0;
+    };
+    int rc = body();
+    cudaFree(dx); cudaFree(dy);
+    return rc;
+}
 // y = A x (transposed: Aᵀ x) through the production kernel; single GPU (no halo)
 extern "C" int cgo_obj_spmv(cgo_obj *obj, int transposed, const double *x_host, double *y_host) {
     CsrObj *o = as_csr(obj);
     CGO_CHECK(o && x_host && y_host, "not a CSR objective / NULL argument");
     CGO_CHECK(o->halo == 0 && !o->lr_sharded, "cgo_obj_spmv is a single-GPU test hook");
+    if (o->nclass > 1) return spmm_hook(o, transposed, x_host, y_host);
     CGO_CHECK(o->have_unblocked, "the single-pass CSR copy was dropped at this size (column-blocked storage only)");
     cgo_ctx *c = o->ctx;
     CGO_CUDA(cudaSetDevice(c->device));

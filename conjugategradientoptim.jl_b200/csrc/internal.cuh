@@ -216,6 +216,8 @@ int cgo_blas1_sumsq(cgo_ctx *ctx, const double *a, int64_t n, int slot);        
 int cgo_blas1_dots3(cgo_ctx *ctx, const double *a, const double *b, int64_t n, int slot);       // {a·b, b·b, a·a}
 // margins → c = −y σ in place, Σ loss → pack slot; dst_all != NULL: also all-gather c over peer memory (flag CGO_F_CALL)
 int cgo_blas1_logit(cgo_ctx *ctx, double *zc, const double *y, int64_t n, int slot, void *const *dst_all, unsigned long long epoch);
+// softmax regression: Z (n × nclass, row-major) → C = P − Y in place (labels y as doubles), Σ loss → pack slot
+int cgo_blas1_softmax(cgo_ctx *ctx, double *zc, const double *y, int64_t n, int nclass, int slot);
 int cgo_blas1_grad_dots(cgo_state *st);     // the eight dots of EpiGrad over (g⁺, g, u) → pack slots CGO_P_DPHI…
 // logistic regression on k_spmv_direct: g⁺ = g⁺ · invN + λ xp in place (g⁺ holds Aᵀc), fused with the dot pack of
 // EpiGrad (slots CGO_P_DPHI .. CGO_P_UU)

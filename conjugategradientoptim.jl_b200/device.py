@@ -145,6 +145,8 @@ def shard_range(n: int, nranks: int, rank: int, align: int = 2):
 class DeviceObjective:
     """Device-resident replacement of the user callback `fdf!(g, x) -> f`."""
 
+    nclasses = 1        # columns of the vectors `spmv` multiplies (the softmax objective's K)
+
     def __init__(self, ctx: Context, handle: C.c_void_p):
         self.ctx, self.h = ctx, handle
         nl, ng, off = C.c_int64(), C.c_int64(), C.c_int64()
@@ -197,7 +199,7 @@ class DeviceObjective:
         nr, nnz = C.c_int64(), C.c_int64()
         check(lib().cgo_obj_csr_nnz(self.h, int(transposed), C.byref(nr), C.byref(nnz)))
         x = np.ascontiguousarray(x, dtype=np.float64)
-        y = np.empty(nr.value)
+        y = np.empty(nr.value * self.nclasses)
         check(lib().cgo_obj_spmv(self.h, int(transposed), dptr(x), dptr(y)))
         return y
 
@@ -320,6 +322,33 @@ def LogRegGPU_from_csr(nsamples, nfeat, rowptr, col, val, y, lam: float = 1e-6,
     check(lib().cgo_obj_logreg_create_csr(ctx.h, nsamples, nfeat, rowptr.ctypes.data, col.ctypes.data,
                                           val.ctypes.data, y.ctypes.data, lam, C.byref(h)))
     return DeviceObjective(ctx, h)
+
+
+def SoftmaxRegGPU_from_csr(nsamples, nfeat, nclasses, rowptr, col, val, labels, lam: float = 1e-6,
+                           ctx: Optional[Context] = None) -> DeviceObjective:
+    """(1/N) Σ_i [logsumexp(a_i W) − (a_i W)_{y_i}] + (λ/2)‖W‖² (multinomial logistic regression) on the caller's CSR
+    (0-based int64 row pointers, int32 columns) and labels y_i ∈ [0, nclasses), 2 <= nclasses <= 256; single GPU.
+    The state vector is W (nfeat × nclasses) feature-major, w[j·K + k], of length nfeat·nclasses: a result's
+    `minimizer.reshape(nfeat, nclasses)` is W.  An intercept is a column of ones, penalised like the other weights.
+    `spmv` takes and returns K-wide vectors: Z = A W (nfeat·K → nsamples·K) and Aᵀ C (nsamples·K → nfeat·K)."""
+    ctx = ctx or default_context()
+    rowptr = np.ascontiguousarray(rowptr, dtype=np.int64)
+    col = np.ascontiguousarray(col, dtype=np.int32)
+    val = np.ascontiguousarray(val, dtype=np.float64)
+    labels = np.asarray(labels)
+    if labels.size != nsamples or rowptr.size != nsamples + 1:
+        raise CgoError(f"rowptr needs nsamples + 1 = {nsamples + 1} entries and labels nsamples (got {rowptr.size}, {labels.size})")
+    if col.size < rowptr[-1] or val.size < rowptr[-1]:
+        raise CgoError(f"col and val need rowptr[-1] = {rowptr[-1]} entries (got {col.size}, {val.size})")
+    if not np.issubdtype(labels.dtype, np.integer) or labels.size and (labels.min() < -2**31 or labels.max() >= 2**31):
+        raise CgoError("labels must be integers")
+    labels = np.ascontiguousarray(labels, dtype=np.int32)
+    h = C.c_void_p()
+    check(lib().cgo_obj_softmax_create_csr(ctx.h, nsamples, nfeat, int(nclasses), rowptr.ctypes.data, col.ctypes.data,
+                                           val.ctypes.data, labels.ctypes.data, lam, C.byref(h)))
+    obj = DeviceObjective(ctx, h)
+    obj.nclasses = int(nclasses)
+    return obj
 
 
 class BoxBarrierGPU(DeviceObjective):

@@ -27,8 +27,9 @@
  *   by the last-arriving block in exactly the same way (lane t takes partials t, t+256, ...).
  *   Long rows (logistic regression from a host CSR, cgo_obj_logreg_create_csr, on the k_spmv_direct family): a row
  *   of A or Aᵀ with more than CGO_LONG_ROW entries is summed in this order too — its products val_k · x[col_k], k in
- *   storage order, are the items, with V=1, U=4 and the ctx's G.  Every other row of every CSR matrix is summed
- *   sequentially in storage order.
+ *   storage order, are the items, with V=1, U=4 and the ctx's G.  The softmax objective (cgo_obj_softmax_create_csr)
+ *   applies the rule to A ⊗ I_K: for each class k, the items of a long row are val_k · x[col_k·K + k].  Every other
+ *   row of every CSR matrix is summed sequentially in storage order.
  *   CSR matrices whose gathers do not coalesce (the synthetic least-squares matrix with coh_log2 < 4; a host
  *   CSR whose warp-level gathers touch more than four lines on average: cgo_obj_reduction_site tells) are
  *   multiplied by a kernel without reductions, and their dots come from BLAS-1 passes (V=2, U=4).
@@ -171,6 +172,15 @@ int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t nsamples, int64_t nfea
  * it keeps sequential row sums, exact but slow on long rows. */
 int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, const int64_t *rowptr,
                               const int32_t *col, const double *val, const double *y, double lambda, cgo_obj **out);
+/* (1/N) Σ_i [log Σ_k exp(z_ik) − z_{i,y_i}] + (λ/2)‖W‖², z_i = a_i W, from a host CSR (0-based int64 row pointers,
+ * int32 columns) and labels y_i ∈ [0, K); single GPU.  The state vector is W (nfeat × nclasses) feature-major:
+ * w[j·K + k], n = nfeat·nclasses.  2 <= K <= 256.  Z = A W is the SpMV of A ⊗ I_K on the flat W, and every row sum
+ * follows that matrix's order (long rows included).  Runs on the K-column SpMM whatever cgo_ctx_set_csr_mode says,
+ * except mode 1, which is rejected.  No Hessian-vector product or quadratic-aware line search.  The CSR test hooks
+ * return A / Aᵀ; cgo_obj_spmv takes and returns K-wide vectors (Z = A W, d·K → N·K; Aᵀ C, N·K → d·K). */
+int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, int32_t nclasses,
+                               const int64_t *rowptr, const int32_t *col, const double *val,
+                               const int32_t *labels, double lambda, cgo_obj **out);
 /* t·f0(x) − Σ log(ubs − x) − Σ log(x − lbs) around `inner` (which must outlive it): evalbarrier!
  * (src/engine/primal_barrier.jl:112-133) with the box constraints of examples/constrained.jl:17-47;
  * lbs / ubs are this rank's shard.  cgo_obj_barrier_set_t changes t between centering steps (:246);

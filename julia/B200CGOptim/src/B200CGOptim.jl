@@ -22,7 +22,7 @@ import ConjugateGradientOptim: CGConfig, Results, TraceContainer, EnableTrace, D
     minimizeobjective, minimizeobjectivererun, linesearch!, evalϕdϕ!, getβ, updatedir!,
     initializeβ, initializeLineSearchContainer!, evalwolfeconditions, evalbacktrackcondition
 
-export Context, RosenbrockGPU, RosenbrockChainedGPU, UserObjectiveGPU, SparseLSGPU, LogRegGPU, LBFGS, DeviceObjective,
+export Context, RosenbrockGPU, RosenbrockChainedGPU, UserObjectiveGPU, SparseLSGPU, LogRegGPU, SoftmaxRegGPU, LBFGS, DeviceObjective,
     DeviceStart, trial_site, set_csr_mode!, trim_pools!,
     BoxConstraint, BoxBarrierGPU, BatchedConfig, minimizeobjective_batched
 

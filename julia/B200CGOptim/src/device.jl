@@ -125,6 +125,17 @@ function LogRegGPU(nsamples::Integer, nfeat::Integer, rowptr::Vector{Int64}, col
         ctx.h, nsamples, nfeat, rowptr, col, val, y, λ, h))
     return _wrap(ctx, h[])
 end
+"Softmax (multinomial logistic) regression on the caller's CSR (0-based int64 row pointers, int32 columns) and labels in
+[0, nclasses), 2 <= nclasses <= 256; single GPU.  The state vector is W (nfeat × nclasses) feature-major, w[j·K + k]:
+`permutedims(reshape(x, nclasses, nfeat))` is W.  An intercept is a column of ones, and λ penalises its weights."
+function SoftmaxRegGPU(nsamples::Integer, nfeat::Integer, nclasses::Integer, rowptr::Vector{Int64}, col::Vector{Int32},
+                       val::Vector{Float64}, labels::Vector{Int32}, ctx::Context; λ = 1e-6)
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:cgo_obj_softmax_create_csr, LIBCGOPTIM[]), Cint,
+        (Ptr{Cvoid}, Int64, Int64, Int32, Ptr{Int64}, Ptr{Int32}, Ptr{Float64}, Ptr{Int32}, Float64, Ref{Ptr{Cvoid}}),
+        ctx.h, nsamples, nfeat, nclasses, rowptr, col, val, labels, λ, h))
+    return _wrap(ctx, h[])
+end
 
 "Token for one of the device vectors of a workspace (keeps the reference's call shapes)."
 struct DeviceVector{W}
