@@ -67,6 +67,10 @@ _SIGS = {
     "cgo_obj_logreg_create_synthetic": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int32, C.c_uint64, C.c_double, C.POINTER(_vp)]),
     "cgo_obj_logreg_create_csr": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp, C.c_double, C.POINTER(_vp)]),
     "cgo_obj_softmax_create_csr": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int32, _vp, _vp, _vp, _vp, C.c_double, C.POINTER(_vp)]),
+    "cgo_obj_logreg_create_csr_ex": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp, _vp, C.c_int32, C.c_double,
+                                               C.POINTER(_vp)]),
+    "cgo_obj_softmax_create_csr_ex": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int32, _vp, _vp, _vp, _vp, _vp, C.c_int32,
+                                                C.c_double, C.POINTER(_vp)]),
     "cgo_obj_box_barrier_create": (C.c_int, [_vp, _vp, _dp, _dp, C.c_double, C.POINTER(_vp)]),
     "cgo_obj_barrier_set_t": (C.c_int, [_vp, C.c_double]),
     "cgo_obj_barrier_infeasible": (C.c_int, [_vp, _dp, C.POINTER(C.c_int64)]),

@@ -358,6 +358,45 @@ struct GradDots {
     }
 };
 
+// The GLM objectives with an intercept (csr.cu): AxpyDir<FUSED, 0> and GradCombine for a state whose coordinates
+// [npen, n) are intercepts that λ does not penalise.  K_a reduces P instead of xp·xp, in the same positions: each
+// intercept coordinate adds +0.0 instead of its square.  The combine pass leaves λ w out of an intercept's gradient.
+template <bool FUSED>
+struct AxpyDirPen : AxpyDir<FUSED, 0> {
+    int64_t npen;
+    __device__ __forceinline__ void apply(int64_t q, const typename AxpyDir<FUSED, 0>::In &in, double (&acc)[3], bool v2) const {
+        double2 uu = in.u;
+        if (FUSED) {
+            uu.x = -in.g.x + this->beta * in.u.x;
+            uu.y = v2 ? -in.g.y + this->beta * in.u.y : 0.0;
+            cgo_st2(this->u + q, uu);
+        }
+        double2 p;
+        p.x = in.x.x + this->a * uu.x;
+        p.y = v2 ? in.x.y + this->a * uu.y : 0.0;
+        cgo_st2(this->xp + q, p);
+        acc[0] = acc[0] + in.g.x * uu.x;
+        acc[1] = acc[1] + uu.x * uu.x;
+        acc[2] = acc[2] + (2 * q < npen ? p.x * p.x : 0.0);
+        if (v2) {
+            acc[0] = acc[0] + in.g.y * uu.y;
+            acc[1] = acc[1] + uu.y * uu.y;
+            acc[2] = acc[2] + (2 * q + 1 < npen ? p.y * p.y : 0.0);
+        }
+    }
+};
+struct GradCombinePen : GradCombine {
+    int64_t npen;
+    __device__ __forceinline__ void apply(int64_t i, const In &in, double (&acc)[K], bool v2) const {
+        double2 gn;
+        gn.x = 2 * i < npen ? in.s.x * invN + lambda * in.w.x : in.s.x * invN;
+        gn.y = !v2 ? 0.0 : 2 * i + 1 < npen ? in.s.y * invN + lambda * in.w.y : in.s.y * invN;
+        cgo_st2(gp + i, gn);
+        GradDots().one(gn.x, in.g.x, in.u.x, acc);           // the eight dots, in GradCombine's order
+        if (v2) GradDots().one(gn.y, in.g.y, in.u.y, acc);
+    }
+};
+
 // logistic loss and its derivative from the margins (csr.cu EpiLogit, oracle logreg_fdf), in place: z → c = −y σ;
 // Σ ℓ.  PUSH: this rank's shard of c also goes into every rank's all-gathered copy (peer memory), then flag
 // CGO_F_CALL + me of every rank
@@ -419,6 +458,74 @@ struct SoftmaxLoss {
     __device__ __forceinline__ void apply(int64_t q, const In &in, double (&acc)[K], bool v2) const {
         one(2 * q, in.y.x, acc);
         if (v2) one(2 * q + 1, in.y.y, acc);
+    }
+};
+
+// The losses with per-sample weights s_i (wt == nullptr: unit weights) and an unpenalised intercept read from the
+// trial point (bias == nullptr: none; binary: b = bias[0], softmax: b_k = bias[k]).  The margins are the row sums plus
+// the intercept, z_i + b (z_ik + b_k); then the loss and c of LogitLoss / SoftmaxLoss, scaled by s_i: Σ s_i ℓ_i,
+// c_i = s_i · (−y_i σ_i), c_ik = s_i · (p_ik − [k = y_i]).
+struct LogitLossGlm {
+    static constexpr int TCLASS = CGO_T_OTHER;
+    static constexpr int K = 1;
+    static constexpr int OCC = 2;
+    struct In { double2 z, y, s; };
+    double2 *zc;
+    const double2 *y, *wt;
+    const double *bias;
+    double b;
+    __device__ __forceinline__ void prologue() { b = bias ? *bias : 0.0; }
+    __device__ __forceinline__ In load(int64_t q) const {
+        return In{ld2rw(zc + q), cgo_ld2(y + q), wt ? cgo_ld2(wt + q) : make_double2(1.0, 1.0)};
+    }
+    __device__ __forceinline__ double one(double z, double yy, double sw, double (&acc)[K]) const {
+        const double m = bias ? z + b : z;
+        const double t = -yy * m;
+        const double e = exp(-fabs(t));
+        const double l = (t > 0.0 ? t : 0.0) + log1p(e);
+        const double sg = t >= 0.0 ? 1.0 / (1.0 + e) : e / (1.0 + e);
+        acc[0] = acc[0] + sw * l;
+        return sw * (-yy * sg);
+    }
+    __device__ __forceinline__ void apply(int64_t q, const In &in, double (&acc)[K], bool v2) const {
+        double2 c;
+        c.x = one(in.z.x, in.y.x, in.s.x, acc);
+        c.y = v2 ? one(in.z.y, in.y.y, in.s.y, acc) : 0.0;
+        cgo_st2(zc + q, c);
+    }
+};
+struct SoftmaxLossGlm {
+    static constexpr int TCLASS = CGO_T_OTHER;
+    static constexpr int K = 1;
+    static constexpr int OCC = 2;
+    struct In { double2 y, s; };
+    double *zc;
+    const double2 *y, *wt;
+    const double *bias;
+    int nc;
+    __device__ __forceinline__ void prologue() {}
+    __device__ __forceinline__ In load(int64_t q) const {
+        return In{cgo_ld2(y + q), wt ? cgo_ld2(wt + q) : make_double2(1.0, 1.0)};
+    }
+    // z_ik + b_k is formed where it is read (the same bits every time): storing it first would cost the sample's
+    // L1-resident logits on every later pass
+    __device__ __forceinline__ double zb(const double *z, int k) const { return bias ? z[k] + bias[k] : z[k]; }
+    __device__ __forceinline__ void one(int64_t i, double yy, double sw, double (&acc)[K]) const {
+        double *z = zc + i * nc;
+        const int lab = (int)yy;
+        double m = zb(z, 0);
+        for (int k = 1; k < nc; ++k) { const double v = zb(z, k); m = v > m ? v : m; }
+        double s = 0.0;
+        for (int k = 0; k < nc; ++k) s = s + exp(zb(z, k) - m);
+        acc[0] = acc[0] + sw * ((m + log(s)) - zb(z, lab));
+        for (int k = 0; k < nc; ++k) {
+            const double p = exp(zb(z, k) - m) / s;
+            z[k] = sw * (k == lab ? p - 1.0 : p);
+        }
+    }
+    __device__ __forceinline__ void apply(int64_t q, const In &in, double (&acc)[K], bool v2) const {
+        one(2 * q, in.y.x, in.s.x, acc);
+        if (v2) one(2 * q + 1, in.y.y, in.s.y, acc);
     }
 };
 
@@ -1178,6 +1285,19 @@ int cgo_blas1_axpy_dir(cgo_state *st, double a, bool fused, double beta, const H
     if (push) return fused ? launch_axpy_dir<true, 1>(st, a, beta, push) : launch_axpy_dir<false, 1>(st, a, beta, push);
     return fused ? launch_axpy_dir<true, 0>(st, a, beta, nullptr) : launch_axpy_dir<false, 0>(st, a, beta, nullptr);
 }
+template <bool FUSED>
+static int launch_axpy_dir_pen(cgo_state *st, double a, double beta, int64_t npen) {
+    AxpyDirPen<FUSED> op;
+    op.x = (const double2 *)st->x; op.g = (const double2 *)st->g; op.u = (double2 *)st->u;
+    op.xp = (double2 *)st->xp; op.a = a; op.beta = FUSED ? beta : 0.0;
+    op.prev_right = op.next_left = nullptr; op.hq = 0; op.nq = st->n / 2;
+    op.dst_all = nullptr; op.nranks = 1;
+    op.npen = npen;
+    return launch_blas1(st->ctx, op, st->n, cgo_red_args(st->ctx, CGO_P_DIR_GU));
+}
+int cgo_blas1_axpy_dir_pen(cgo_state *st, double a, bool fused, double beta, int64_t npen) {
+    return fused ? launch_axpy_dir_pen<true>(st, a, beta, npen) : launch_axpy_dir_pen<false>(st, a, beta, npen);
+}
 
 int cgo_blas1_sumsq(cgo_ctx *c, const double *a, int64_t n, int slot) {
     VecSumSq op;
@@ -1207,6 +1327,17 @@ int cgo_blas1_softmax(cgo_ctx *c, double *zc, const double *y, int64_t n, int nc
     op.zc = zc; op.y = (const double2 *)y; op.nc = nclass;
     return launch_blas1(c, op, n, cgo_red_args(c, slot));
 }
+int cgo_blas1_logit_glm(cgo_ctx *c, double *zc, const double *y, const double *wt, const double *bias, int64_t n, int slot) {
+    LogitLossGlm op;
+    op.zc = (double2 *)zc; op.y = (const double2 *)y; op.wt = (const double2 *)wt; op.bias = bias; op.b = 0.0;
+    return launch_blas1(c, op, n, cgo_red_args(c, slot));
+}
+int cgo_blas1_softmax_glm(cgo_ctx *c, double *zc, const double *y, const double *wt, const double *bias, int64_t n,
+                          int nclass, int slot) {
+    SoftmaxLossGlm op;
+    op.zc = zc; op.y = (const double2 *)y; op.wt = (const double2 *)wt; op.bias = bias; op.nc = nclass;
+    return launch_blas1(c, op, n, cgo_red_args(c, slot));
+}
 int cgo_blas1_grad_dots(cgo_state *st) {
     GradDots op;
     op.gp = (const double2 *)st->gp; op.g = (const double2 *)st->g; op.u = (const double2 *)st->u;
@@ -1218,6 +1349,13 @@ int cgo_blas1_grad_combine(cgo_state *st, double invN, double lambda) {
     op.u = (const double2 *)st->u; op.g = (const double2 *)st->g;
     op.w = (const double2 *)st->xp; op.gp = (double2 *)st->gp;
     op.invN = invN; op.lambda = lambda;
+    return launch_blas1(st->ctx, op, st->n, cgo_red_args(st->ctx, CGO_P_DPHI));
+}
+int cgo_blas1_grad_combine_pen(cgo_state *st, double invS, double lambda, int64_t npen) {
+    GradCombinePen op;
+    op.u = (const double2 *)st->u; op.g = (const double2 *)st->g;
+    op.w = (const double2 *)st->xp; op.gp = (double2 *)st->gp;
+    op.invN = invS; op.lambda = lambda; op.npen = npen;
     return launch_blas1(st->ctx, op, st->n, cgo_red_args(st->ctx, CGO_P_DPHI));
 }
 

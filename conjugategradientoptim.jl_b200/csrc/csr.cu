@@ -20,6 +20,7 @@
 // order.  Rows and tiles of any length work.
 #include <cub/device/device_scan.cuh>
 #include <cmath>
+#include <utility>
 
 #include "internal.cuh"
 #include "reduce.cuh"
@@ -1262,6 +1263,8 @@ struct LongRows {
     std::vector<int64_t> h_row, h_rowptr;    // host copies of `row` and M.rowptr
     int G = 0;                               // the G the work units are laid out for
     int width = 1;                           // sums per long row (K for the K-column SpMM)
+    // an intercept's unit row (add_unit_row): the last of the n rows, not stored in M, with ulen entries 1.0
+    int64_t ulen = 0;
     int64_t nunits = 0;
     int2 *unit = nullptr;                    // (long row, virtual CTA) of every unit
     int64_t *ubase = nullptr;                // first unit of every long row, n + 1
@@ -1273,14 +1276,18 @@ struct LongRows {
     }
 };
 
-__global__ void __launch_bounds__(CGO_B) k_long_rows(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G,
-                                                     const double *__restrict__ xg, double *__restrict__ partial) {
+// UNIT: the last long row may be the unit row of an intercept (row index >= L.nrows): a virtual row of Aᵀ whose
+// entries are 1.0 at columns 0 … ulen − 1, synthesised instead of stored
+template <bool UNIT>
+__device__ __forceinline__ void long_rows_body(const CsrMat &L, const int2 *__restrict__ unit, int64_t nunits, int G,
+                                               int64_t ulen, const double *__restrict__ xg, double *__restrict__ partial) {
     __shared__ double s_red[CGO_NW];
     const int t = threadIdx.x;
     const uint64_t gpol = l2_policy_evict_last();
     for (int64_t u = blockIdx.x; u < nunits; u += gridDim.x) {
         const int2 w = unit[u];
-        const int64_t p0 = L.rowptr[w.x], len = L.rowptr[w.x + 1] - p0;
+        const bool urow = UNIT && w.x >= L.nrows;
+        const int64_t p0 = urow ? 0 : L.rowptr[w.x], len = urow ? ulen : L.rowptr[w.x + 1] - p0;
         const int64_t ntiles = (len + LONG_TILE - 1) / LONG_TILE;
         double acc[1] = {0.0};
 #pragma unroll 1
@@ -1294,8 +1301,13 @@ __global__ void __launch_bounds__(CGO_B) k_long_rows(CsrMat L, const int2 *__res
             for (int j = 0; j < NI; ++j) {
                 const int64_t k = (tile + (int64_t)(j / LONG_U) * G) * LONG_TILE + (j % LONG_U) * CGO_B + t;
                 on[j] = k < len;
-                cj[j] = ld_stream_s32_if(L.col + p0 + k, on[j]);
-                vj[j] = ld_stream_f64_if(L.val + p0 + k, on[j]);
+                if (urow) {
+                    cj[j] = (int32_t)k;
+                    vj[j] = 1.0;
+                } else {
+                    cj[j] = ld_stream_s32_if(L.col + p0 + k, on[j]);
+                    vj[j] = ld_stream_f64_if(L.val + p0 + k, on[j]);
+                }
             }
 #pragma unroll
             for (int j = 0; j < NI; ++j) xj[j] = ld_gather_f64_if(xg + cj[j], gpol, on[j]);
@@ -1308,6 +1320,15 @@ __global__ void __launch_bounds__(CGO_B) k_long_rows(CsrMat L, const int2 *__res
         cgo_cta_combine<1>(acc, s_red);
         if (t == 0) partial[u] = acc[0];
     }
+}
+__global__ void __launch_bounds__(CGO_B) k_long_rows(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G,
+                                                     const double *__restrict__ xg, double *__restrict__ partial) {
+    long_rows_body<false>(L, unit, nunits, G, 0, xg, partial);
+}
+__global__ void __launch_bounds__(CGO_B) k_long_rows_unit(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G,
+                                                          int64_t ulen, const double *__restrict__ xg,
+                                                          double *__restrict__ partial) {
+    long_rows_body<true>(L, unit, nunits, G, ulen, xg, partial);
 }
 // one CTA per long row: lane t adds the row's partials t, t + 256, …, then the CTA combine
 __global__ void __launch_bounds__(CGO_B) k_long_finish(const int64_t *__restrict__ ubase, const int64_t *__restrict__ row,
@@ -1349,7 +1370,8 @@ static int long_rows_sum(cgo_ctx *c, LongRows &L, const double *xg, double *out,
     const int64_t phys = (int64_t)c->sms * 8;
     const int grid = (int)(L.nunits < phys ? L.nunits : phys);
     cgo_timer_begin(c, tclass);
-    k_long_rows<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, xg, L.partial);
+    if (L.ulen > 0) k_long_rows_unit<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, L.ulen, xg, L.partial);
+    else k_long_rows<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, xg, L.partial);
     cgo_timer_end(c);
     c->launches++;
     CGO_CUDA(cudaGetLastError());
@@ -1367,8 +1389,10 @@ static int long_rows_sum(cgo_ctx *c, LongRows &L, const double *xg, double *out,
 // per class tile and keeps LONG_KT accumulators, and the CTA combine reduces each of them as it reduces one.
 // Partials are stored unit-major, K per unit; k_long_finish_k runs one CTA per (long row, class).
 constexpr int LONG_KT = 8;
-__global__ void __launch_bounds__(CGO_B) k_long_rows_k(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G, int K,
-                                                       const double *__restrict__ xg, double *__restrict__ partial) {
+template <bool UNIT>
+__device__ __forceinline__ void long_rows_k_body(const CsrMat &L, const int2 *__restrict__ unit, int64_t nunits, int G,
+                                                 int K, int64_t ulen, const double *__restrict__ xg,
+                                                 double *__restrict__ partial) {
     __shared__ double s_red[LONG_KT * CGO_NW];
     const int t = threadIdx.x;
     const uint64_t gpol = l2_policy_evict_last();
@@ -1377,7 +1401,8 @@ __global__ void __launch_bounds__(CGO_B) k_long_rows_k(CsrMat L, const int2 *__r
         const int64_t u = wi / nct;
         const int k0 = (int)(wi - u * nct) * LONG_KT;
         const int2 w = unit[u];
-        const int64_t p0 = L.rowptr[w.x], len = L.rowptr[w.x + 1] - p0;
+        const bool urow = UNIT && w.x >= L.nrows;
+        const int64_t p0 = urow ? 0 : L.rowptr[w.x], len = urow ? ulen : L.rowptr[w.x + 1] - p0;
         const int64_t ntiles = (len + LONG_TILE - 1) / LONG_TILE;
         double acc[LONG_KT];
 #pragma unroll
@@ -1391,8 +1416,13 @@ __global__ void __launch_bounds__(CGO_B) k_long_rows_k(CsrMat L, const int2 *__r
             for (int j = 0; j < LONG_U; ++j) {
                 const int64_t k = tile * LONG_TILE + j * CGO_B + t;
                 on[j] = k < len;
-                cj[j] = ld_stream_s32_if(L.col + p0 + k, on[j]);
-                vj[j] = ld_stream_f64_if(L.val + p0 + k, on[j]);
+                if (urow) {
+                    cj[j] = (int32_t)k;
+                    vj[j] = 1.0;
+                } else {
+                    cj[j] = ld_stream_s32_if(L.col + p0 + k, on[j]);
+                    vj[j] = ld_stream_f64_if(L.val + p0 + k, on[j]);
+                }
             }
             double xj[LONG_U][LONG_KT];
 #pragma unroll
@@ -1416,6 +1446,15 @@ __global__ void __launch_bounds__(CGO_B) k_long_rows_k(CsrMat L, const int2 *__r
         }
     }
 }
+__global__ void __launch_bounds__(CGO_B) k_long_rows_k(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G, int K,
+                                                       const double *__restrict__ xg, double *__restrict__ partial) {
+    long_rows_k_body<false>(L, unit, nunits, G, K, 0, xg, partial);
+}
+__global__ void __launch_bounds__(CGO_B) k_long_rows_k_unit(CsrMat L, const int2 *__restrict__ unit, int64_t nunits, int G,
+                                                            int K, int64_t ulen, const double *__restrict__ xg,
+                                                            double *__restrict__ partial) {
+    long_rows_k_body<true>(L, unit, nunits, G, K, ulen, xg, partial);
+}
 __global__ void __launch_bounds__(CGO_B) k_long_finish_k(const int64_t *__restrict__ ubase, const int64_t *__restrict__ row, int K,
                                                          const double *__restrict__ partial, double *out) {
     __shared__ double s_red[CGO_NW];
@@ -1433,7 +1472,8 @@ static int long_rows_sum_k(cgo_ctx *c, LongRows &L, const double *xg, double *ou
     const int64_t items = L.nunits * ((K + LONG_KT - 1) / LONG_KT), phys = (int64_t)c->sms * 8;
     const int grid = (int)(items < phys ? items : phys);
     cgo_timer_begin(c, tclass);
-    k_long_rows_k<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, K, xg, L.partial);
+    if (L.ulen > 0) k_long_rows_k_unit<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, K, L.ulen, xg, L.partial);
+    else k_long_rows_k<<<grid, CGO_B, 0, c->stream>>>(L.M, L.unit, L.nunits, L.G, K, xg, L.partial);
     cgo_timer_end(c);
     c->launches++;
     CGO_CUDA(cudaGetLastError());
@@ -1508,6 +1548,21 @@ static int split_long_rows(cgo_ctx *c, CsrMat &A, LongRows &L) {
     A = S;
     return 0;
 }
+// an intercept: its gradient is the sum of a row of Aᵀ that is not stored, 1.0 at every sample.  It joins L as one
+// more long row, stored at index `row` of the output, so the intercept adds work units, not launches
+static int add_unit_row(cgo_ctx *c, LongRows &L, int64_t row, int64_t len) {
+    L.h_row.push_back(row);
+    L.h_rowptr.push_back(L.h_rowptr.back() + len);
+    L.n = (int64_t)L.h_row.size();
+    L.ulen = len;
+    cudaFree(L.row); cudaFree(L.ubase);
+    L.row = nullptr; L.ubase = nullptr;
+    CGO_CUDA(cudaMalloc(&L.row, sizeof(int64_t) * (size_t)L.n));
+    CGO_CUDA(cudaMalloc(&L.ubase, sizeof(int64_t) * (size_t)(L.n + 1)));
+    CGO_CUDA(cudaMemcpyAsync(L.row, L.h_row.data(), sizeof(int64_t) * (size_t)L.n, cudaMemcpyHostToDevice, c->stream));
+    CGO_CUDA(cudaStreamSynchronize(c->stream));
+    return 0;
+}
 
 // ------------------------------------------------------------------ the objective
 struct CsrObj : cgo_obj {
@@ -1537,6 +1592,14 @@ struct CsrObj : cgo_obj {
     bool r_is_peer = false;
     double lambda = 0.0;
     int64_t nsamples = 0;
+    // logistic and softmax regression: S, the sum of the sample weights (nsamples without weights); the weights
+    // (nullptr: unit weights, nsamples + CSR_PAD); fit_intercept: the last nclass coordinates of the state are the
+    // intercept, which λ does not penalise (k_spmv_direct / the SpMM only)
+    double wsum = 0.0;
+    double *wt = nullptr;
+    bool icpt = false;
+    bool glm() const { return wt != nullptr || icpt; }
+    int64_t npen() const { return icpt ? n_local - nclass : n_local; }
     // sharded logistic regression (nranks > 1): samples AND features are sharded.  A holds this rank's samples ×
     // all features and gathers the all-gathered trial point; AT holds this rank's FEATURES × all samples (built
     // straight from the generator) and gathers the all-gathered c, so every row of Aᵀc is added over all samples in
@@ -1561,7 +1624,7 @@ struct CsrObj : cgo_obj {
             cgo_peer_free(ctx, c_full, cf_peers, true); c_full = nullptr;
         }
         cudaFree(d_xpf_dst); cudaFree(d_cf_dst);
-        cudaFree(b); cudaFree(r_base); cudaFree(qv);
+        cudaFree(b); cudaFree(wt); cudaFree(r_base); cudaFree(qv);
         cudaFree(xp_full); cudaFree(c_full);
     }
     int alloc_r() {
@@ -1746,18 +1809,19 @@ struct CsrObj : cgo_obj {
             wx.wait_all = ctx->flags_local + CGO_F_XPALL; wx.wait_val = e; wx.nranks = R; pwx = &wx;
             wc.wait_all = ctx->flags_local + CGO_F_CALL; wc.wait_val = e; wc.nranks = R; pwc = &wc;
         } else {
-            CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                          // K_a
+            CGO_TRY(trial_axpy(st, a, fused, beta));                                   // K_a
             if (R > 1) CGO_TRY(cgo_allgatherv_f64(ctx, st->xp, xp_full, flo.data()));
         }
         const double *w_all = R > 1 ? xp_full : st->xp;
         CGO_TRY(spmv_direct_passes(ctx, A, Ab, w_all, r, pwx, CGO_T_SPMV));            // K_b: margins of my samples
         CGO_TRY(long_rows_sum(ctx, LA, w_all, r, CGO_T_SPMV));                           // … of the long rows
-        CGO_TRY(cgo_blas1_logit(ctx, r, b, nrows, CGO_P_PHI, (R > 1 && lr_peer) ? d_cf_dst : nullptr, e));   // c, Σ loss [+ all-gather of c]
+        if (glm()) CGO_TRY(cgo_blas1_logit_glm(ctx, r, b, wt, icpt ? st->xp + npen() : nullptr, nrows, CGO_P_PHI));   // c, Σ s ℓ
+        else CGO_TRY(cgo_blas1_logit(ctx, r, b, nrows, CGO_P_PHI, (R > 1 && lr_peer) ? d_cf_dst : nullptr, e));   // c, Σ loss [+ all-gather of c]
         if (R > 1 && !lr_peer) CGO_TRY(cgo_allgatherv_f64(ctx, r, c_full, slo.data()));
         const double *c_all = R > 1 ? c_full : r;
         CGO_TRY(spmv_direct_passes(ctx, AT, ATb, c_all, st->gp, pwc, CGO_T_SPMVT));    // K_c: Aᵀc over my features
-        CGO_TRY(long_rows_sum(ctx, LAT, c_all, st->gp, CGO_T_SPMVT));                    // … and over the long rows
-        CGO_TRY(cgo_blas1_grad_combine(st, 1.0 / (double)nsamples, lambda));           // /N + λw, dots
+        CGO_TRY(long_rows_sum(ctx, LAT, c_all, st->gp, CGO_T_SPMVT));                    // … and over the long rows [and Σ c]
+        CGO_TRY(grad_combine(st));                                                      // /S + λw, dots
         return finish_lr(out);
     }
     // the fused k_csr_rows, one pass of each matrix (single rank)
@@ -1772,18 +1836,26 @@ struct CsrObj : cgo_obj {
     // softmax regression, single rank: K_a | SpMM passes of A → Z | softmax + loss (BLAS-1) | SpMM passes of Aᵀ |
     // /N + λW + dots (BLAS-1)
     int eval_trial_softmax(cgo_state *st, double a, bool fused, double beta, double *out) {
-        CGO_TRY(cgo_blas1_axpy_dir(st, a, fused, beta));                                   // K_a
+        CGO_TRY(trial_axpy(st, a, fused, beta));                                           // K_a
         CGO_TRY(spmm_passes(ctx, A, Ab, nclass, st->xp, r, CGO_T_SPMV));                    // K_b: Z = A W
         CGO_TRY(long_rows_sum_k(ctx, LA, st->xp, r, CGO_T_SPMV));                           // … of the long rows
-        CGO_TRY(cgo_blas1_softmax(ctx, r, b, nrows, nclass, CGO_P_PHI));                   // C = P − Y, Σ loss
+        if (glm()) CGO_TRY(cgo_blas1_softmax_glm(ctx, r, b, wt, icpt ? st->xp + npen() : nullptr, nrows, nclass, CGO_P_PHI));
+        else CGO_TRY(cgo_blas1_softmax(ctx, r, b, nrows, nclass, CGO_P_PHI));              // C = P − Y, Σ loss
         CGO_TRY(spmm_passes(ctx, AT, ATb, nclass, r, st->gp, CGO_T_SPMVT));                 // K_c: Aᵀ C
-        CGO_TRY(long_rows_sum_k(ctx, LAT, r, st->gp, CGO_T_SPMVT));                         // … and over the long rows
-        CGO_TRY(cgo_blas1_grad_combine(st, 1.0 / (double)nsamples, lambda));               // /N + λW, dots
+        CGO_TRY(long_rows_sum_k(ctx, LAT, r, st->gp, CGO_T_SPMVT));                         // … and over the long rows [and Σ C]
+        CGO_TRY(grad_combine(st));                                                          // /S + λW, dots
         return finish_lr(out);
+    }
+    // K_a; with an intercept P, the penalised part of xp·xp, replaces xp·xp in slot CGO_P_XPXP
+    int trial_axpy(cgo_state *st, double a, bool fused, double beta) {
+        return icpt ? cgo_blas1_axpy_dir_pen(st, a, fused, beta, npen()) : cgo_blas1_axpy_dir(st, a, fused, beta);
+    }
+    int grad_combine(cgo_state *st) {
+        return icpt ? cgo_blas1_grad_combine_pen(st, 1.0 / wsum, lambda, npen()) : cgo_blas1_grad_combine(st, 1.0 / wsum, lambda);
     }
     int finish_lr(double *out) {
         CGO_TRY(cgo_finish_pack(ctx, 12, out));
-        out[CGO_P_PHI] = out[CGO_P_PHI] / (double)nsamples + (0.5 * lambda) * out[CGO_P_XPXP];
+        out[CGO_P_PHI] = out[CGO_P_PHI] / wsum + (0.5 * lambda) * out[CGO_P_XPXP];
         return 0;
     }
 
@@ -1801,12 +1873,15 @@ struct CsrObj : cgo_obj {
     // SURVEY.md §8(d): A and Aᵀ streamed once (8 B value + 4 B index per entry + row pointers)
     // plus the vector passes R x,u W xp | gather xp, R b, W r | gather r, W g⁺, R u (,g)
     double bytes_per_eval() const override {
+        // weights: the loss op reads s (8N); intercept: its unit row reads c (8N, 8NK), and no matrix bytes
+        const double glm_bytes = 8.0 * ((wt ? (double)nrows : 0.0) + (icpt ? (double)nrows * (double)nclass : 0.0));
         if (nclass > 1)         // K_a 24n | A_r + W Z | softmax R Z, y W C | Aᵀ_r + W g⁺ | R g⁺, u, g, w W g⁺  (n = d K)
             return 12.0 * (double)(A.nnz + AT.nnz + LA.M.nnz + LAT.M.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
-                   8.0 * (3.0 * (double)nrows * (double)nclass + (double)nrows + 11.0 * (double)n_local);
+                   8.0 * (3.0 * (double)nrows * (double)nclass + (double)nrows + 11.0 * (double)n_local) + glm_bytes;
         if (logreg && direct)   // K_a 24d_loc | A_r + gather + W z | logit R z, y W c | Aᵀ_f + gather + W q | R q, u, g, w W g⁺
             return 12.0 * (double)(A.nnz + AT.nnz + LA.M.nnz + LAT.M.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
-                   8.0 * (5.0 * (double)nrows + (ctx->nranks > 1 ? (double)n_global + (double)nsamples : 0.0) + 11.0 * (double)n_local);
+                   8.0 * (5.0 * (double)nrows + (ctx->nranks > 1 ? (double)n_global + (double)nsamples : 0.0) + 11.0 * (double)n_local) +
+                   glm_bytes;
         // (k_spmv_direct: the dots are separate BLAS-1 passes, R r | R g⁺, g, u instead of the staged u, g)
         return 12.0 * (double)(A.nnz + AT.nnz) + 8.0 * (double)(A.nrows + 1 + AT.nrows + 1) +
                8.0 * (3.0 * (double)nrows + 6.0 * (double)n_local) + (direct ? 8.0 * ((double)nrows + (double)n_local) : 0.0);
@@ -1969,13 +2044,14 @@ struct LrFeatFin {                  // key = global entry index of the generator
 };
 
 // column blocks, kernel family and layout of a logistic regression's A (samples × all features) and Aᵀ (both
-// constructors).  `long_rows`: rows were taken out of A or Aᵀ (split_long_rows), which only k_spmv_direct adds back.
+// constructors).  `long_rows`: rows were taken out of A or Aᵀ (split_long_rows), which only k_spmv_direct adds back;
+// also set for weights or an intercept, which only the k_spmv_direct trial applies.
 static int lr_layout(cgo_ctx *ctx, CsrObj *o, bool long_rows) {
     const int R = ctx->nranks;
     // K_b gathers over all d features, K_c over all N samples.  Column blocks are k_spmv_direct passes: the
     // forced k_csr_rows (CGO_CSR_MODE=1) runs single-pass whatever the gather range
     if (ctx->csr_mode != 1) {
-        CGO_TRY(build_blocked(ctx, o->A, o->n_global, 1, o->Ab));
+        CGO_TRY(build_blocked(ctx, o->A, o->n_global - (o->icpt ? 1 : 0), 1, o->Ab));
         CGO_TRY(build_blocked(ctx, o->AT, o->nsamples, 1, o->ATb));
     }
     const bool blocked = !o->Ab.blk.empty() || !o->ATb.blk.empty();
@@ -2009,7 +2085,7 @@ extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t 
     CGO_CHECK(R == 1 || ctx->csr_mode != 1, "logreg: the sharded objective runs on k_spmv_direct (CGO_CSR_MODE=1 forbids it)");
     CGO_CUDA(cudaSetDevice(ctx->device));
     CsrObj *o = new CsrObj();
-    o->ctx = ctx; o->logreg = true; o->lambda = lambda; o->nsamples = N;
+    o->ctx = ctx; o->logreg = true; o->lambda = lambda; o->nsamples = N; o->wsum = (double)N;
     o->n_global = d; o->halo = 0;
     LrSpec sp;
     sp.N = N; sp.d = d; sp.K = K; sp.w = d / K; sp.seed = seed;
@@ -2082,8 +2158,65 @@ extern "C" int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t N, int64_t 
     return 0;
 }
 
-extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, const int64_t *rowptr, const int32_t *col,
-                                         const double *val, const double *y, double lambda, cgo_obj **out) {
+// the correctly rounded sum of x[0 … n) (Shewchuk's exact partials, rounded as Python's math.fsum rounds them)
+static double exact_sum(const double *x, int64_t n) {
+    std::vector<double> part;
+    for (int64_t k = 0; k < n; ++k) {
+        double v = x[k];
+        size_t i = 0;
+        for (double y : part) {
+            if (std::fabs(v) < std::fabs(y)) std::swap(v, y);
+            const double hi = v + y, lo = y - (hi - v);
+            if (lo != 0.0) part[i++] = lo;
+            v = hi;
+        }
+        part.resize(i);
+        part.push_back(v);
+    }
+    size_t m = part.size();
+    if (m == 0) return 0.0;
+    double hi = part[--m], lo = 0.0;
+    while (m > 0) {
+        const double v = hi, y = part[--m];
+        hi = v + y;
+        lo = y - (hi - v);
+        if (lo != 0.0) break;
+    }
+    if (m > 0 && ((lo < 0.0 && part[m - 1] < 0.0) || (lo > 0.0 && part[m - 1] > 0.0))) {
+        const double y = lo * 2.0, v = hi + y;
+        if (y == v - hi) hi = v;
+    }
+    return hi;
+}
+
+// weights and intercept of the logistic and softmax objectives: argument errors name the offending sample or value.
+// S = Σ s_i, correctly rounded (N without weights)
+static int check_glm(cgo_ctx *ctx, const char *who, int64_t N, int64_t d, const double *w, int32_t fit_intercept, double *S) {
+    CGO_CHECK(fit_intercept == 0 || fit_intercept == 1, "%s: fit_intercept = %d must be 0 or 1", who, (int)fit_intercept);
+    *S = (double)N;
+    if (!w && !fit_intercept) return 0;
+    CGO_CHECK(ctx->csr_mode != 1, "%s: weights and the intercept run on k_spmv_direct (CGO_CSR_MODE=1 forbids them)", who);
+    if (fit_intercept) CGO_TRY(check_i32(d + 1, "nfeat + 1 (the intercept's feature)"));
+    if (!w) return 0;
+    for (int64_t i = 0; i < N; ++i)
+        CGO_CHECK(std::isfinite(w[i]) && w[i] >= 0.0, "%s: sample_weight %g of sample %lld must be finite and >= 0", who, w[i],
+                  (long long)i);
+    *S = exact_sum(w, N);
+    CGO_CHECK(std::isfinite(*S) && *S > 0.0, "%s: the sample weights add up to %g; their sum must be finite and > 0", who, *S);
+    return 0;
+}
+// weights on the device, padded for the double2 loads of the loss ops
+static int upload_weights(cgo_ctx *ctx, CsrObj *o, const double *w, int64_t N) {
+    if (!w) return 0;
+    CGO_CUDA(cudaMalloc(&o->wt, sizeof(double) * (size_t)(N + CSR_PAD)));
+    CGO_CUDA(cudaMemsetAsync(o->wt, 0, sizeof(double) * (size_t)(N + CSR_PAD), ctx->stream));
+    CGO_CUDA(cudaMemcpyAsync(o->wt, w, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+}
+
+extern "C" int cgo_obj_logreg_create_csr_ex(cgo_ctx *ctx, int64_t N, int64_t d, const int64_t *rowptr, const int32_t *col,
+                                            const double *val, const double *y, const double *sample_weight,
+                                            int32_t fit_intercept, double lambda, cgo_obj **out) {
     CGO_CHECK(ctx && rowptr && y && out, "NULL argument");
     CGO_CHECK(ctx->nranks == 1, "cgo_obj_logreg_create_csr is single-GPU");
     CGO_CHECK(N >= 1 && d >= 1, "logreg: need nsamples >= 1 and nfeat >= 1 (nsamples=%lld, nfeat=%lld)", (long long)N, (long long)d);
@@ -2093,11 +2226,13 @@ extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, con
     CGO_TRY(check_host_csr(N, d, rowptr, col, val));
     for (int64_t i = 0; i < N; ++i) CGO_CHECK(y[i] == 1.0 || y[i] == -1.0, "label %g of sample %lld is not +1 or -1", y[i], (long long)i);
     CGO_CHECK(std::isfinite(lambda) && lambda >= 0.0, "logreg: lambda = %g must be finite and >= 0", lambda);
+    double S;
+    CGO_TRY(check_glm(ctx, "logreg", N, d, sample_weight, fit_intercept, &S));
     CGO_CUDA(cudaSetDevice(ctx->device));
-    const int64_t nnz = rowptr[N];
+    const int64_t nnz = rowptr[N], n = d + fit_intercept;
     CsrObj *o = new CsrObj();
-    o->ctx = ctx; o->logreg = true; o->lambda = lambda; o->nsamples = N;
-    o->n_global = d; o->n_local = d; o->offset = 0; o->nrows = N; o->halo = 0;
+    o->ctx = ctx; o->logreg = true; o->lambda = lambda; o->nsamples = N; o->wsum = S; o->icpt = fit_intercept == 1;
+    o->n_global = n; o->n_local = n; o->offset = 0; o->nrows = N; o->halo = 0;
     auto body = [&]() -> int {
         cudaStream_t s = ctx->stream;
         CGO_TRY(csr_alloc(o->A, N, nnz));
@@ -2109,6 +2244,7 @@ extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, con
         CGO_CUDA(cudaMalloc(&o->b, sizeof(double) * (size_t)(N + CSR_PAD)));
         CGO_CUDA(cudaMemsetAsync(o->b, 0, sizeof(double) * (size_t)(N + CSR_PAD), s));
         CGO_CUDA(cudaMemcpyAsync(o->b, y, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, s));
+        CGO_TRY(upload_weights(ctx, o, sample_weight, N));
         CGO_TRY(o->alloc_r());
         CsrSrc src{o->A.col, nnz};
         CsrFin fin{o->A.rowptr, N, o->A.val};
@@ -2117,17 +2253,23 @@ extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, con
             CGO_TRY(split_long_rows(ctx, o->A, o->LA));
             CGO_TRY(split_long_rows(ctx, o->AT, o->LAT));
         }
-        return lr_layout(ctx, o, o->LA.n > 0 || o->LAT.n > 0);
+        if (o->icpt) CGO_TRY(add_unit_row(ctx, o->LAT, d, N));
+        return lr_layout(ctx, o, o->LA.n > 0 || o->LAT.n > 0 || o->glm());
     };
     int rc = body();
     if (rc) { delete o; return rc; }
     *out = o;
     return 0;
 }
+extern "C" int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, const int64_t *rowptr, const int32_t *col,
+                                         const double *val, const double *y, double lambda, cgo_obj **out) {
+    return cgo_obj_logreg_create_csr_ex(ctx, N, d, rowptr, col, val, y, nullptr, 0, lambda, out);
+}
 
-extern "C" int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, int32_t K, const int64_t *rowptr,
-                                          const int32_t *col, const double *val, const int32_t *labels, double lambda,
-                                          cgo_obj **out) {
+extern "C" int cgo_obj_softmax_create_csr_ex(cgo_ctx *ctx, int64_t N, int64_t d, int32_t K, const int64_t *rowptr,
+                                             const int32_t *col, const double *val, const int32_t *labels,
+                                             const double *sample_weight, int32_t fit_intercept, double lambda,
+                                             cgo_obj **out) {
     CGO_CHECK(ctx && rowptr && labels && out, "NULL argument");
     CGO_CHECK(ctx->nranks == 1, "cgo_obj_softmax_create_csr is single-GPU");
     CGO_CHECK(ctx->csr_mode != 1, "softmax: the objective runs on the K-column SpMM (CGO_CSR_MODE=1 forbids it)");
@@ -2140,11 +2282,14 @@ extern "C" int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, in
     for (int64_t i = 0; i < N; ++i)
         CGO_CHECK(labels[i] >= 0 && labels[i] < K, "label %d of sample %lld is not in [0, %d)", (int)labels[i], (long long)i, (int)K);
     CGO_CHECK(std::isfinite(lambda) && lambda >= 0.0, "softmax: lambda = %g must be finite and >= 0", lambda);
+    double S;
+    CGO_TRY(check_glm(ctx, "softmax", N, d, sample_weight, fit_intercept, &S));
     CGO_CUDA(cudaSetDevice(ctx->device));
-    const int64_t nnz = rowptr[N];
+    const int64_t nnz = rowptr[N], n = (d + fit_intercept) * K;
     CsrObj *o = new CsrObj();
-    o->ctx = ctx; o->logreg = true; o->nclass = K; o->lambda = lambda; o->nsamples = N;
-    o->n_global = d * K; o->n_local = d * K; o->offset = 0; o->nrows = N; o->halo = 0;
+    o->ctx = ctx; o->logreg = true; o->nclass = K; o->lambda = lambda; o->nsamples = N; o->wsum = S;
+    o->icpt = fit_intercept == 1;
+    o->n_global = n; o->n_local = n; o->offset = 0; o->nrows = N; o->halo = 0;
     o->LA.width = o->LAT.width = K;
     auto body = [&]() -> int {
         cudaStream_t s = ctx->stream;
@@ -2160,12 +2305,14 @@ extern "C" int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, in
         CGO_CUDA(cudaMalloc(&o->b, sizeof(double) * (size_t)(N + CSR_PAD)));
         CGO_CUDA(cudaMemsetAsync(o->b, 0, sizeof(double) * (size_t)(N + CSR_PAD), s));
         CGO_CUDA(cudaMemcpyAsync(o->b, yd.data(), sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, s));
+        CGO_TRY(upload_weights(ctx, o, sample_weight, N));
         CGO_TRY(o->alloc_r());
         CsrSrc src{o->A.col, nnz};
         CsrFin fin{o->A.rowptr, N, o->A.val};
         CGO_TRY(build_transpose(ctx, src, fin, d, o->AT));
         CGO_TRY(split_long_rows(ctx, o->A, o->LA));
         CGO_TRY(split_long_rows(ctx, o->AT, o->LAT));
+        if (o->icpt) CGO_TRY(add_unit_row(ctx, o->LAT, d, N));
         // K_b gathers d·K doubles, K_c N·K: column blocks of gather_block_bytes / 8K features / samples
         CGO_TRY(build_blocked(ctx, o->A, d, K, o->Ab));
         CGO_TRY(build_blocked(ctx, o->AT, N, K, o->ATb));
@@ -2183,6 +2330,11 @@ extern "C" int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, in
     if (rc) { delete o; return rc; }
     *out = o;
     return 0;
+}
+extern "C" int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t N, int64_t d, int32_t K, const int64_t *rowptr,
+                                          const int32_t *col, const double *val, const int32_t *labels, double lambda,
+                                          cgo_obj **out) {
+    return cgo_obj_softmax_create_csr_ex(ctx, N, d, K, rowptr, col, val, labels, nullptr, 0, lambda, out);
 }
 
 // ------------------------------------------------------------------ test hooks
@@ -2268,7 +2420,8 @@ extern "C" int cgo_obj_csr_download(cgo_obj *obj, int transposed, int64_t *rowpt
 static int spmm_hook(CsrObj *o, int transposed, const double *x_host, double *y_host) {
     cgo_ctx *c = o->ctx;
     CGO_CUDA(cudaSetDevice(c->device));
-    const int64_t K = o->nclass, nin = (transposed ? o->A.nrows : o->AT.nrows) * K, nout = (transposed ? o->AT.nrows : o->A.nrows) * K;
+    // transposed: all n entries of the state, Aᵀ C followed by the intercept's sums
+    const int64_t K = o->nclass, nin = (transposed ? o->A.nrows : o->AT.nrows) * K, nout = transposed ? o->n_local : o->A.nrows * K;
     const int tclass = transposed ? CGO_T_SPMVT : CGO_T_SPMV;
     double *dx = nullptr, *dy = nullptr;
     auto body = [&]() -> int {
@@ -2295,7 +2448,7 @@ extern "C" int cgo_obj_spmv(cgo_obj *obj, int transposed, const double *x_host, 
     cgo_ctx *c = o->ctx;
     CGO_CUDA(cudaSetDevice(c->device));
     const CsrMat &M = transposed ? o->AT : o->A;
-    const int64_t nin = transposed ? o->A.nrows : o->AT.nrows, nout = M.nrows;
+    const int64_t nin = transposed ? o->A.nrows : o->AT.nrows, nout = transposed ? o->n_local : M.nrows;   // Aᵀ x [, Σ x]
     double *dx = nullptr, *dy = nullptr;
     auto body = [&]() -> int {
         CGO_CUDA(cudaMalloc(&dx, sizeof(double) * (size_t)nin));

@@ -222,6 +222,14 @@ int cgo_blas1_grad_dots(cgo_state *st);     // the eight dots of EpiGrad over (g
 // logistic regression on k_spmv_direct: g⁺ = g⁺ · invN + λ xp in place (g⁺ holds Aᵀc), fused with the dot pack of
 // EpiGrad (slots CGO_P_DPHI .. CGO_P_UU)
 int cgo_blas1_grad_combine(cgo_state *st, double invN, double lambda);
+// the GLM objectives with weights or an intercept (coordinates [npen, n) unpenalised): K_a with P, the penalised part
+// of xp·xp, in slot CGO_P_XPXP; the loss ops with weights wt (NULL: unit) and the intercept at bias (NULL: none);
+// the combine pass without λ w on the intercept coordinates
+int cgo_blas1_axpy_dir_pen(cgo_state *st, double a, bool fused_dir, double beta, int64_t npen);
+int cgo_blas1_logit_glm(cgo_ctx *ctx, double *zc, const double *y, const double *wt, const double *bias, int64_t n, int slot);
+int cgo_blas1_softmax_glm(cgo_ctx *ctx, double *zc, const double *y, const double *wt, const double *bias, int64_t n,
+                          int nclass, int slot);
+int cgo_blas1_grad_combine_pen(cgo_state *st, double invS, double lambda, int64_t npen);
 
 // ------------------------------------------------------------------ CSR (csr.cu)
 struct CsrMat {

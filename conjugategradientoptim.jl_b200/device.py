@@ -146,6 +146,7 @@ class DeviceObjective:
     """Device-resident replacement of the user callback `fdf!(g, x) -> f`."""
 
     nclasses = 1        # columns of the vectors `spmv` multiplies (the softmax objective's K)
+    intercept = 0       # 1: the state ends with an intercept row, which `spmv(transposed=True)` returns too
 
     def __init__(self, ctx: Context, handle: C.c_void_p):
         self.ctx, self.h = ctx, handle
@@ -199,7 +200,7 @@ class DeviceObjective:
         nr, nnz = C.c_int64(), C.c_int64()
         check(lib().cgo_obj_csr_nnz(self.h, int(transposed), C.byref(nr), C.byref(nnz)))
         x = np.ascontiguousarray(x, dtype=np.float64)
-        y = np.empty(nr.value * self.nclasses)
+        y = np.empty((nr.value + (self.intercept if transposed else 0)) * self.nclasses)
         check(lib().cgo_obj_spmv(self.h, int(transposed), dptr(x), dptr(y)))
         return y
 
@@ -304,11 +305,28 @@ def LogRegGPU(nsamples: int, nfeat: int, nnz_per_row: int = 20, seed: int = 24, 
     return DeviceObjective(ctx, h)
 
 
+def _glm_options(nsamples, sample_weight, fit_intercept):
+    """(weights pointer or None, the array that owns it, 0 / 1) of the GLM constructors"""
+    if fit_intercept not in (False, True, 0, 1):
+        raise CgoError(f"fit_intercept must be a bool (got {fit_intercept!r})")
+    if sample_weight is None:
+        return None, None, int(fit_intercept)
+    sw = np.ascontiguousarray(sample_weight, dtype=np.float64)
+    if sw.shape != (nsamples,):
+        raise CgoError(f"sample_weight needs nsamples = {nsamples} entries (got shape {sw.shape})")
+    return sw.ctypes.data, sw, int(fit_intercept)
+
+
 def LogRegGPU_from_csr(nsamples, nfeat, rowptr, col, val, y, lam: float = 1e-6,
-                       ctx: Optional[Context] = None) -> DeviceObjective:
-    """(1/N) Σ log(1 + exp(−y_i a_i·w)) + (λ/2)‖w‖² on the caller's CSR (0-based int64 row pointers, int32 columns)
-    and labels y_i ∈ {−1, +1}; single GPU.  An intercept is a column of ones in every row, and λ penalises its
-    weight like the others."""
+                       ctx: Optional[Context] = None, sample_weight=None, fit_intercept=False) -> DeviceObjective:
+    """(1/S) Σ s_i log(1 + exp(−y_i (a_i·w + b))) + (λ/2)‖w‖² on the caller's CSR (0-based int64 row pointers, int32
+    columns) and labels y_i ∈ {−1, +1}; single GPU.
+
+    `sample_weight`: nsamples finite weights s_i >= 0 with a positive sum S, or None for s_i = 1 (S = nsamples).
+    `fit_intercept`: fit b, which λ does not penalise.  The state is then (w, b) of length nfeat + 1: b is
+    `minimizer[nfeat]`, where an explicit column of ones appended as feature nfeat would put its weight.  Without it
+    there is no b; a column of ones in A is an intercept that λ penalises like the other weights.  Weights or an
+    intercept need the k_spmv_direct kernel family (a ctx with csr_mode 1 rejects them)."""
     ctx = ctx or default_context()
     rowptr = np.ascontiguousarray(rowptr, dtype=np.int64)
     col = np.ascontiguousarray(col, dtype=np.int32)
@@ -318,19 +336,28 @@ def LogRegGPU_from_csr(nsamples, nfeat, rowptr, col, val, y, lam: float = 1e-6,
         raise CgoError(f"rowptr needs nsamples + 1 = {nsamples + 1} entries and y nsamples (got {rowptr.size}, {y.size})")
     if col.size < rowptr[-1] or val.size < rowptr[-1]:
         raise CgoError(f"col and val need rowptr[-1] = {rowptr[-1]} entries (got {col.size}, {val.size})")
+    sw_ptr, _sw, icpt = _glm_options(nsamples, sample_weight, fit_intercept)
     h = C.c_void_p()
-    check(lib().cgo_obj_logreg_create_csr(ctx.h, nsamples, nfeat, rowptr.ctypes.data, col.ctypes.data,
-                                          val.ctypes.data, y.ctypes.data, lam, C.byref(h)))
-    return DeviceObjective(ctx, h)
+    check(lib().cgo_obj_logreg_create_csr_ex(ctx.h, nsamples, nfeat, rowptr.ctypes.data, col.ctypes.data,
+                                             val.ctypes.data, y.ctypes.data, sw_ptr, icpt, lam, C.byref(h)))
+    obj = DeviceObjective(ctx, h)
+    obj.intercept = icpt
+    return obj
 
 
 def SoftmaxRegGPU_from_csr(nsamples, nfeat, nclasses, rowptr, col, val, labels, lam: float = 1e-6,
-                           ctx: Optional[Context] = None) -> DeviceObjective:
-    """(1/N) Σ_i [logsumexp(a_i W) − (a_i W)_{y_i}] + (λ/2)‖W‖² (multinomial logistic regression) on the caller's CSR
-    (0-based int64 row pointers, int32 columns) and labels y_i ∈ [0, nclasses), 2 <= nclasses <= 256; single GPU.
-    The state vector is W (nfeat × nclasses) feature-major, w[j·K + k], of length nfeat·nclasses: a result's
-    `minimizer.reshape(nfeat, nclasses)` is W.  An intercept is a column of ones, penalised like the other weights.
-    `spmv` takes and returns K-wide vectors: Z = A W (nfeat·K → nsamples·K) and Aᵀ C (nsamples·K → nfeat·K)."""
+                           ctx: Optional[Context] = None, sample_weight=None, fit_intercept=False) -> DeviceObjective:
+    """(1/S) Σ_i s_i [logsumexp(a_i W + b) − (a_i W + b)_{y_i}] + (λ/2)‖W‖² (multinomial logistic regression) on the
+    caller's CSR (0-based int64 row pointers, int32 columns) and labels y_i ∈ [0, nclasses), 2 <= nclasses <= 256;
+    single GPU.  The state vector is W (nfeat × nclasses) feature-major, w[j·K + k], of length nfeat·nclasses: a
+    result's `minimizer.reshape(nfeat, nclasses)` is W.
+
+    `sample_weight`: nsamples finite weights s_i >= 0 with a positive sum S, or None for s_i = 1 (S = nsamples).
+    `fit_intercept`: fit b (one per class), which λ does not penalise.  The state then has nfeat + 1 rows:
+    `minimizer.reshape(nfeat + 1, nclasses)[nfeat]` is b, where an explicit column of ones appended as feature nfeat
+    would put its weights.  Without it there is no b; a column of ones in A is an intercept penalised like the
+    other weights.  `spmv` takes and returns K-wide vectors: Z = A W (nfeat·K → nsamples·K) and Aᵀ C (nsamples·K →
+    nfeat·K, followed by the K intercept sums Σ_i c_ik with an intercept)."""
     ctx = ctx or default_context()
     rowptr = np.ascontiguousarray(rowptr, dtype=np.int64)
     col = np.ascontiguousarray(col, dtype=np.int32)
@@ -343,11 +370,14 @@ def SoftmaxRegGPU_from_csr(nsamples, nfeat, nclasses, rowptr, col, val, labels, 
     if not np.issubdtype(labels.dtype, np.integer) or labels.size and (labels.min() < -2**31 or labels.max() >= 2**31):
         raise CgoError("labels must be integers")
     labels = np.ascontiguousarray(labels, dtype=np.int32)
+    sw_ptr, _sw, icpt = _glm_options(nsamples, sample_weight, fit_intercept)
     h = C.c_void_p()
-    check(lib().cgo_obj_softmax_create_csr(ctx.h, nsamples, nfeat, int(nclasses), rowptr.ctypes.data, col.ctypes.data,
-                                           val.ctypes.data, labels.ctypes.data, lam, C.byref(h)))
+    check(lib().cgo_obj_softmax_create_csr_ex(ctx.h, nsamples, nfeat, int(nclasses), rowptr.ctypes.data,
+                                              col.ctypes.data, val.ctypes.data, labels.ctypes.data, sw_ptr, icpt, lam,
+                                              C.byref(h)))
     obj = DeviceObjective(ctx, h)
     obj.nclasses = int(nclasses)
+    obj.intercept = icpt
     return obj
 
 

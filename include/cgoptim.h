@@ -28,8 +28,10 @@
  *   Long rows (logistic regression from a host CSR, cgo_obj_logreg_create_csr, on the k_spmv_direct family): a row
  *   of A or Aᵀ with more than CGO_LONG_ROW entries is summed in this order too — its products val_k · x[col_k], k in
  *   storage order, are the items, with V=1, U=4 and the ctx's G.  The softmax objective (cgo_obj_softmax_create_csr)
- *   applies the rule to A ⊗ I_K: for each class k, the items of a long row are val_k · x[col_k·K + k].  Every other
- *   row of every CSR matrix is summed sequentially in storage order.
+ *   applies the rule to A ⊗ I_K: for each class k, the items of a long row are val_k · x[col_k·K + k].  An intercept
+ *   (cgo_obj_logreg_create_csr_ex / cgo_obj_softmax_create_csr_ex) has the unit row: a row of Aᵀ that is not stored,
+ *   with entry 1.0 at every sample.  Its items are 1.0 · c_i (1.0 · c_ik for class k), summed in the long-row order
+ *   (V=1, U=4, the ctx's G) whatever N is.  Every other row of every CSR matrix is summed sequentially in storage order.
  *   CSR matrices whose gathers do not coalesce (the synthetic least-squares matrix with coh_log2 < 4; a host
  *   CSR whose warp-level gathers touch more than four lines on average: cgo_obj_reduction_site tells) are
  *   multiplied by a kernel without reductions, and their dots come from BLAS-1 passes (V=2, U=4).
@@ -167,7 +169,8 @@ int cgo_obj_logreg_create_synthetic(cgo_ctx *ctx, int64_t nsamples, int64_t nfea
  * summed by the whole grid in the canonical order instead of on one lane (see the canonical reduction order above) */
 #define CGO_LONG_ROW 1024
 /* (1/N) Σ log(1 + exp(−y_i a_i·w)) + (λ/2)‖w‖² from a host CSR (int64 row pointers, int32 columns, 0-based), labels
- * y_i ∈ {−1, +1}; single GPU.  An intercept is a column of ones, and λ penalises it like every other weight.  Every
+ * y_i ∈ {−1, +1}; single GPU.  A column of ones is an intercept that λ penalises like every other weight
+ * (cgo_obj_logreg_create_csr_ex fits one that it does not penalise).  Every
  * matrix with a row longer than CGO_LONG_ROW runs on k_spmv_direct; forced onto k_csr_rows (cgo_ctx_set_csr_mode 1)
  * it keeps sequential row sums, exact but slow on long rows. */
 int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, const int64_t *rowptr,
@@ -181,6 +184,27 @@ int cgo_obj_logreg_create_csr(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, con
 int cgo_obj_softmax_create_csr(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, int32_t nclasses,
                                const int64_t *rowptr, const int32_t *col, const double *val,
                                const int32_t *labels, double lambda, cgo_obj **out);
+/* The two objectives above with per-sample weights and an intercept that λ does not penalise:
+ *   binary   f(w, b) = (1/S) Σ_i s_i log(1 + exp(−y_i (a_i·w + b))) + (λ/2)‖w‖²
+ *   softmax  f(W, b) = (1/S) Σ_i s_i [logsumexp(a_i W + b) − (a_i W + b)_{y_i}] + (λ/2)‖W‖²
+ * with S = Σ_i s_i, correctly rounded on the host.  sample_weight: N finite weights >= 0 with S > 0, or NULL for unit
+ * weights (S = N).  fit_intercept 0 or 1.  The intercept is feature nfeat: the binary state is (w, b), n = nfeat + 1,
+ * x[nfeat] = b; the softmax state is feature-major W with b as its last row, n = (nfeat + 1)·K, b_k = x[nfeat·K + k].
+ * It is the layout of an explicit ones column appended as feature nfeat, which A no longer needs to store.
+ * Arithmetic: the margins are the row sums of A plus b (b_k); the loss op reduces s_i ℓ_i and writes c_i = s_i·(−y_i σ_i)
+ * (c_ik = s_i·(p_ik − [k = y_i])); the intercept's gradient is the sum of the unit row (see the canonical order above)
+ * times 1/S; a feature's gradient is (Aᵀc)_j / S + λ w_j; f = Σ/S + (λ/2) P, where P is xp·xp reduced by K_a with +0.0
+ * in place of every intercept coordinate's square.  With (NULL, 0) these are the constructors above.  Otherwise the
+ * objective runs on k_spmv_direct (binary) or the SpMM (softmax) and rejects cgo_ctx_set_csr_mode 1.  Single GPU; no
+ * Hessian-vector product or quadratic-aware line search.  cgo_obj_spmv(transposed = 1) returns all n entries: Aᵀc
+ * followed by the intercept's sums; transposed = 0 multiplies A by the feature part; the CSR download returns A. */
+int cgo_obj_logreg_create_csr_ex(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, const int64_t *rowptr,
+                                 const int32_t *col, const double *val, const double *y, const double *sample_weight,
+                                 int32_t fit_intercept, double lambda, cgo_obj **out);
+int cgo_obj_softmax_create_csr_ex(cgo_ctx *ctx, int64_t nsamples, int64_t nfeat, int32_t nclasses,
+                                  const int64_t *rowptr, const int32_t *col, const double *val,
+                                  const int32_t *labels, const double *sample_weight, int32_t fit_intercept,
+                                  double lambda, cgo_obj **out);
 /* t·f0(x) − Σ log(ubs − x) − Σ log(x − lbs) around `inner` (which must outlive it): evalbarrier!
  * (src/engine/primal_barrier.jl:112-133) with the box constraints of examples/constrained.jl:17-47;
  * lbs / ubs are this rank's shard.  cgo_obj_barrier_set_t changes t between centering steps (:246);

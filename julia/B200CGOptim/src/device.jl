@@ -116,24 +116,36 @@ function LogRegGPU(nsamples::Integer, nfeat::Integer, ctx::Context; nnz_per_row 
     return _wrap(ctx, h[])
 end
 "CSR logistic regression on the caller's CSR (0-based int64 row pointers, int32 columns) and labels ±1; single GPU.
-An intercept is a column of ones, and λ penalises its weight like the others."
+`sample_weight`: nsamples finite weights >= 0 with a positive sum S (`nothing`: unit weights, S = nsamples); the loss
+is (1/S) Σ s_i ℓ_i.  `fit_intercept = true` fits b, which λ does not penalise: the state is (w, b), n = nfeat + 1,
+and `x[nfeat + 1]` is b.  Without it, a column of ones in A is an intercept that λ penalises like the other weights."
 function LogRegGPU(nsamples::Integer, nfeat::Integer, rowptr::Vector{Int64}, col::Vector{Int32},
-                   val::Vector{Float64}, y::Vector{Float64}, ctx::Context; λ = 1e-6)
+                   val::Vector{Float64}, y::Vector{Float64}, ctx::Context; λ = 1e-6,
+                   sample_weight::Union{Nothing, Vector{Float64}} = nothing, fit_intercept::Bool = false)
+    sample_weight === nothing || length(sample_weight) == nsamples || throw(ArgumentError("sample_weight needs nsamples entries"))
+    sw = sample_weight === nothing ? Ptr{Float64}(C_NULL) : pointer(sample_weight)
     h = Ref{Ptr{Cvoid}}(C_NULL)
-    check(ccall((:cgo_obj_logreg_create_csr, LIBCGOPTIM[]), Cint,
-        (Ptr{Cvoid}, Int64, Int64, Ptr{Int64}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Float64, Ref{Ptr{Cvoid}}),
-        ctx.h, nsamples, nfeat, rowptr, col, val, y, λ, h))
+    GC.@preserve sample_weight check(ccall((:cgo_obj_logreg_create_csr_ex, LIBCGOPTIM[]), Cint,
+        (Ptr{Cvoid}, Int64, Int64, Ptr{Int64}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int32, Float64,
+         Ref{Ptr{Cvoid}}),
+        ctx.h, nsamples, nfeat, rowptr, col, val, y, sw, Int32(fit_intercept), λ, h))
     return _wrap(ctx, h[])
 end
 "Softmax (multinomial logistic) regression on the caller's CSR (0-based int64 row pointers, int32 columns) and labels in
 [0, nclasses), 2 <= nclasses <= 256; single GPU.  The state vector is W (nfeat × nclasses) feature-major, w[j·K + k]:
-`permutedims(reshape(x, nclasses, nfeat))` is W.  An intercept is a column of ones, and λ penalises its weights."
+`permutedims(reshape(x, nclasses, nfeat))` is W.  `sample_weight` as for `LogRegGPU`.  `fit_intercept = true` fits
+b_k, which λ does not penalise: the state has nfeat + 1 rows and `permutedims(reshape(x, nclasses, nfeat + 1))[end, :]`
+is b.  Without it, a column of ones in A is an intercept whose weights λ penalises."
 function SoftmaxRegGPU(nsamples::Integer, nfeat::Integer, nclasses::Integer, rowptr::Vector{Int64}, col::Vector{Int32},
-                       val::Vector{Float64}, labels::Vector{Int32}, ctx::Context; λ = 1e-6)
+                       val::Vector{Float64}, labels::Vector{Int32}, ctx::Context; λ = 1e-6,
+                       sample_weight::Union{Nothing, Vector{Float64}} = nothing, fit_intercept::Bool = false)
+    sample_weight === nothing || length(sample_weight) == nsamples || throw(ArgumentError("sample_weight needs nsamples entries"))
+    sw = sample_weight === nothing ? Ptr{Float64}(C_NULL) : pointer(sample_weight)
     h = Ref{Ptr{Cvoid}}(C_NULL)
-    check(ccall((:cgo_obj_softmax_create_csr, LIBCGOPTIM[]), Cint,
-        (Ptr{Cvoid}, Int64, Int64, Int32, Ptr{Int64}, Ptr{Int32}, Ptr{Float64}, Ptr{Int32}, Float64, Ref{Ptr{Cvoid}}),
-        ctx.h, nsamples, nfeat, nclasses, rowptr, col, val, labels, λ, h))
+    GC.@preserve sample_weight check(ccall((:cgo_obj_softmax_create_csr_ex, LIBCGOPTIM[]), Cint,
+        (Ptr{Cvoid}, Int64, Int64, Int32, Ptr{Int64}, Ptr{Int32}, Ptr{Float64}, Ptr{Int32}, Ptr{Float64}, Int32, Float64,
+         Ref{Ptr{Cvoid}}),
+        ctx.h, nsamples, nfeat, nclasses, rowptr, col, val, labels, sw, Int32(fit_intercept), λ, h))
     return _wrap(ctx, h[])
 end
 
